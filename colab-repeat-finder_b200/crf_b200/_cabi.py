@@ -27,6 +27,7 @@ EXPORTS = [
     "crf_seq_load_packed_runs", "crf_seq_load_packed_runs_ranges", "crf_mask_runs",
     "crf_fasta_packed", "crf_seq_load_ascii", "crf_seq_load_ascii_ranges", "crf_seq_set_output_map", "crf_seq_destroy", "crf_seq_info", "crf_scan", "crf_fetch",
     "crf_scan_stats", "crf_run_end", "crf_fetch_open", "crf_patch_end", "crf_write_rows",
+    "crf_write_rows_at",
     "crf_fasta_open", "crf_fasta_info", "crf_fasta_data", "crf_fasta_close", "crf_gunzip",
     "crf_xchg_create", "crf_xchg_destroy", "crf_xchg_export", "crf_xchg_connect_ipc", "crf_xchg_connect_local",
     "crf_xchg_set_timeout", "crf_xchg_set_compact", "crf_scan_gather", "crf_xchg_push", "crf_xchg_wait", "crf_xchg_step_result", "crf_xchg_fetch",
@@ -110,6 +111,7 @@ def lib():
         L.crf_fetch_open.argtypes = [vp, vp, u32, P(u32)]
         L.crf_patch_end.argtypes = [vp, u64, u32]
         L.crf_write_rows.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
+        L.crf_write_rows_at.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
         L.crf_fasta_open.argtypes = [ctypes.c_char_p, u32, i, P(vp)]
         L.crf_fasta_info.argtypes = [vp, P(u64), P(u64), P(i)]
         L.crf_fasta_data.argtypes = [vp, P(vp), P(vp), P(vp), P(u64)]
@@ -627,9 +629,10 @@ class Fasta:
             pass
 
 
-def write_rows(path, names, bases, offsets, record, start, end, k, tsv=False, append=False):
+def write_rows(path, names, bases, offsets, record, start, end, k, tsv=False, append=False, origin=None):
     """Native BED / TSV writer (crf_write_rows).  bases: bytes or uint8 array with all records back to back;
-    names: list of str, or the NUL-separated blob."""
+    names: list of str, or the NUL-separated blob.  origin: per record, a uint64 added to the printed start and end
+    (crf_write_rows_at; the rows of a record longer than 2^32 bases are written unit by unit, relative to each unit)."""
     if isinstance(names, (bytes, bytearray)):
         blob = bytes(names)
     else:
@@ -641,8 +644,13 @@ def write_rows(path, names, bases, offsets, record, start, end, k, tsv=False, ap
     else:
         bptr = ctypes.cast(ctypes.c_char_p(bases), ctypes.c_void_p).value or 0
     nbytes = ctypes.c_uint64()
-    _check(lib().crf_write_rows(os.fsencode(path), int(append), int(tsv),
-                                ctypes.cast(ctypes.c_char_p(blob), ctypes.c_void_p) if blob is not None else None,
-                                ctypes.c_void_p(bptr), ctypes.c_void_p(offsets.ctypes.data),
-                                *(ctypes.c_void_p(a.ctypes.data) for a in arrs), len(arrs[0]), ctypes.byref(nbytes)))
+    head = (os.fsencode(path), int(append), int(tsv),
+            ctypes.cast(ctypes.c_char_p(blob), ctypes.c_void_p) if blob is not None else None,
+            ctypes.c_void_p(bptr), ctypes.c_void_p(offsets.ctypes.data))
+    tail = (*(ctypes.c_void_p(a.ctypes.data) for a in arrs), len(arrs[0]), ctypes.byref(nbytes))
+    if origin is None:
+        _check(lib().crf_write_rows(*head, *tail))
+    else:
+        origin = np.ascontiguousarray(origin, dtype=np.uint64)
+        _check(lib().crf_write_rows_at(*head, ctypes.c_void_p(origin.ctypes.data), *tail))
     return nbytes.value

@@ -71,11 +71,26 @@ def _upper_slice(seq, start, k):
 
 
 def scan_arrays(raw, kmin, kmax, min_repeats, min_span, device=None, **knobs):
-    """One record (bytes / uint8 array) -> (start, end, k) uint32 arrays, sorted by (start, end)."""
+    """One record (bytes / uint8 array) -> (start, end, k), sorted by (start, end).  uint32 arrays when the record fits
+    one device load; a longer record is cut into units spread over several loads (multi.RankScan) and start / end come
+    back as uint64."""
     ctx = get_context(device)
-    with ctx.load(raw, max_motif_cap=kmax) as seq:
-        n = seq.scan(kmin, kmax, min_repeats, min_span, **knobs)
-        _, start, end, k = seq.fetch(n)
+    if len(raw) + kmax <= _cabi.load_limit(kmax):
+        with ctx.load(raw, max_motif_cap=kmax) as seq:
+            n = seq.scan(kmin, kmax, min_repeats, min_span, **knobs)
+            _, start, end, k = seq.fetch(n)
+        return start, end, k
+    from . import multi, partition
+    if not isinstance(raw, np.ndarray):
+        raw = np.frombuffer(raw, dtype=np.uint8)
+    rs = multi.RankScan(ctx, multi.ThreadComm.split(1)[0], raw, [0], [len(raw)], kmin, kmax, min_repeats, min_span,
+                        chunk=partition.DEFAULT_CHUNK, halo=partition.DEFAULT_HALO, knobs=knobs)
+    try:
+        rs.step_async()
+        rs.finish()
+        _, start, end, k = rs.fetch()
+    finally:
+        rs.close()
     return start, end, k
 
 

@@ -8,7 +8,8 @@ Same flags, defaults, stdout lines and output files as the reference's main()
 
 Deliberate deviations (SURVEY.md section 8b):
   * a FASTA file WITHOUT --interval works (the reference raises AttributeError at :139): all records go to the GPU
-    in one load and one scan, rows are written by the native writer (crf_write_rows);
+    in one load and one scan (a record longer than one load: in several), rows are written by the native writer
+    (crf_write_rows);
   * --plot is accepted but plotting is out of scope here (matplotlib is not a dependency).
 """
 import argparse
@@ -89,8 +90,8 @@ def parse_devices(text):
 def group_records(lengths, max_motif_size, limit=None):
     """Cut the record list into consecutive groups that each fit one device load: a load lays every record out
     as length + max_motif_size positions and holds at most crf_load_limit() of them (32-bit positions on the
-    device).  A single record above the limit is its own group (and is refused by the load with a clear message).
-    Returns [(first, last)), ...]."""
+    device).  A single record above the limit is its own group (its units are spread over several
+    loads, see _whole_fasta_to_bed).  Returns [(first, last)), ...]."""
     limit = _cabi.load_limit(max_motif_size) if limit is None else limit
     groups, first, n = [], 0, len(lengths)
     while first < n:
@@ -114,11 +115,26 @@ def _whole_fasta_to_bed(fa, args, bed_path):
     # the text is packed to 2-bit planes + mask on the host (threaded, at ingest) and uploaded at 0.375 B/bp; the ASCII
     # buffer stays on the host for the motif column
     planes = fa.packed() if fa.total_bases else None
+    limit = _cabi.load_limit(args.max_motif_size)
     for first, last in group_records(lengths, args.max_motif_size):
         total = int(lengths[first:last].sum())
         base0 = int(fa.offsets[first])
         blob = fa.bases[base0:base0 + total]
         offsets = fa.offsets[first:last + 1] - np.uint64(base0)
+        if total and int(lengths[first:last].max()) + args.max_motif_size > limit:
+            # a record longer than one load (its group holds only it): its units go to several loads, on one GPU or over
+            # --devices; rows come back relative to their unit and the writer adds the unit's 64-bit origin
+            from . import multi, partition
+            (unit, start, end, k), units = multi.scan_on_devices(
+                devices, planes, fa.offsets[first:last], lengths[first:last], args.min_motif_size, args.max_motif_size,
+                args.min_repeats, args.min_span, chunk=partition.DEFAULT_CHUNK, halo=partition.DEFAULT_HALO,
+                contexts=[api.get_context(d) for d in devices], by_unit=True)
+            rec_of = np.array([u.record for u in units], dtype=np.int64)
+            origin = np.array([u.d0 for u in units], dtype=np.uint64)
+            names = [fa.names[first + r] for r in rec_of.tolist()]
+            _cabi.write_rows(bed_path, names, blob, offsets[rec_of] + origin, unit, start, end, k, append=True, origin=origin)
+            counts[first:last] += np.bincount(rec_of[unit.astype(np.int64)], minlength=last - first)
+            continue
         if total:
             if len(devices) > 1:
                 from . import multi

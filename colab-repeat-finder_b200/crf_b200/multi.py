@@ -71,6 +71,15 @@ def global_rows(rows_of_rank, rank, local_rows):
     return np.asarray(local_rows, dtype=np.int64) + int(offsets[rank])
 
 
+def unit_rows_to_records(units, unit, start, end, k):
+    """Unit-relative rows (unit index, start, end, k) -> (record uint32, start uint64, end uint64, k): each unit's
+    origin d0 is added in 64 bits (partition.localize does the same arithmetic in int64)."""
+    rec = np.array([u.record for u in units], dtype=np.uint32)
+    d0 = np.array([u.d0 for u in units], dtype=np.uint64)
+    unit = np.asarray(unit, dtype=np.int64)
+    return rec[unit], np.asarray(start).astype(np.uint64) + d0[unit], np.asarray(end).astype(np.uint64) + d0[unit], k
+
+
 class RankScan:
     """One rank (one GPU) of a partitioned scan.
 
@@ -78,11 +87,16 @@ class RankScan:
     rank's view of the bytes: a host array, _cabi.PackedPlanes or, with on_device, a device pointer).  reads=True
     splits the records by count instead of cutting them into chunks (config C5: many short independent sequences).
 
-    phases > 1 (N > 1 only): the genome-ordered unit list is cut into phases x N contiguous shares and rank r takes
-    share p * N + r in phase p -- one sequence per phase.  A step scans the phases one after the other while the rows
-    of the phase before travel to rank 0 on the exchange's own stream: the gather, which is bound by rank 0's NVLink
-    ingress, hides behind the next phase's scan.  Genome order = phase-major, rank-minor, so rank 0's buffer still
-    holds the sorted result."""
+    phases > 1: the genome-ordered unit list is cut into phases x N contiguous shares and rank r takes share p * N + r in
+    phase p -- one sequence per phase.  A step scans the phases one after the other while the rows of the phase before
+    travel to rank 0 on the exchange's own stream: the gather, which is bound by rank 0's NVLink ingress, hides behind
+    the next phase's scan.  Genome order = phase-major, rank-minor, so rank 0's buffer still holds the sorted result.
+    The phase count is raised above `phases` when a share would not fit one load (crf_load_limit): that is how a record
+    longer than one load is scanned, on one GPU (N = 1: several loads, scanned one after the other) or on several.
+
+    Records longer than one load ("long" mode): every unit is reported as a record of its own (output map: out_record =
+    global unit index, no shift), so the rows stay unit-relative and 32-bit on the device; fetch() adds each unit's
+    origin on the host in 64 bits (start / end come back as uint64), fetch_units() hands the unit-relative rows out."""
 
     def __init__(self, ctx, comm, bases, record_starts, lengths, kmin, kmax, min_repeats, min_span, on_device=False,
                  chunk=partition.DEFAULT_CHUNK, halo=partition.DEFAULT_HALO, reads=False, row_cap=None, knobs=None,
@@ -94,7 +108,11 @@ class RankScan:
         lengths = [int(x) for x in lengths]
         self.total_bp = int(sum(lengths))
         self.reads = reads
-        self.phases = max(1, int(phases)) if self.world > 1 else 1
+        self.limit = _cabi.load_limit(kmax)
+        self.long = not reads and any(n + kmax > self.limit for n in lengths)
+        if self.long:                                  # any filter a single load accepts works with units of a long record
+            halo = max(halo, partition.halo_needed(kmax, min_repeats, min_span))
+        self.phases = max(1, int(phases))
         self._lengths, self._record_starts = lengths, record_starts
         self._plan_args = dict(chunk=chunk, halo=halo, kmax=kmax, min_repeats=min_repeats, min_span=min_span)
         self._source = (bases, on_device, base_offset)
@@ -106,7 +124,8 @@ class RankScan:
             self.xchg = _cabi.Xchg(ctx, self.rank, self.world, row_cap or default_row_cap(self.total_bp))
             if timeout_s:
                 self.xchg.set_timeout(timeout_s)
-            if len(lengths) < 65536 and kmax < 65536:  # 12-byte rows over NVLink (record and motif size share a word)
+            n_out = len(self.plan.units) if self.long else len(lengths)     # record numbers the rows carry
+            if n_out < 65536 and kmax < 65536:         # 12-byte rows over NVLink (record and motif size share a word)
                 self.xchg.set_compact(True)
             if comm.same_process:
                 peers = comm.allgather_obj(self.xchg)
@@ -144,7 +163,10 @@ class RankScan:
             self.n_units = n_rec
         else:
             whole = self.world == 1 and self._plan_args["chunk"] >= max(lengths + [1])
-            self.plan = partition.Plan(lengths, shares, density=density, **self._plan_args)
+            self.plan, P = partition.plan_loads(lengths, self.world, P, self.limit, density=density, **self._plan_args)
+            if P != self.phases:
+                self.phases = P
+                self.seqs = [None] * P
             for p in range(P):
                 v = p * self.world + self.rank
                 starts, lens, own_lo, own_hi = self.plan.load_args(v, record_starts)
@@ -215,6 +237,10 @@ class RankScan:
                     if self.world > 1:
                         seq.set_output_map(out_record=np.arange(self.first_record[p], self.first_record[p] + len(starts),
                                                                 dtype=np.uint32))
+                elif self.long:
+                    us = self.units[p]
+                    seq.set_output_map(out_record=[u.index for u in us],
+                                       open_ended=[int(u.d1 < u.rec_len) for u in us])
                 elif self.world > 1 or own_lo is not None:
                     us = self.units[p]
                     seq.set_output_map(out_record=[u.record for u in us], out_shift=[u.d0 for u in us],
@@ -232,7 +258,7 @@ class RankScan:
         """Queue one whole step on this rank's streams (per phase: scan, assembly, push to rank 0); returns at once."""
         kmin, kmax, mr, ms = self.filters
         if self.world == 1:
-            self._n = self.seqs[0].scan(kmin, kmax, mr, ms, **self.knobs)
+            self._n = [0 if seq is None else seq.scan(kmin, kmax, mr, ms, **self.knobs) for seq in self.seqs]
         else:
             for p, seq in enumerate(self.seqs):
                 seq.scan_gather(self.xchg, kmin, kmax, mr, ms, append=p > 0, **self.knobs)
@@ -242,9 +268,10 @@ class RankScan:
         self.steps_repeated = 0
         if self.world == 1:
             self.last = None
-            if self.plan is not None and self.load_args[0][2] is not None and self.seqs[0].stats().n_open:
+            if self.plan is not None and self.load_args[0][2] is not None and \
+                    any(seq is not None and seq.stats().n_open for seq in self.seqs):
                 self._stitch_local()
-            return self._n
+            return sum(self._n)
         kmin, kmax, mr, ms = self.filters
         res = self.xchg.wait()
         if res.worst_status == _cabi.XCHG_VOID_STEP:
@@ -278,11 +305,7 @@ class RankScan:
             if n_open:
                 mine += [(p,) + tuple(int(x) for x in row) for row in seq.fetch_open(cap=n_open)]
         per_rank = self.comm.allgather_obj(mine)
-        open_all = [row[2:] for part in per_rank for row in part]          # (record, start, end_lower_bound, k)
-
-        def run_end(unit, local_pos, k):               # unit belongs to one of this rank's shares
-            v = self.plan.rank_of_unit(unit.index)
-            return self.seqs[v // N].run_end(unit.index - self.plan.bounds[v], local_pos, k)
+        open_all = [self._in_records(row[2:]) for part in per_rank for row in part]   # (record, start, end_lower_bound, k)
 
         def exchange(answers):
             merged = {}
@@ -290,26 +313,51 @@ class RankScan:
                 merged.update(part)
             return merged
 
-        fixed = partition.stitch(self.plan, open_all, run_end, exchange, self.rank, owner=lambda v: v % N)
+        fixed = partition.stitch(self.plan, open_all, self._run_end, exchange, self.rank, owner=lambda v: v % N)
         if self.rank == 0:
             rows, ends, i = [], [], 0
             for r, part in enumerate(per_rank):
-                for (p, local_row, *_rest) in part:
+                for (p, local_row, record, *_rest) in part:
                     pr = self.phase_results[p]
                     g = global_rows(pr.rows_of_rank[:N], r, [local_row])
                     rows.append(int(pr.base_rows) + int(g[0]))
-                    ends.append(fixed[i][2])
+                    ends.append(self._as_reported(record, fixed[i][2]))
                     i += 1
             self.xchg.patch_end(rows, ends)
 
     def _stitch_local(self):
-        """One rank, records cut into chunks: finish the open-ended rows in place."""
-        seq = self.seqs[0]
-        rows = seq.fetch_open(cap=int(seq.stats().n_open))
-        fixed = partition.stitch(self.plan, [tuple(int(x) for x in r[1:]) for r in rows],
-                                 lambda unit, lp, k: seq.run_end(unit.index, lp, k))
-        for row, (_r, _s, e, _k) in zip(rows, fixed):
-            seq.patch_end(int(row[0]), e)
+        """One rank, records cut into chunks: finish the open-ended rows in place (every phase's sequence)."""
+        opened = []                                    # (phase, row, record, start, end, k)
+        for p, seq in enumerate(self.seqs):
+            n_open = 0 if seq is None else int(seq.stats().n_open)
+            if n_open:
+                opened += [(p,) + tuple(int(x) for x in r) for r in seq.fetch_open(cap=n_open)]
+        fixed = partition.stitch(self.plan, [self._in_records(r[2:]) for r in opened], self._run_end, owner=lambda v: 0)
+        for (p, row, record, *_rest), (_r, _s, e, _k) in zip(opened, fixed):
+            self.seqs[p].patch_end(row, self._as_reported(record, e))
+
+    def _run_end(self, unit, local_pos, k):
+        """crf_run_end on the sequence that holds `unit` (one of this rank's shares)."""
+        v = self.plan.rank_of_unit(unit.index)
+        return self.seqs[v // self.world].run_end(unit.index - self.plan.bounds[v], local_pos, k)
+
+    def _in_records(self, row):
+        """An open row as the device reports it -> (record, start, end, k) in record coordinates (Python ints)."""
+        record, start, end, k = row
+        if not self.long:
+            return record, start, end, k
+        u = self.plan.units[record]
+        return u.record, start + u.d0, end + u.d0, k
+
+    def _as_reported(self, record, end):
+        """A stitched end (record coordinates) -> the value patched into the device row (unit-relative in long mode)."""
+        if not self.long:
+            return end
+        end -= self.plan.units[record].d0
+        if end > 0xFFFFFFFF:
+            raise _cabi.CrfError(f"a perfect repeat of unit {record} ends {end} bases after the unit's origin: runs longer "
+                                 f"than 2^32 bases are not supported")
+        return end
 
     def stats(self):
         """Scan statistics of the last step, summed over this rank's phases (kernel_ms, scan_ms, launches, ...)."""
@@ -322,12 +370,33 @@ class RankScan:
         return out
 
     def fetch(self):
-        """Rank 0: the whole job's rows (record, start, end, k), sorted by (record, start, end)."""
+        """Rank 0: the whole job's rows (record, start, end, k), sorted by (record, start, end).  uint32 columns; in long
+        mode start and end are uint64 (record coordinates may pass 2^32)."""
+        rows = self._fetch_reported()
+        return unit_rows_to_records(self.plan.units, *rows) if self.long else rows
+
+    def fetch_units(self):
+        """Rank 0, long mode: the rows as the device holds them, (unit index, start, end, k) uint32 with start / end
+        relative to the unit's origin plan.units[unit].d0 -- what crf_write_rows_at takes."""
+        if not self.long:
+            raise _cabi.CrfError("fetch_units(): the rows are unit-relative only when a record is longer than one load")
+        return self._fetch_reported()
+
+    def _fetch_reported(self):
         if self.world == 1:
-            rec, st, en, k = self.seqs[0].fetch(self._n)
-            if self.plan is not None and self.load_args[0][2] is None:
-                rec = np.array([u.record for u in self.units[0]], dtype=np.uint32)[rec] if len(rec) else rec
-            return rec, st, en, k
+            parts = []
+            for p, seq in enumerate(self.seqs):
+                if seq is None:
+                    continue
+                rec, st, en, k = seq.fetch(self._n[p])
+                if self.plan is not None and self.load_args[p][2] is None:
+                    rec = np.array([u.record for u in self.units[p]], dtype=np.uint32)[rec] if len(rec) else rec
+                parts.append((rec, st, en, k))
+            if len(parts) == 1:
+                return parts[0]
+            if not parts:
+                return tuple(np.zeros(0, np.uint32) for _ in range(4))
+            return tuple(np.concatenate(col) for col in zip(*parts))
         if self.rank != 0:
             raise _cabi.CrfError("the gathered rows live on rank 0")
         return self.xchg.fetch(int(self.last.total_rows))
@@ -344,9 +413,11 @@ class RankScan:
 
 
 def scan_on_devices(devices, bases, record_starts, lengths, kmin, kmax, min_repeats, min_span, chunk=partition.DEFAULT_CHUNK,
-                    halo=partition.DEFAULT_HALO, reads=False, contexts=None, knobs=None, timeout_s=None, phases=1):
+                    halo=partition.DEFAULT_HALO, reads=False, contexts=None, knobs=None, timeout_s=None, phases=1,
+                    by_unit=False):
     """One process, one thread per device: scan host `bases` (a uint8 array, or _cabi.PackedPlanes) on all `devices`;
-    returns (record, start, end, k) of the whole job.  `contexts`: reuse these _cabi.Context objects (one per device) instead of creating new ones."""
+    returns (record, start, end, k) of the whole job.  `contexts`: reuse these _cabi.Context objects (one per device) instead of creating new ones.
+    by_unit (a record longer than one load among them): return (RankScan.fetch_units() rows, the plan's units) instead."""
     world = len(devices)
     comms = ThreadComm.split(world)
     ctxs = list(contexts) if contexts else [_cabi.Context(d) for d in devices]
@@ -363,7 +434,7 @@ def scan_on_devices(devices, bases, record_starts, lengths, kmin, kmax, min_repe
             rs.step_async()
             rs.finish()
             if rank == 0:
-                out["rows"] = rs.fetch()
+                out["rows"] = (rs.fetch_units(), rs.plan.units) if by_unit else rs.fetch()
         except BaseException as exc:          # noqa: BLE001 -- re-raised in the caller's thread
             errors.append(exc)
             comms[rank]._s.barrier.abort()

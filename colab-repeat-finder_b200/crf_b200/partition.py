@@ -30,6 +30,11 @@ DEFAULT_HALO = 1 << 20      # 1 Mbp (3 % of a unit): only a perfect repeat longe
 MIN_SPLIT = 1 << 20        # a share boundary closer than this to a chunk boundary moves onto it
 
 
+def halo_needed(kmax, min_repeats, min_span):
+    """The shortest halo that holds one qualifying repeat of the largest motif (and the base that ends it)."""
+    return max(min_span, min_repeats * kmax) + kmax + 2
+
+
 class Plan:
     """Records -> units (owned chunk + 1 base of left context + halo) -> contiguous shares, one per rank.
 
@@ -40,7 +45,7 @@ class Plan:
 
     def __init__(self, lengths, n_ranks, chunk=DEFAULT_CHUNK, halo=DEFAULT_HALO, kmax=50, min_repeats=3, min_span=9,
                  density=None):
-        need = max(min_span, min_repeats * kmax) + kmax + 2
+        need = halo_needed(kmax, min_repeats, min_span)
         if halo < need:
             raise ValueError(f"halo {halo} is shorter than one qualifying repeat of the largest motif ({need})")
         if chunk < 1:
@@ -145,6 +150,24 @@ class Plan:
         own_lo = np.array([u.u0 - u.d0 for u in mine], dtype=np.uint64)
         own_hi = np.array([u.u1 - u.d0 for u in mine], dtype=np.uint64)
         return starts, lens, own_lo, own_hi
+
+
+def load_positions(plan, share, kmax):
+    """Layout positions the load of `share` takes (crf_load_limit: every unit's data plus a gap of kmax)."""
+    return sum(u.d1 - u.d0 + kmax for u in plan.units_of(share))
+
+
+def plan_loads(lengths, world, phases, limit, density=None, **plan_args):
+    """The Plan of phases x world shares with the fewest phases (at least `phases`) whose every share fits one load of
+    `limit` layout positions -- a record longer than one load ends up spread over several loads of the same rank.
+    Returns (plan, phases).  A single unit above the limit (a chunk as long as a load) stays as it is: its load refuses it."""
+    kmax = plan_args.get("kmax", 50)
+    while True:
+        plan = Plan(lengths, phases * world, density=density, **plan_args)
+        worst = max(load_positions(plan, v, kmax) for v in range(phases * world))
+        if worst <= limit or max(u.d1 - u.d0 + kmax for u in plan.units) > limit:
+            return plan, phases
+        phases = max(phases + 1, -(-phases * worst // limit))
 
 
 def localize(plan, rank, unit_local, start, end, k):

@@ -163,6 +163,24 @@ def generate_records(lengths, seed, device=None, kmax=50, lower_case=True, telom
     return out, offsets, meta
 
 
+def long_record(length, seed=64, device=None, kmax=50, chunk=1 << 26):
+    """One record of `length` bases, which may pass 2^32 (the test workload of records longer than one device load).
+    The background of _fill_chunk repeats with period 2^32 (32-bit hashes of the position), so every 2^32-block of
+    positions gets a salt of its own: the bases at p and p - 2^32 differ, and a position read 2^32 off is caught.
+    Returns (bases, offsets, meta) like generate_records."""
+    be = _Backend(device)
+    ktab = be.from_numpy(_k_table(kmax))
+    out = be.empty_u8(length)
+    block = 1 << 32
+    assert block % chunk == 0
+    for lo in range(0, length, chunk):
+        salt = int(hash32(np.array([(seed * 1000003 + (lo // block) * 0x9E3779B1) & M32], dtype=np.int64))[0])
+        _fill_chunk(be, out, salt, lo, min(length, lo + chunk), kmax, ktab, True)
+    be.sync()
+    meta = {"workload": f"one record of {length} bp, seed {seed}"}
+    return out, np.array([0, length], dtype=np.uint64), meta
+
+
 def s38(device=None, scale=1.0, seed=38):
     """hg38-sized genome (config C3).  scale < 1 shrinks every record (CPU tests)."""
     lengths = [max(1000, int(n * scale)) for n in HG38_LENGTHS]

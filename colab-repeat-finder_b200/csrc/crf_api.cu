@@ -525,6 +525,13 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
         run_last = a;
     }
     const uint64_t n_runs_rel = run_last - run_first;
+    if (n_runs_rel > 0xFFFFFF00ull) {                                    // mask_runs_kernel takes a 32-bit run count
+        if (d_planes_own) ctx_free(d_planes_own);
+        if (d_src_own) ctx_free(d_src_own);
+        if (d_mask_own) ctx_free(d_mask_own);
+        set_err("%s: more than 2^32 masked runs in one load", who);
+        return CRF_ERR_UNSUPPORTED;
+    }
     trace.mark("source allocs + runs_rel");
     auto copy_span = [&](uint64_t lo, uint64_t n, cudaStream_t cs) -> cudaError_t {    // source positions [src_lo + lo, + n)
         if (!n) return cudaSuccess;

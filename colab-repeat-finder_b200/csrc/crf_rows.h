@@ -15,16 +15,17 @@
 #include <thread>
 #include <vector>
 
-static inline char *put_u32(char *p, uint32_t v) {
-    char tmp[10];
+static inline char *put_u64(char *p, uint64_t v) {
+    char tmp[20];
     int n = 0;
     do { tmp[n++] = (char)('0' + v % 10); v /= 10; } while (v);
     while (n) *p++ = tmp[--n];
     return p;
 }
 
+// origin (may be null): per record, added to the printed start and end (the motif is still read at offsets[r] + start)
 static int write_rows_impl(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
-                           const uint64_t *offsets, const uint32_t *record, const uint32_t *start,
+                           const uint64_t *offsets, const uint64_t *origin, const uint32_t *record, const uint32_t *start,
                            const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
     FILE *f = fopen(path, append ? "ab" : "wb");
     if (!f) { set_err("crf_write_rows: cannot open %s", path); return CRF_ERR_ARG; }
@@ -56,7 +57,7 @@ static int write_rows_impl(const char *path, int append, int tsv, const char *na
     if (tsv && !append) put("start_0based\tend\tmotif\n", 23);
     // Rows are formatted by a few threads, each a contiguous slice of a "wave" into its own buffer (the motif column is a
     // random read into the text: a cache miss per row), and the buffers of a wave are written in row order.
-    auto row_bytes = [&](uint64_t i) -> size_t { return (tsv ? 0 : name_len[record[i]] + 1) + 24 + motif_size[i] + 1; };
+    auto row_bytes = [&](uint64_t i) -> size_t { return (tsv ? 0 : name_len[record[i]] + 1) + 42 + motif_size[i] + 1; };
     auto format_rows = [&](uint64_t lo, uint64_t hi, std::vector<char> &buf) -> size_t {
         size_t need = 0;
         for (uint64_t i = lo; i < hi; ++i) need += row_bytes(i);
@@ -64,9 +65,10 @@ static int write_rows_impl(const char *path, int append, int tsv, const char *na
         char *p = buf.data();
         for (uint64_t i = lo; i < hi; ++i) {
             const uint32_t r = record[i], k = motif_size[i];
+            const uint64_t o = origin ? origin[r] : 0;
             if (!tsv) { memcpy(p, name_ptr[r], name_len[r]); p += name_len[r]; *p++ = '\t'; }
-            p = put_u32(p, start[i]); *p++ = '\t';
-            p = put_u32(p, end[i]); *p++ = '\t';
+            p = put_u64(p, o + start[i]); *p++ = '\t';
+            p = put_u64(p, o + end[i]); *p++ = '\t';
             const uint8_t *m = bases + offsets[r] + start[i];
             for (uint32_t j = 0; j < k; ++j) {
                 uint8_t c = m[j];
@@ -107,17 +109,23 @@ static int write_rows_impl(const char *path, int append, int tsv, const char *na
     return CRF_OK;
 }
 
-extern "C" int crf_write_rows(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
-                              const uint64_t *offsets, const uint32_t *record, const uint32_t *start,
-                              const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
+extern "C" int crf_write_rows_at(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
+                                 const uint64_t *offsets, const uint64_t *origin, const uint32_t *record, const uint32_t *start,
+                                 const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
     if (!path || (n_rows && (!bases || !offsets || !record || !start || !end || !motif_size)) || (!tsv && !names)) {
         set_err("crf_write_rows: null argument");
         return CRF_ERR_ARG;
     }
     try {                                            // no exception crosses the C boundary
-        return write_rows_impl(path, append, tsv, names, bases, offsets, record, start, end, motif_size, n_rows, bytes);
+        return write_rows_impl(path, append, tsv, names, bases, offsets, origin, record, start, end, motif_size, n_rows, bytes);
     } catch (const std::bad_alloc &) {
         set_err("crf_write_rows: out of host memory");
         return CRF_ERR_NOMEM;
     }
+}
+
+extern "C" int crf_write_rows(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
+                              const uint64_t *offsets, const uint32_t *record, const uint32_t *start,
+                              const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
+    return crf_write_rows_at(path, append, tsv, names, bases, offsets, nullptr, record, start, end, motif_size, n_rows, bytes);
 }

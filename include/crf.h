@@ -101,12 +101,20 @@ int crf_pack_ascii(const uint8_t *bases, uint64_t n_bases, uint32_t n_threads, u
                    uint64_t *exotic, uint64_t exotic_cap, uint64_t *n_exotic);
 int crf_seq_destroy(crf_seq *seq);
 /* Layout positions one load can hold: the sum over its records of (length + max_motif_cap) must not exceed this
- * (positions are 32-bit on the device); callers with more split the records over several loads. */
+ * (positions are 32-bit on the device); callers with more split the records over several loads.  A single record
+ * longer than this is cut into units (owned range, one base of left context, a halo of at least one qualifying
+ * repeat) that go to several *_ranges loads with own_lo / own_hi; each load maps its units to themselves with
+ * crf_seq_set_output_map (out_record = the caller's unit number, out_shift = NULL), so rows stay unit-relative and
+ * the caller adds each unit's 64-bit origin; open-ended rows are followed into the next unit with crf_run_end and
+ * patched with crf_patch_end (crf_b200/multi.py does this; crf_write_rows_at prints the sums). */
 uint64_t crf_load_limit(uint32_t max_motif_cap);
 /* Optional, for partitioned loads: report record r of this load as record out_record[r] with start/end
  * shifted by out_shift[r] (a unit's offset inside its chromosome), and count as "open" every result that
  * ends exactly at the end of a record flagged in open_ended[r] (the unit's data stops before the
- * chromosome does, so the run may continue: crf_scan_stats().n_open, see crf_run_end).  NULLs reset. */
+ * chromosome does, so the run may continue: crf_scan_stats().n_open, see crf_run_end).  NULLs reset.
+ * Shifted coordinates must fit 32 bits (CRF_ERR_UNSUPPORTED otherwise): for units of a chromosome longer than
+ * 2^32 bases, map every unit to a record number of its own with no shift and add the unit's origin on the host
+ * (see crf_load_limit). */
 int crf_seq_set_output_map(crf_seq *seq, const uint32_t *out_record, const uint64_t *out_shift,
                            const uint8_t *open_ended);
 
@@ -261,6 +269,12 @@ int crf_xchg_patch_end(crf_xchg *xchg, const uint64_t *rows, const uint32_t *new
 int crf_write_rows(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
                    const uint64_t *offsets, const uint32_t *record, const uint32_t *start, const uint32_t *end,
                    const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes);
+/* The same with origin[r] (NULL = 0 for every record) added to the printed start and end of record r's rows: the
+ * rows of a chromosome longer than 2^32 bases, written unit by unit (names repeated, offsets[u] = the host offset of
+ * the unit's origin, start / end relative to it).  crf_write_rows is this call with origin = NULL. */
+int crf_write_rows_at(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
+                      const uint64_t *offsets, const uint64_t *origin, const uint32_t *record, const uint32_t *start,
+                      const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes);
 
 /* ---- input (host only, no GPU) ---------------------------------------------------------------
  * Native FASTA ingest, replacing what the reference takes from pyfastx (prf:117-137: the records in file
