@@ -19,6 +19,7 @@ SCAN_BLOCK_TILES = 4
 SCAN_TWO_STRIPS = 8
 
 CRF_OK, CRF_ERR_CUDA, CRF_ERR_ARG, CRF_ERR_NOMEM, CRF_ERR_UNSUPPORTED, CRF_ERR_CAPACITY, CRF_ERR_IO = range(7)
+STOP_TO_END, STOP_UNDECIDED = -1, -2          # crf_interval_stop
 
 #: every symbol include/crf.h declares (tests check the library exports all of them)
 EXPORTS = [
@@ -26,7 +27,7 @@ EXPORTS = [
     "crf_ctx_synchronize", "crf_load_limit", "crf_seq_load_packed", "crf_seq_load_packed_ranges", "crf_pack_ascii",
     "crf_seq_load_packed_runs", "crf_seq_load_packed_runs_ranges", "crf_mask_runs",
     "crf_fasta_packed", "crf_seq_load_ascii", "crf_seq_load_ascii_ranges", "crf_seq_set_output_map", "crf_seq_destroy", "crf_seq_info", "crf_scan", "crf_fetch",
-    "crf_scan_stats", "crf_run_end", "crf_fetch_open", "crf_patch_end", "crf_write_rows",
+    "crf_scan_stats", "crf_run_end", "crf_interval_stop", "crf_fetch_open", "crf_patch_end", "crf_write_rows",
     "crf_write_rows_at",
     "crf_fasta_open", "crf_fasta_info", "crf_fasta_data", "crf_fasta_close", "crf_gunzip",
     "crf_xchg_create", "crf_xchg_destroy", "crf_xchg_export", "crf_xchg_connect_ipc", "crf_xchg_connect_local",
@@ -108,6 +109,7 @@ def lib():
         L.crf_fetch.argtypes = [vp, vp, vp, vp, vp, u64, i]
         L.crf_scan_stats.argtypes = [vp, P(ScanStats)]
         L.crf_run_end.argtypes = [vp, u32, u32, u32, P(u32)]
+        L.crf_interval_stop.argtypes = [vp, u32, u32, vp, vp, vp]
         L.crf_fetch_open.argtypes = [vp, vp, u32, P(u32)]
         L.crf_patch_end.argtypes = [vp, u64, u32]
         L.crf_write_rows.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
@@ -391,6 +393,19 @@ class Sequence:
         out = ctypes.c_uint32()
         _check(lib().crf_run_end(self._h, int(record), int(pos), int(k), ctypes.byref(out)))
         return out.value
+
+    @_serialised
+    def interval_stop(self, min_motif_size, max_motif_size, end_pos, full_len):
+        """crf_interval_stop: per record, where the interval-mode loop that ends its interval at end_pos breaks, the
+        record being the prefix of a sequence of full_len bases.  int64 array: a position, STOP_TO_END or STOP_UNDECIDED."""
+        end_pos = np.ascontiguousarray(end_pos, dtype=np.uint64)
+        full_len = np.ascontiguousarray(full_len, dtype=np.uint64)
+        if end_pos.shape != (self.n_records,) or full_len.shape != (self.n_records,):
+            raise ValueError("end_pos and full_len need one entry per record of the load")
+        stop = np.empty(self.n_records, np.int64)
+        _check(lib().crf_interval_stop(self._h, int(min_motif_size), int(max_motif_size), ctypes.c_void_p(end_pos.ctypes.data),
+                                       ctypes.c_void_p(full_len.ctypes.data), ctypes.c_void_p(stop.ctypes.data)))
+        return stop
 
     @_serialised
     def close(self):

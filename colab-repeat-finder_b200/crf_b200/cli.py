@@ -31,6 +31,11 @@ _FILTER_OPTIONS = [
 ]
 _OTHER_OPTIONS = [
     (("-i", "--interval"), dict(help="Restrict the scan to chrom:start_0based-end (FASTA input only).")),
+    # not in the reference: its Hail pipeline runs --interval once per 500 kb tile and concatenates the BED files
+    (("--intervals",), dict(metavar="BED", help="Run --interval for every line (chrom start_0based end ...) of a BED file "
+                                                "in one pass (FASTA input only): the output is the concatenation, in file "
+                                                "order, of what --interval writes for each line.  With --devices, the "
+                                                "intervals run on the first GPU.")),
     (("-p", "--plot"), dict(help="Plot file name (accepted for compatibility; plotting is not part of this build).")),
     (("-o", "--output-prefix"), dict(help="Prefix of the output file: <prefix>.tsv for a sequence given on the command "
                                           "line, <basename(prefix)>.bed for a FASTA file.")),
@@ -154,13 +159,95 @@ def _whole_fasta_to_bed(fa, args, bed_path):
     return counts
 
 
+def read_bed_intervals(parser, path):
+    """(chrom, start, end) of every interval line of a BED file; '#', 'track' and 'browser' lines and blank lines are
+    skipped, columns after the third are ignored.  A malformed line is a parser error naming it."""
+    out = []
+    with open(path, "rt") as f:
+        for lineno, line in enumerate(f, 1):
+            fields = line.split()
+            if not fields or fields[0].startswith("#") or fields[0] in ("track", "browser"):
+                continue
+            try:
+                out.append((fields[0], int(fields[1]), int(fields[2])))
+            except (IndexError, ValueError):
+                parser.error(f"--intervals {path}, line {lineno}: expected 'chrom start_0based end', got {line.rstrip()!r}")
+    return out
+
+
+def _intervals_to_bed(parser, fa, args, bed_path):
+    """--intervals: every line as --interval would run it (same rows, same exceptions), batched by
+    intervals.run_intervals on the first of --devices; one BED file, the lines' outputs concatenated in file order."""
+    from . import intervals
+    lines = read_bed_intervals(parser, args.intervals)
+    first_index = {}
+    for i, name in enumerate(fa.names):                                   # duplicate names: the first one (names.index)
+        first_index.setdefault(name, i)
+    for chrom, _, _ in lines:                                             # every line is checked before any scan
+        if chrom not in first_index:
+            parser.error(f"Chromosome {chrom} not found in the input FASTA file")
+    m = len(lines)
+    rec = np.array([first_index[c] for c, _, _ in lines], dtype=np.int64)
+    lengths = np.diff(fa.offsets.astype(np.int64))
+    a = np.array([s for _, s, _ in lines], dtype=np.int64)
+    b = np.minimum(np.array([e for _, _, e in lines], dtype=np.int64), lengths[rec])        # prf:139-140
+    device = parse_devices(getattr(args, "devices", None))[0]
+
+    def single(i):
+        return api.detect_repeats(fa.record(int(rec[i])).tobytes(), intervals._settings_for(args, int(a[i]), int(b[i])),
+                                  device=device)
+
+    planes = fa.packed() if fa.total_bases else _cabi.pack_ascii(b"").with_runs()
+    outcome, origin, iv, start, end, k = intervals.run_intervals(planes, fa.offsets.astype(np.int64)[rec], lengths[rec], a, b,
+                                                                 args, device, None, single)
+    for o in outcome:
+        if isinstance(o, BaseException):
+            raise o
+    counts = np.bincount(iv, minlength=m)
+    start, end = start + origin[iv], end + origin[iv]                     # record coordinates, 64-bit
+    extra = [(i, o) for i, o in enumerate(outcome) if o]                 # rows of the intervals done one by one
+    if extra:
+        for i, rows in extra:
+            origin[i] = rows[0][0]
+            counts[i] = len(rows)
+        iv = np.concatenate([iv] + [np.full(len(rows), i, np.int64) for i, rows in extra])
+        start = np.concatenate([start] + [np.array([r[0] for r in rows], np.int64) for _, rows in extra])
+        end = np.concatenate([end] + [np.array([r[1] for r in rows], np.int64) for _, rows in extra])
+        k = np.concatenate([k] + [np.array([len(r[2]) for r in rows], np.int64) for _, rows in extra])
+        order = np.argsort(iv, kind="stable")
+        iv, start, end, k = iv[order], start[order], end[order], k[order]
+    # The writer takes 32-bit start / end relative to a 64-bit origin per writer record.  A row of a batched interval lies
+    # in a prefix that fits one load, but an interval of the single-interval path may cover a whole record longer than
+    # 2^32 bases: an interval's rows are cut into writer records at every 2^31 bases past its origin (in row order, so
+    # the file order is unchanged), which keeps start and end below 2^32 for every run shorter than 2^31 bases.
+    if (end - start >= 1 << 31).any():
+        raise NotImplementedError("--intervals: a repeat of 2^31 bases or more cannot be written")
+    chunk = (start - origin[iv]) >> 31
+    new = np.ones(iv.size, dtype=bool)
+    new[1:] = (iv[1:] != iv[:-1]) | (chunk[1:] != chunk[:-1])
+    wrec = np.cumsum(new) - 1
+    first = np.flatnonzero(new)
+    w_iv = iv[first]
+    w_origin = origin[w_iv] + (chunk[first] << 31)
+    _cabi.write_rows(bed_path, [lines[i][0] for i in w_iv.tolist()], fa.bases, fa.offsets.astype(np.int64)[rec[w_iv]] + w_origin,
+                     wrec, start - w_origin[wrec], end - w_origin[wrec], k, origin=w_origin.astype(np.uint64))
+    for lo in range(0, m, 65536):                                         # the two lines of --interval, per line, batched
+        sys.stdout.write("".join(f"Processing {c_} ({e_ - s_:,d} bp)\nFound {n_:,d} repeats\n"
+                                 for (c_, s_, _), e_, n_ in zip(lines[lo:lo + 65536], b[lo:lo + 65536].tolist(),
+                                                                 counts[lo:lo + 65536].tolist())))
+
+
 def _run_fasta(parser, args):
     if not args.output_prefix:
         args.output_prefix = re.sub(".fa(sta)?(.gz)?", "", args.input_sequence)   # the (unanchored) regex of prf:114
     bed_path = f"{os.path.basename(args.output_prefix)}.bed"                       # always in the working directory
+    if args.intervals and args.interval:
+        parser.error("--intervals and --interval cannot be used together")
     # (page-locked planes only: the planes are what is uploaded, the text stays on the host for the motif column)
     with fasta.open_fasta(args.input_sequence, pinned=2) as fa:
-        if args.interval:
+        if args.intervals:
+            _intervals_to_bed(parser, fa, args, bed_path)
+        elif args.interval:
             fields = re.split("[:-]", args.interval)
             if len(fields) != 3:
                 parser.error("Invalid --interval format. Must be chrom:start_0based-end")
@@ -197,6 +284,8 @@ def _run_fasta(parser, args):
 def _run_raw(parser, args):
     if args.interval:
         parser.error("The --interval option is only supported for FASTA files.")
+    if args.intervals:
+        parser.error("The --intervals option is only supported for FASTA files.")
     if not args.output_prefix:
         args.output_prefix = "repeats"
     tsv_path = f"{args.output_prefix}.tsv"

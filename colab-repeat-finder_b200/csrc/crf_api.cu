@@ -23,6 +23,7 @@
 #include "crf_aux.cuh"
 #include "crf_scan.cuh"
 #include "crf_scan_warp.cuh"
+#include "crf_stop.cuh"
 #include "crf_xchg.cuh"
 
 using namespace crf;
@@ -1457,6 +1458,55 @@ extern "C" int crf_run_end(crf_seq *s, uint32_t record, uint32_t pos, uint32_t k
     return CRF_OK;
 }
 
+extern "C" int crf_interval_stop(crf_seq *s, uint32_t min_motif_size, uint32_t max_motif_size, const uint64_t *end_pos,
+                                 const uint64_t *full_len, int64_t *stop) {
+    if (!s) { set_err("crf_interval_stop: null sequence"); return CRF_ERR_ARG; }
+    if (min_motif_size < 1 || max_motif_size < min_motif_size || max_motif_size > s->cap) {
+        set_err("crf_interval_stop: motif sizes [%u, %u] not inside [1, max_motif_cap %u]", min_motif_size, max_motif_size, s->cap);
+        return CRF_ERR_ARG;
+    }
+    const uint32_t n = s->n_records;
+    if (!n) return CRF_OK;
+    if (!end_pos || !full_len || !stop) { set_err("crf_interval_stop: null argument"); return CRF_ERR_ARG; }
+    const size_t per_warp = (size_t)(max_motif_size - min_motif_size + 1) * sizeof(uint32_t);
+    uint32_t warps = STOP_WARPS;
+    while (warps > 1 && warps * per_warp > (48u << 10)) warps /= 2;
+    const size_t smem = warps * per_warp;
+    if (smem > (227u << 10)) {
+        set_err("crf_interval_stop: %u motif sizes need more shared memory than a block has", max_motif_size - min_motif_size + 1);
+        return CRF_ERR_UNSUPPORTED;
+    }
+    crf_ctx *c = s->ctx;
+    CU(cudaSetDevice(c->device));
+    g_ctx = c;
+    cudaStream_t st = c->stream;
+    if (smem > (48u << 10)) CU(cudaFuncSetAttribute(interval_stop_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    uint64_t *d_buf = nullptr;                            // end_pos | full_len | stop
+    CHECK(dev_alloc(&d_buf, 3 * (size_t)n));
+    StopParams p = {};
+    p.H = s->H; p.L = s->L; p.NM = s->NM; p.X = s->X;
+    p.ex_key = s->ex_key; p.n_exotic = s->n_exotic;
+    p.rec_dev_off = s->d_rec_dev_off; p.rec_len = s->d_rec_len; p.n_records = n;
+    p.kmin = min_motif_size; p.kmax = max_motif_size;
+    p.end_pos = d_buf; p.full_len = d_buf + n; p.stop = reinterpret_cast<int64_t *>(d_buf + 2 * (size_t)n);
+    cudaError_t e = cudaMemcpyAsync(d_buf, end_pos, (size_t)n * 8, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_buf + n, full_len, (size_t)n * 8, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) {
+        interval_stop_kernel<<<(n + warps - 1) / warps, 32 * warps, smem, st>>>(p);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(stop, p.stop, (size_t)n * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    dev_free(d_buf);
+    if (e != cudaSuccess) { set_err("crf_interval_stop: %s", cudaGetErrorString(e)); return CRF_ERR_CUDA; }
+    for (uint32_t r = 0; r < n; ++r)
+        if (stop[r] == STOP_BAD_ARG) {
+            set_err("crf_interval_stop: record %u of the load is longer than its full_len %llu", r, (unsigned long long)full_len[r]);
+            return CRF_ERR_ARG;
+        }
+    return CRF_OK;
+}
+
 // ---- multi-GPU gather over peer memory (crf_xchg.cuh) ---------------------------------------------
 static const size_t XCHG_ROWS_OFFSET = (sizeof(XchgBlock) + 255) & ~(size_t)255;
 static const uint32_t XCHG_RING = 64;
@@ -1791,6 +1841,7 @@ static cudaError_t preload_kernels() {
     if (e == cudaSuccess) e = preload(bitonic_step_kernel);
     if (e == cudaSuccess) e = preload(fill_u64_kernel);
     if (e == cudaSuccess) e = preload(run_end_kernel);
+    if (e == cudaSuccess) e = preload(interval_stop_kernel);
     if (e == cudaSuccess) e = preload(publish_kernel);
     if (e == cudaSuccess) e = preload(push_kernel);
     if (e == cudaSuccess) e = preload(settle_kernel);

@@ -202,6 +202,22 @@ int crf_patch_end(crf_seq *seq, uint64_t row, uint32_t new_end);
  * Used to stitch runs that leave a partition (chunk/GPU) -- see DESIGN.md "multi-GPU". */
 int crf_run_end(crf_seq *seq, uint32_t record, uint32_t pos, uint32_t k, uint32_t *run_end);
 
+/* Interval mode, for every record r of the load: record r is the prefix s_r[0 .. W_r) of a sequence s_r of full_len[r]
+ * bases (W_r = the record's loaded length).  stop[r] = the position T after which the reference's lock-step loop breaks
+ * (prf:70-74: the first t > end_pos[r] at which no tracker k in [min_motif_size, max_motif_size] is mid-repeat; tracker k
+ * is mid-repeat at t iff the k compares of M_k ending at min(t, full_len[r] - k - 1) are all matches),
+ * CRF_STOP_TO_END (-1) if the loop runs to the end of s_r (end_pos[r] >= full_len[r] - 1 included), CRF_STOP_UNDECIDED
+ * (-2) if W_r < full_len[r] and every t the loaded prefix can decide (t <= W_r - 1 - max_motif_size) is covered: load a
+ * longer prefix and ask again.  T is relative to the record.  One warp per record walks from just before end_pos[r] + 1
+ * to T, one 32-base word per step: a repeat that straddles end_pos costs a walk over its length.  CRF_ERR_ARG if some
+ * W_r > full_len[r] or max_motif_size exceeds the load's max_motif_cap; CRF_ERR_UNSUPPORTED above ~58 000 motif sizes.
+ * end_pos, full_len, stop: host arrays of n_records entries.  One stream sync.  crf_b200/intervals.py scans many intervals
+ * of one sequence in one load with it (DESIGN.md section 6, "Many intervals"). */
+#define CRF_STOP_TO_END (-1)
+#define CRF_STOP_UNDECIDED (-2)
+int crf_interval_stop(crf_seq *seq, uint32_t min_motif_size, uint32_t max_motif_size, const uint64_t *end_pos,
+                      const uint64_t *full_len, int64_t *stop);
+
 /* ---- multi-GPU: gathering the compacted rows of N GPUs on rank 0 over NVLink peer memory -----------------
  * The reference scales out by fanning `--interval` jobs over CPU workers and concatenating their BED files
  * (hail_batch_pipeline/run_hail_batch_pipeline.py:76-77, 115-123, 153).  Here each rank (one GPU: one process

@@ -9,6 +9,7 @@ if _PKG_PARENT not in sys.path:
     sys.path.insert(0, _PKG_PARENT)
 
 from crf_b200.api import detect_repeats  # noqa: E402,F401
+from crf_b200.intervals import detect_repeats_intervals  # noqa: E402,F401
 
 
 def main(argv=None):
