@@ -20,6 +20,9 @@ SCAN_TWO_STRIPS = 8
 
 CRF_OK, CRF_ERR_CUDA, CRF_ERR_ARG, CRF_ERR_NOMEM, CRF_ERR_UNSUPPORTED, CRF_ERR_CAPACITY, CRF_ERR_IO = range(7)
 STOP_TO_END, STOP_UNDECIDED = -1, -2          # crf_interval_stop
+#: most motif sizes (max - min + 1) crf_interval_stop takes: one uint32 of shared memory each, 227 KB per block; it refuses
+#: more with CRF_ERR_UNSUPPORTED
+STOP_MAX_MOTIF_SIZES = (227 << 10) // 4
 
 #: every symbol include/crf.h declares (tests check the library exports all of them)
 EXPORTS = [

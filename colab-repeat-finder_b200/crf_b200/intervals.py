@@ -127,7 +127,8 @@ def _settings_for(filter_settings, a, b):
 def run_intervals(planes, base, n, a, b, filter_settings, device=None, knobs=None, single=None, load_limit=None):
     """Interval mode for intervals [a_i, b_i) of records of n_i bases that start at source position base_i of `planes`.
     single(i) runs interval i through api.detect_repeats and returns its rows as (start, end, motif) tuples; it is used
-    for min_repeats == 1, a >= b, negative coordinates, b > n, and intervals whose prefix alone outgrows one load.
+    for min_repeats == 1, more motif sizes than crf_interval_stop takes, a >= b, negative coordinates, b > n, and intervals
+    whose prefix alone outgrows one load.
     Returns (outcome, a', iv, start, end, k): outcome[i] = None (rows in the columns; start / end relative to a'_i),
     a list of tuples (from single), or the exception interval i raises."""
     kmin, kmax = int(filter_settings.min_motif_size), int(filter_settings.max_motif_size)
@@ -137,7 +138,7 @@ def run_intervals(planes, base, n, a, b, filter_settings, device=None, knobs=Non
     m = a.size
     outcome = [None] * m
     batched = (a >= 0) & (b >= 0) & (a < b) & (b <= n)
-    if min_repeats == 1:
+    if min_repeats == 1 or kmax - kmin + 1 > _cabi.STOP_MAX_MOTIF_SIZES:
         batched[:] = False
     bi = np.flatnonzero(batched)
     a2, b2, lt = n_trim(*n_runs(planes), base[bi], a[bi], b[bi], n[bi]) if bi.size else (np.zeros(0, np.int64),) * 3
