@@ -96,14 +96,14 @@ def group_records(lengths, max_motif_size, limit=None):
     """Cut the record list into consecutive groups that each fit one device load: a load lays every record out
     as length + max_motif_size positions and holds at most crf_load_limit() of them (32-bit positions on the
     device).  A single record above the limit is its own group (its units are spread over several
-    loads, see _whole_fasta_to_bed).  Returns [(first, last)), ...]."""
+    loads, see _whole_fasta_to_bed).  Returns [(first, last)), ...].  One search per group, not a Python step per
+    record: a reads file has millions of them."""
     limit = _cabi.load_limit(max_motif_size) if limit is None else limit
-    groups, first, n = [], 0, len(lengths)
+    csum = np.cumsum(np.asarray(lengths, dtype=np.int64) + max_motif_size)
+    groups, first, n = [], 0, csum.size
     while first < n:
-        last, need = first, 0
-        while last < n and (last == first or need + int(lengths[last]) + max_motif_size <= limit):
-            need += int(lengths[last]) + max_motif_size
-            last += 1
+        before = int(csum[first - 1]) if first else 0
+        last = max(int(np.searchsorted(csum, before + limit, side="right")), first + 1)
         groups.append((first, last))
         first = last
     return groups
