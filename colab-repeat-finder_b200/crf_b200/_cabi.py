@@ -31,7 +31,7 @@ EXPORTS = [
     "crf_seq_load_packed_runs", "crf_seq_load_packed_runs_ranges", "crf_mask_runs",
     "crf_fasta_packed", "crf_seq_load_ascii", "crf_seq_load_ascii_ranges", "crf_seq_set_output_map", "crf_seq_destroy", "crf_seq_info", "crf_scan", "crf_fetch",
     "crf_scan_stats", "crf_run_end", "crf_interval_stop", "crf_fetch_open", "crf_patch_end", "crf_write_rows",
-    "crf_write_rows_at",
+    "crf_write_rows_at", "crf_mask_rows", "crf_write_fasta_masked",
     "crf_fasta_open", "crf_fasta_info", "crf_fasta_data", "crf_fasta_close", "crf_gunzip",
     "crf_xchg_create", "crf_xchg_destroy", "crf_xchg_export", "crf_xchg_connect_ipc", "crf_xchg_connect_local",
     "crf_xchg_set_timeout", "crf_xchg_set_compact", "crf_scan_gather", "crf_xchg_push", "crf_xchg_wait", "crf_xchg_step_result", "crf_xchg_fetch",
@@ -117,6 +117,8 @@ def lib():
         L.crf_patch_end.argtypes = [vp, u64, u32]
         L.crf_write_rows.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
         L.crf_write_rows_at.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
+        L.crf_mask_rows.argtypes = [vp, vp, vp, vp, u64, i, vp, u32, vp, u64, i]
+        L.crf_write_fasta_masked.argtypes = [ctypes.c_char_p, vp, vp, vp, u64, vp, i, u32, P(u64)]
         L.crf_fasta_open.argtypes = [ctypes.c_char_p, u32, i, P(vp)]
         L.crf_fasta_info.argtypes = [vp, P(u64), P(u64), P(i)]
         L.crf_fasta_data.argtypes = [vp, P(vp), P(vp), P(vp), P(u64)]
@@ -206,6 +208,28 @@ class Context:
         if offsets is None and ranges is None:
             offsets = np.array([0, planes.n_bases], dtype=np.uint64)
         return Sequence(self, None, offsets, max_motif_cap, False, ranges=ranges, packed=planes)
+
+    @_serialised
+    def mask_rows(self, record, start, end, dst_offset, mask_bits, n_rows=None, mask=None):
+        """crf_mask_rows: the union of the rows [dst_offset[record] + start, dst_offset[record] + end) as a bit mask.
+        record / start / end: host arrays, or device pointers (ints) with n_rows given.  dst_offset: host array, one
+        uint64 per record.  mask: None returns a new host uint32 array of ceil(mask_bits / 32) words; an int is a device
+        pointer to that many words, painted in place (returns None)."""
+        on_device = isinstance(record, int)
+        if on_device:
+            ptrs = [ctypes.c_void_p(int(a)) for a in (record, start, end)]
+        else:
+            cols = [np.ascontiguousarray(a, dtype=np.uint32) for a in (record, start, end)]
+            if not cols[0].shape == cols[1].shape == cols[2].shape or cols[0].ndim != 1:
+                raise ValueError("record, start and end must be 1-d arrays of equal size")
+            n_rows = cols[0].size
+            ptrs = [ctypes.c_void_p(a.ctypes.data) for a in cols]
+        dst = np.ascontiguousarray(dst_offset, dtype=np.uint64)
+        out = np.zeros((int(mask_bits) + 31) // 32, np.uint32) if mask is None else None
+        mptr = out.ctypes.data if out is not None else int(mask)
+        _check(lib().crf_mask_rows(self._h, *ptrs, int(n_rows), int(on_device), ctypes.c_void_p(dst.ctypes.data), dst.size,
+                                   ctypes.c_void_p(mptr), int(mask_bits), int(mask is not None)))
+        return out
 
     def close(self):
         if self._h:
@@ -671,4 +695,30 @@ def write_rows(path, names, bases, offsets, record, start, end, k, tsv=False, ap
     else:
         origin = np.ascontiguousarray(origin, dtype=np.uint64)
         _check(lib().crf_write_rows_at(*head, ctypes.c_void_p(origin.ctypes.data), *tail))
+    return nbytes.value
+
+
+def write_fasta_masked(path, names, bases, offsets, mask, hard=False, line_width=60):
+    """Native repeat-masked FASTA writer (crf_write_fasta_masked).  names: list of str or the NUL-separated blob; bases:
+    bytes or uint8 array with all records back to back, record r = bases[offsets[r]:offsets[r+1]]; mask: uint32 words,
+    bit p for bases[p] (Context.mask_rows).  hard: masked bases become N instead of lower case."""
+    blob = bytes(names) if isinstance(names, (bytes, bytearray)) else b"".join(n.encode("utf-8") + b"\0" for n in names)
+    offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+    if offsets.ndim != 1 or offsets.size < 1:
+        raise ValueError("offsets must hold n_records + 1 entries")
+    mask = np.ascontiguousarray(mask, dtype=np.uint32)
+    n = int(offsets[-1])
+    if isinstance(bases, np.ndarray):
+        if bases.dtype != np.uint8 or bases.ndim != 1 or not bases.flags.c_contiguous:
+            raise ValueError("bases must be a 1-d C-contiguous uint8 array")
+        bptr, size = bases.ctypes.data, bases.size
+    else:
+        bptr, size = ctypes.cast(ctypes.c_char_p(bases), ctypes.c_void_p).value or 0, len(bases)
+    if n > size or 32 * mask.size < n:
+        raise ValueError(f"offsets reach base {n}; bases hold {size} and the mask {32 * mask.size}")
+    nbytes = ctypes.c_uint64()
+    _check(lib().crf_write_fasta_masked(os.fsencode(path), ctypes.cast(ctypes.c_char_p(blob), ctypes.c_void_p),
+                                        ctypes.c_void_p(bptr), ctypes.c_void_p(offsets.ctypes.data), offsets.size - 1,
+                                        ctypes.c_void_p(mask.ctypes.data), int(bool(hard)), int(line_width),
+                                        ctypes.byref(nbytes)))
     return nbytes.value

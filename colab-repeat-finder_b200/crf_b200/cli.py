@@ -47,6 +47,9 @@ _OTHER_OPTIONS = [
                           help="GPUs for whole-FASTA runs, e.g. 0-7 or 0,2,3 (default: $CRF_DEVICES, else one GPU). "
                                "The records are cut into chunks, every GPU scans its share and the rows are gathered on "
                                "the first one over NVLink; the BED file is identical to a single-GPU run.")),
+    (("--mask",), dict(choices=("soft", "hard"), help="Also write <basename(prefix)>.masked.fa (FASTA input only, not with "
+                                                      "--interval / --intervals): the records with every base inside a "
+                                                      "reported repeat lower-cased (soft) or replaced by N (hard).")),
 ]
 
 
@@ -109,10 +112,11 @@ def group_records(lengths, max_motif_size, limit=None):
     return groups
 
 
-def _whole_fasta_to_bed(fa, args, bed_path):
+def _whole_fasta_to_bed(fa, args, bed_path, mask_rows=None):
     """Every record of the file: as few loads as the position limit allows (one for a human genome), one scan per
     load (on one GPU, or split over --devices), native row writer.  The groups are slices of the reader's buffer (no
-    copies on the Python side).  Returns the row count per record."""
+    copies on the Python side).  Returns the row count per record.  mask_rows: a list that gets the rows of every write
+    (see _paint_mask)."""
     devices = parse_devices(getattr(args, "devices", None))
     lengths = np.diff(fa.offsets.astype(np.int64))
     counts = np.zeros(fa.n_records, dtype=np.int64)
@@ -138,6 +142,8 @@ def _whole_fasta_to_bed(fa, args, bed_path):
             origin = np.array([u.d0 for u in units], dtype=np.uint64)
             names = [fa.names[first + r] for r in rec_of.tolist()]
             _cabi.write_rows(bed_path, names, blob, offsets[rec_of] + origin, unit, start, end, k, append=True, origin=origin)
+            if mask_rows is not None:                              # unit-relative rows: the unit's origin goes to dst
+                mask_rows.append((unit, start, end, fa.offsets[first + rec_of] + origin))
             counts[first:last] += np.bincount(rec_of[unit.astype(np.int64)], minlength=last - first)
             continue
         if total:
@@ -155,8 +161,22 @@ def _whole_fasta_to_bed(fa, args, bed_path):
             whole_file = first == 0 and last == fa.n_records          # the usual case: hand the name table over as it is
             _cabi.write_rows(bed_path, fa.names_blob if whole_file else fa.names[first:last], blob, offsets, rec, start,
                              end, k, append=True)
+            if mask_rows is not None:
+                mask_rows.append((rec, start, end, fa.offsets[first:last]))
             counts[first:last] += np.bincount(rec.astype(np.int64, copy=False), minlength=last - first)
     return counts
+
+
+def _paint_mask(ctx, mask_rows, n_bases):
+    """One crf_mask_rows call for the rows of a whole file.  mask_rows: (record, start, end, dst) parts, each numbering its
+    own records, dst[r] = where record r of the part starts in the file's bases.  Returns the mask words."""
+    parts = [(np.zeros(0, np.uint32),) * 3 + (np.zeros(0, np.uint64),)] + mask_rows
+    rec, n_dst = [], 0
+    for r, _, _, d in parts:
+        rec.append(np.asarray(r, dtype=np.int64) + n_dst)
+        n_dst += len(d)
+    start, end, dst = (np.concatenate([p[j] for p in parts]) for j in (1, 2, 3))
+    return ctx.mask_rows(np.concatenate(rec), start, end, dst.astype(np.uint64), n_bases)
 
 
 def read_bed_intervals(parser, path):
@@ -243,6 +263,10 @@ def _run_fasta(parser, args):
     bed_path = f"{os.path.basename(args.output_prefix)}.bed"                       # always in the working directory
     if args.intervals and args.interval:
         parser.error("--intervals and --interval cannot be used together")
+    if args.mask and (args.interval or args.intervals):
+        parser.error("--mask writes whole records: it cannot be used with --interval or --intervals")
+    mask_path = f"{os.path.basename(args.output_prefix)}.masked.fa" if args.mask else None
+    mask_rows = [] if args.mask else None
     # (page-locked planes only: the planes are what is uploaded, the text stays on the host for the motif column)
     with fasta.open_fasta(args.input_sequence, pinned=2) as fa:
         if args.intervals:
@@ -270,15 +294,24 @@ def _run_fasta(parser, args):
                     rows = api.detect_repeats(fa.record(i).tobytes(), args)
                     print(f"Found {len(rows):,d} repeats")
                     bed_file.write("".join(f"{name}\t{s}\t{e}\t{m}\n" for s, e, m in rows))
+                    if mask_rows is not None and rows:             # one mask record per row: 64-bit starts go to dst
+                        s = np.array([r[0] for r in rows], dtype=np.uint64)
+                        e = np.array([r[1] for r in rows], dtype=np.uint64)
+                        mask_rows.append((np.arange(len(rows)), np.zeros(len(rows), np.uint32), e - s, fa.offsets[i] + s))
         else:
-            counts = _whole_fasta_to_bed(fa, args, bed_path)
+            counts = _whole_fasta_to_bed(fa, args, bed_path, mask_rows)
             lengths = np.diff(fa.offsets.astype(np.int64))
             names, lengths, counts = fa.names, lengths.tolist(), counts.tolist()
             for lo in range(0, len(names), 65536):            # the reference's two lines per record; batched, a reads
                 sys.stdout.write("".join(                     # file has millions of records
                     f"Processing {n_} ({l_:,d} bp)\nFound {c_:,d} repeats\n"
                     for n_, l_, c_ in zip(names[lo:lo + 65536], lengths[lo:lo + 65536], counts[lo:lo + 65536])))
+        if mask_rows is not None:                                  # every record has been scanned: paint once, write
+            words = _paint_mask(api.get_context(parse_devices(getattr(args, "devices", None))[0]), mask_rows, fa.total_bases)
+            _cabi.write_fasta_masked(mask_path, fa.names_blob, fa.bases, fa.offsets, words, hard=args.mask == "hard")
     print(f"Wrote results to {bed_path}")
+    if mask_path:
+        print(f"Wrote masked sequence to {mask_path}")
 
 
 def _run_raw(parser, args):
@@ -286,6 +319,8 @@ def _run_raw(parser, args):
         parser.error("The --interval option is only supported for FASTA files.")
     if args.intervals:
         parser.error("The --intervals option is only supported for FASTA files.")
+    if args.mask:
+        parser.error("The --mask option is only supported for FASTA files.")
     if not args.output_prefix:
         args.output_prefix = "repeats"
     tsv_path = f"{args.output_prefix}.tsv"

@@ -25,6 +25,7 @@
 #include "crf_scan_warp.cuh"
 #include "crf_stop.cuh"
 #include "crf_xchg.cuh"
+#include "crf_mask.cuh"
 
 using namespace crf;
 
@@ -1507,6 +1508,84 @@ extern "C" int crf_interval_stop(crf_seq *s, uint32_t min_motif_size, uint32_t m
     return CRF_OK;
 }
 
+// ---- per-base masks (crf_mask.cuh) ------------------------------------------------------------------
+static int mask_rows_impl(crf_ctx *c, const uint32_t *record, const uint32_t *start, const uint32_t *end, uint64_t n_rows,
+                          int rows_on_device, const uint64_t *dst_offset, uint32_t n_records, uint32_t *mask,
+                          uint64_t mask_bits, int mask_on_device, void **scratch) {
+    cudaStream_t st = c->stream;
+    const uint64_t n_words = (mask_bits + 31) / 32;
+    const uint64_t batch = std::min<uint64_t>(n_rows, MASK_BATCH_ROWS);
+    // scratch: queue counter, error flag | dst_offset | queue slots | device mask (host mask) | rows (host rows)
+    size_t off = 16;
+    const size_t at_dst = off;   off += (size_t)n_records * 8;
+    const size_t at_first = off; off += (size_t)batch * 8;
+    const size_t at_slot = off;  off += ((size_t)batch * 4 + 7) & ~(size_t)7;
+    const size_t at_mask = off;  if (!mask_on_device) off += (size_t)n_words * 4;
+    const size_t at_rows = off;  if (!rows_on_device) off += 3 * (size_t)n_rows * 4;
+    CU(ctx_malloc(scratch, off));
+    uint8_t *base = (uint8_t *)*scratch;
+    MaskParams p = {};
+    p.dst_offset = (const uint64_t *)(base + at_dst);
+    p.n_records = n_records;
+    p.mask_bits = mask_bits;
+    p.mask = mask_on_device ? mask : (uint32_t *)(base + at_mask);
+    p.queue_ctr = (unsigned long long *)base;
+    p.err = (uint32_t *)(base + 8);
+    p.queue_first = (uint64_t *)(base + at_first);
+    p.queue_row = (uint32_t *)(base + at_slot);
+    if (!rows_on_device) {
+        uint32_t *rows = (uint32_t *)(base + at_rows);
+        CU(cudaMemcpyAsync(rows, record, n_rows * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(rows + n_rows, start, n_rows * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(rows + 2 * n_rows, end, n_rows * 4, cudaMemcpyHostToDevice, st));
+        record = rows; start = rows + n_rows; end = rows + 2 * n_rows;
+    }
+    if (n_records) CU(cudaMemcpyAsync((void *)p.dst_offset, dst_offset, (size_t)n_records * 8, cudaMemcpyHostToDevice, st));
+    CU(cudaMemsetAsync(base + 8, 0, 8, st));
+    CU(cudaMemsetAsync(p.mask, 0, n_words * 4, st));
+    int sms = 0;
+    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
+    for (uint64_t first = 0; first < n_rows; first += MASK_BATCH_ROWS) {
+        p.n_rows = (uint32_t)std::min<uint64_t>(MASK_BATCH_ROWS, n_rows - first);
+        p.record = record + first; p.start = start + first; p.end = end + first;
+        CU(cudaMemsetAsync(p.queue_ctr, 0, 8, st));
+        mask_rows_kernel<<<(p.n_rows + 255) / 256, 256, 0, st>>>(p);
+        mask_long_rows_kernel<<<8 * sms, 256, 0, st>>>(p);
+        CU(cudaGetLastError());
+    }
+    uint32_t err = 0;
+    CU(cudaMemcpyAsync(&err, p.err, 4, cudaMemcpyDeviceToHost, st));
+    if (!mask_on_device) CU(cudaMemcpyAsync(mask, p.mask, n_words * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (err) {
+        set_err("crf_mask_rows: %s", err & MASK_ERR_ORDER ? "a row ends before it starts"
+                                     : err & MASK_ERR_RECORD ? "a row's record is not below n_records"
+                                                             : "a row reaches past mask_bits");
+        return CRF_ERR_ARG;
+    }
+    return CRF_OK;
+}
+
+extern "C" int crf_mask_rows(crf_ctx *c, const uint32_t *record, const uint32_t *start, const uint32_t *end, uint64_t n_rows,
+                             int rows_on_device, const uint64_t *dst_offset, uint32_t n_records, uint32_t *mask,
+                             uint64_t mask_bits, int mask_on_device) {
+    if (!c) { set_err("crf_mask_rows: null context"); return CRF_ERR_ARG; }
+    if ((n_rows && (!record || !start || !end)) || (n_records && !dst_offset) || (mask_bits && !mask)) {
+        set_err("crf_mask_rows: null argument");
+        return CRF_ERR_ARG;
+    }
+    if (mask_bits > (1ull << 62)) { set_err("crf_mask_rows: mask_bits %llu too large", (unsigned long long)mask_bits); return CRF_ERR_ARG; }
+    if (!mask_bits && !n_rows) return CRF_OK;
+    CU(cudaSetDevice(c->device));
+    g_ctx = c;
+    void *scratch = nullptr;
+    const int rc = mask_rows_impl(c, record, start, end, n_rows, rows_on_device, dst_offset, n_records, mask, mask_bits,
+                                  mask_on_device, &scratch);
+    if (rc == CRF_ERR_CUDA) cudaStreamSynchronize(c->stream);   // nothing queued may still use the block when it is handed out again
+    ctx_free(scratch);
+    return rc;
+}
+
 // ---- multi-GPU gather over peer memory (crf_xchg.cuh) ---------------------------------------------
 static const size_t XCHG_ROWS_OFFSET = (sizeof(XchgBlock) + 255) & ~(size_t)255;
 static const uint32_t XCHG_RING = 64;
@@ -1847,10 +1926,13 @@ static cudaError_t preload_kernels() {
     if (e == cudaSuccess) e = preload(settle_kernel);
     if (e == cudaSuccess) e = preload(patch_rows_kernel);
     if (e == cudaSuccess) e = preload(unpack_kernel);
+    if (e == cudaSuccess) e = preload(mask_rows_kernel);
+    if (e == cudaSuccess) e = preload(mask_long_rows_kernel);
     return e;
 }
 
 #include "crf_rows.h"
+#include "crf_fasta_out.h"
 
 #include "crf_fasta.h"
 #include "crf_pack.h"

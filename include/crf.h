@@ -277,6 +277,20 @@ int crf_xchg_fetch(crf_xchg *xchg, uint32_t *record, uint32_t *start, uint32_t *
 /* Rank 0: overwrite the end of gathered rows (global row numbers) -- stitched open-ended runs. */
 int crf_xchg_patch_end(crf_xchg *xchg, const uint64_t *rows, const uint32_t *new_end, uint32_t n);
 
+/* ---- per-base masks --------------------------------------------------------------------------
+ * Sets mask to exactly the union over i < n_rows of the bits
+ *   [dst_offset[record[i]] + start[i], dst_offset[record[i]] + end[i])
+ * (bit p & 31 of word p >> 5; mask holds ceil(mask_bits / 32) words, written in full, every bit no row covers cleared).
+ * Rows may overlap and come in any order: the union of a scan's rows is its repeat mask (crf_b200/mask.py), with
+ * dst_offset = where each record (or unit of a record longer than one load, crf_load_limit) starts in the mask.
+ * dst_offset: host array of n_records uint64 values, so a destination may lie above 2^32.
+ * rows_on_device / mask_on_device select device or host pointers for record / start / end and for mask.
+ * A row with end < start, record >= n_records, or a range past mask_bits gives CRF_ERR_ARG (the mask is then
+ * unspecified).  One stream sync. */
+int crf_mask_rows(crf_ctx *ctx, const uint32_t *record, const uint32_t *start, const uint32_t *end, uint64_t n_rows,
+                  int rows_on_device, const uint64_t *dst_offset, uint32_t n_records,
+                  uint32_t *mask, uint64_t mask_bits, int mask_on_device);
+
 /* ---- output (host only, no GPU) -------------------------------------------------------------
  * Writes result rows as text, replacing the per-row Python of prf:148-149 (BED: chrom, start, end, motif) and
  * prf:166-170 (TSV: start_0based, end, motif, with header).  names = NUL-separated record names in record
@@ -291,6 +305,13 @@ int crf_write_rows(const char *path, int append, int tsv, const char *names, con
 int crf_write_rows_at(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
                       const uint64_t *offsets, const uint64_t *origin, const uint32_t *record, const uint32_t *start,
                       const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes);
+/* A repeat-masked FASTA file: per record a header line ">name" (names NUL-separated, as crf_write_rows takes them), then
+ * its bases, line_width per line.  Mask bit p (as crf_mask_rows lays it out) stands for bases[p], with the indexing of
+ * offsets (record r = bases[offsets[r] .. offsets[r+1])).  A masked byte is lower-cased when it is an ASCII letter A-Z
+ * (hard == 0: soft masking) or becomes 'N' (hard != 0); every other byte is written as it is.  Formatted on up to 16
+ * threads.  *bytes = bytes written; a short write is CRF_ERR_IO. */
+int crf_write_fasta_masked(const char *path, const char *names, const uint8_t *bases, const uint64_t *offsets,
+                           uint64_t n_records, const uint32_t *mask, int hard, uint32_t line_width, uint64_t *bytes);
 
 /* ---- input (host only, no GPU) ---------------------------------------------------------------
  * Native FASTA ingest, replacing what the reference takes from pyfastx (prf:117-137: the records in file

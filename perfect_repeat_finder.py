@@ -11,6 +11,7 @@ if _PKG_PARENT not in sys.path:
 from crf_b200.api import detect_repeats  # noqa: E402,F401
 from crf_b200.intervals import detect_repeats_intervals  # noqa: E402,F401
 from crf_b200.batch import detect_repeats_batch, scan_batch  # noqa: E402,F401
+from crf_b200.mask import repeat_mask  # noqa: E402,F401
 
 
 def main(argv=None):
