@@ -31,8 +31,9 @@ EXPORTS = [
     "crf_seq_load_packed_runs", "crf_seq_load_packed_runs_ranges", "crf_mask_runs",
     "crf_fasta_packed", "crf_seq_load_ascii", "crf_seq_load_ascii_ranges", "crf_seq_set_output_map", "crf_seq_destroy", "crf_seq_info", "crf_scan", "crf_fetch",
     "crf_scan_stats", "crf_run_end", "crf_interval_stop", "crf_fetch_open", "crf_patch_end", "crf_write_rows",
-    "crf_write_rows_at", "crf_mask_rows", "crf_write_fasta_masked",
-    "crf_fasta_open", "crf_fasta_info", "crf_fasta_data", "crf_fasta_close", "crf_gunzip",
+    "crf_write_rows_at", "crf_mask_rows", "crf_write_fasta_masked", "crf_write_fastq_masked",
+    "crf_fasta_open", "crf_fasta_info", "crf_fasta_data", "crf_fasta_format", "crf_fasta_quals", "crf_fasta_close",
+    "crf_gunzip",
     "crf_xchg_create", "crf_xchg_destroy", "crf_xchg_export", "crf_xchg_connect_ipc", "crf_xchg_connect_local",
     "crf_xchg_set_timeout", "crf_xchg_set_compact", "crf_scan_gather", "crf_xchg_push", "crf_xchg_wait", "crf_xchg_step_result", "crf_xchg_fetch",
     "crf_xchg_patch_end",
@@ -119,9 +120,12 @@ def lib():
         L.crf_write_rows_at.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
         L.crf_mask_rows.argtypes = [vp, vp, vp, vp, u64, i, vp, u32, vp, u64, i]
         L.crf_write_fasta_masked.argtypes = [ctypes.c_char_p, vp, vp, vp, u64, vp, i, u32, P(u64)]
+        L.crf_write_fastq_masked.argtypes = [ctypes.c_char_p, vp, vp, vp, vp, u64, vp, i, P(u64)]
         L.crf_fasta_open.argtypes = [ctypes.c_char_p, u32, i, P(vp)]
         L.crf_fasta_info.argtypes = [vp, P(u64), P(u64), P(i)]
         L.crf_fasta_data.argtypes = [vp, P(vp), P(vp), P(vp), P(u64)]
+        L.crf_fasta_format.argtypes = [vp, P(i)]
+        L.crf_fasta_quals.argtypes = [vp, P(vp)]
         L.crf_fasta_close.argtypes = [vp]
         L.crf_gunzip.argtypes = [vp, ctypes.c_uint64, vp, ctypes.c_uint64, ctypes.POINTER(ctypes.c_uint64), ctypes.c_int]
         L.crf_xchg_create.argtypes = [vp, u32, u32, u64, P(vp)]
@@ -610,14 +614,17 @@ class Xchg:
 
 
 class Fasta:
-    """A FASTA file read by the native reader (crf_fasta_open): `bases` (uint8 view of all records back to
-    back, owned by the library until close()), `offsets` (n_records+1, uint64), `names` (list of str) and
-    `names_blob` (NUL-separated, as crf_write_rows takes them)."""
+    """A FASTA or FASTQ file read by the native reader (crf_fasta_open): `bases` (uint8 view of all records back to
+    back, owned by the library until close()), `offsets` (n_records+1, uint64), `names` (list of str),
+    `names_blob` (NUL-separated, as crf_write_rows takes them), `format` ("fasta" / "fastq") and `quals` (a FASTQ file's
+    qualities as a uint8 view laid out like `bases`, or None)."""
 
-    def __init__(self, path, n_threads=0, pinned=False):
-        """pinned: False / True (page-locked base buffer and planes) / 2 (page-locked planes only: the text stays pageable)."""
+    def __init__(self, path, n_threads=0, pinned=False, qualities=False):
+        """pinned: False / True (page-locked base buffer and planes) / 2 (page-locked planes only: the text stays pageable).
+        qualities: keep a FASTQ file's qualities (else they are checked and dropped: no host memory for them)."""
         self._h = ctypes.c_void_p()
-        _check(lib().crf_fasta_open(os.fsencode(path), n_threads, int(pinned), ctypes.byref(self._h)))
+        _check(lib().crf_fasta_open(os.fsencode(path), n_threads, int(pinned) | (4 if qualities else 0),
+                                    ctypes.byref(self._h)))
         n_rec, total, pin = ctypes.c_uint64(), ctypes.c_uint64(), ctypes.c_int()
         _check(lib().crf_fasta_info(self._h, ctypes.byref(n_rec), ctypes.byref(total), ctypes.byref(pin)))
         bases, offsets, names, nbytes = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_uint64()
@@ -630,6 +637,12 @@ class Fasta:
                                              shape=(self.n_records + 1,)).copy()
         self.names_blob = ctypes.string_at(names, nbytes.value) if nbytes.value else b""
         self._names = None
+        fmt, quals = ctypes.c_int(), ctypes.c_void_p()
+        _check(lib().crf_fasta_format(self._h, ctypes.byref(fmt)))
+        _check(lib().crf_fasta_quals(self._h, ctypes.byref(quals)))
+        self.format = "fastq" if fmt.value == 1 else "fasta"
+        self.quals = np.ctypeslib.as_array(ctypes.cast(quals, ctypes.POINTER(ctypes.c_uint8)),
+                                           shape=(max(self.total_bases, 1),))[:self.total_bases] if quals.value else None
 
     @property
     def names(self):
@@ -654,7 +667,7 @@ class Fasta:
 
     def close(self):
         if self._h:
-            self.bases = None
+            self.bases = self.quals = None
             lib().crf_fasta_close(self._h)
             self._h = ctypes.c_void_p()
 
@@ -698,27 +711,54 @@ def write_rows(path, names, bases, offsets, record, start, end, k, tsv=False, ap
     return nbytes.value
 
 
-def write_fasta_masked(path, names, bases, offsets, mask, hard=False, line_width=60):
-    """Native repeat-masked FASTA writer (crf_write_fasta_masked).  names: list of str or the NUL-separated blob; bases:
-    bytes or uint8 array with all records back to back, record r = bases[offsets[r]:offsets[r+1]]; mask: uint32 words,
-    bit p for bases[p] (Context.mask_rows).  hard: masked bases become N instead of lower case."""
+def _host_bytes(what, buf):
+    """(address, size) of bytes or a 1-d C-contiguous uint8 array."""
+    if isinstance(buf, np.ndarray):
+        if buf.dtype != np.uint8 or buf.ndim != 1 or not buf.flags.c_contiguous:
+            raise ValueError(f"{what} must be a 1-d C-contiguous uint8 array")
+        return buf.ctypes.data, buf.size
+    return ctypes.cast(ctypes.c_char_p(buf), ctypes.c_void_p).value or 0, len(buf)
+
+
+def _masked_args(names, bases, offsets, mask, quals=None):
+    """The checked arguments both masked writers take: names blob, bases address, offsets, mask (and quals address)."""
     blob = bytes(names) if isinstance(names, (bytes, bytearray)) else b"".join(n.encode("utf-8") + b"\0" for n in names)
     offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
     if offsets.ndim != 1 or offsets.size < 1:
         raise ValueError("offsets must hold n_records + 1 entries")
     mask = np.ascontiguousarray(mask, dtype=np.uint32)
     n = int(offsets[-1])
-    if isinstance(bases, np.ndarray):
-        if bases.dtype != np.uint8 or bases.ndim != 1 or not bases.flags.c_contiguous:
-            raise ValueError("bases must be a 1-d C-contiguous uint8 array")
-        bptr, size = bases.ctypes.data, bases.size
-    else:
-        bptr, size = ctypes.cast(ctypes.c_char_p(bases), ctypes.c_void_p).value or 0, len(bases)
+    bptr, size = _host_bytes("bases", bases)
     if n > size or 32 * mask.size < n:
         raise ValueError(f"offsets reach base {n}; bases hold {size} and the mask {32 * mask.size}")
+    qptr = None
+    if quals is not None:
+        qptr, qsize = _host_bytes("quals", quals)
+        if n > qsize:
+            raise ValueError(f"offsets reach base {n}; quals hold {qsize}")
+    return blob, bptr, offsets, mask, qptr
+
+
+def write_fasta_masked(path, names, bases, offsets, mask, hard=False, line_width=60):
+    """Native repeat-masked FASTA writer (crf_write_fasta_masked).  names: list of str or the NUL-separated blob; bases:
+    bytes or uint8 array with all records back to back, record r = bases[offsets[r]:offsets[r+1]]; mask: uint32 words,
+    bit p for bases[p] (Context.mask_rows).  hard: masked bases become N instead of lower case."""
+    blob, bptr, offsets, mask, _ = _masked_args(names, bases, offsets, mask)
     nbytes = ctypes.c_uint64()
     _check(lib().crf_write_fasta_masked(os.fsencode(path), ctypes.cast(ctypes.c_char_p(blob), ctypes.c_void_p),
                                         ctypes.c_void_p(bptr), ctypes.c_void_p(offsets.ctypes.data), offsets.size - 1,
                                         ctypes.c_void_p(mask.ctypes.data), int(bool(hard)), int(line_width),
+                                        ctypes.byref(nbytes)))
+    return nbytes.value
+
+
+def write_fastq_masked(path, names, bases, quals, offsets, mask, hard=False):
+    """Native repeat-masked FASTQ writer (crf_write_fastq_masked): as write_fasta_masked, with quals (bytes or uint8 array
+    laid out like bases, Fasta.quals) written unchanged on each record's quality line."""
+    blob, bptr, offsets, mask, qptr = _masked_args(names, bases, offsets, mask, quals)
+    nbytes = ctypes.c_uint64()
+    _check(lib().crf_write_fastq_masked(os.fsencode(path), ctypes.cast(ctypes.c_char_p(blob), ctypes.c_void_p),
+                                        ctypes.c_void_p(bptr), ctypes.c_void_p(qptr), ctypes.c_void_p(offsets.ctypes.data),
+                                        offsets.size - 1, ctypes.c_void_p(mask.ctypes.data), int(bool(hard)),
                                         ctypes.byref(nbytes)))
     return nbytes.value

@@ -3,7 +3,8 @@
 Same flags, defaults, stdout lines and output files as the reference's main()
 (the reference's perfect_repeat_finder.py:83-179), re-organised around two code paths:
 
-  FASTA file  -> <basename(prefix)>.bed in the working directory (chrom, start_0based, end, motif)
+  FASTA file  -> <basename(prefix)>.bed in the working directory (chrom, start_0based, end, motif); a FASTQ file is
+                 read the same way, its read names as chrom
   raw string  -> <prefix>.tsv with a header line (start_0based, end, motif)
 
 Deliberate deviations (SURVEY.md section 8b):
@@ -49,7 +50,8 @@ _OTHER_OPTIONS = [
                                "the first one over NVLink; the BED file is identical to a single-GPU run.")),
     (("--mask",), dict(choices=("soft", "hard"), help="Also write <basename(prefix)>.masked.fa (FASTA input only, not with "
                                                       "--interval / --intervals): the records with every base inside a "
-                                                      "reported repeat lower-cased (soft) or replaced by N (hard).")),
+                                                      "reported repeat lower-cased (soft) or replaced by N (hard).  For "
+                                                      "FASTQ input: <basename(prefix)>.masked.fq, qualities unchanged.")),
 ]
 
 
@@ -61,7 +63,7 @@ def build_parser():
         filters.add_argument(*flags, **kw)
     for flags, kw in _OTHER_OPTIONS:
         parser.add_argument(*flags, **kw)
-    parser.add_argument("input_sequence", help="A nucleotide string, or the path of a FASTA file (plain or .gz)")
+    parser.add_argument("input_sequence", help="A nucleotide string, or the path of a FASTA or FASTQ file (plain or .gz)")
     return parser
 
 
@@ -257,18 +259,28 @@ def _intervals_to_bed(parser, fa, args, bed_path):
                                                                  counts[lo:lo + 65536].tolist())))
 
 
+def default_prefix(path, fmt):
+    """The output prefix when -o is not given.  FASTA: the (unanchored) regex of prf:114, as the reference has it.  FASTQ:
+    the path without a trailing .fastq / .fq, optionally followed by .gz / .bgz (reads.fq.gz -> reads)."""
+    if fmt == "fastq":
+        return re.sub(r"\.(fastq|fq)(\.(gz|bgz))?$", "", path)
+    return re.sub(".fa(sta)?(.gz)?", "", path)
+
+
 def _run_fasta(parser, args):
-    if not args.output_prefix:
-        args.output_prefix = re.sub(".fa(sta)?(.gz)?", "", args.input_sequence)   # the (unanchored) regex of prf:114
-    bed_path = f"{os.path.basename(args.output_prefix)}.bed"                       # always in the working directory
     if args.intervals and args.interval:
         parser.error("--intervals and --interval cannot be used together")
     if args.mask and (args.interval or args.intervals):
         parser.error("--mask writes whole records: it cannot be used with --interval or --intervals")
-    mask_path = f"{os.path.basename(args.output_prefix)}.masked.fa" if args.mask else None
     mask_rows = [] if args.mask else None
-    # (page-locked planes only: the planes are what is uploaded, the text stays on the host for the motif column)
-    with fasta.open_fasta(args.input_sequence, pinned=2) as fa:
+    # (page-locked planes only: the planes are what is uploaded, the text stays on the host for the motif column; a FASTQ
+    # file's qualities are kept only for the masked FASTQ)
+    with fasta.open_fasta(args.input_sequence, pinned=2, qualities=bool(args.mask)) as fa:
+        if not args.output_prefix:                                                 # FASTA or FASTQ: known once it is read
+            args.output_prefix = default_prefix(args.input_sequence, fa.format)
+        bed_path = f"{os.path.basename(args.output_prefix)}.bed"                   # always in the working directory
+        mask_path = f"{os.path.basename(args.output_prefix)}.masked.{'fq' if fa.format == 'fastq' else 'fa'}" \
+            if args.mask else None
         if args.intervals:
             _intervals_to_bed(parser, fa, args, bed_path)
         elif args.interval:
@@ -308,7 +320,11 @@ def _run_fasta(parser, args):
                     for n_, l_, c_ in zip(names[lo:lo + 65536], lengths[lo:lo + 65536], counts[lo:lo + 65536])))
         if mask_rows is not None:                                  # every record has been scanned: paint once, write
             words = _paint_mask(api.get_context(parse_devices(getattr(args, "devices", None))[0]), mask_rows, fa.total_bases)
-            _cabi.write_fasta_masked(mask_path, fa.names_blob, fa.bases, fa.offsets, words, hard=args.mask == "hard")
+            if fa.format == "fastq":
+                _cabi.write_fastq_masked(mask_path, fa.names_blob, fa.bases, fa.quals, fa.offsets, words,
+                                         hard=args.mask == "hard")
+            else:
+                _cabi.write_fasta_masked(mask_path, fa.names_blob, fa.bases, fa.offsets, words, hard=args.mask == "hard")
     print(f"Wrote results to {bed_path}")
     if mask_path:
         print(f"Wrote masked sequence to {mask_path}")

@@ -1,6 +1,7 @@
 """FASTA input through the library's native reader (crf_fasta_open), standing in for pyfastx
 (perfect_repeat_finder.py:117-137 uses only `.name` -- the first whitespace-delimited token of the header --
-and `.seq`, the record's lines joined without line ends, case preserved).  Plain or gzip input."""
+and `.seq`, the record's lines joined without line ends, case preserved).  Plain or gzip input.  A FASTQ file (first
+byte that is not whitespace: '@') is read too: read names and sequences in the same layout, qualities on request."""
 import os
 
 from . import _cabi
@@ -14,14 +15,15 @@ class FastaRecord:
         self.seq = seq        # uint8 view into the file's base buffer, one byte per base, case preserved
 
 
-def open_fasta(path, pinned=False):
-    """The whole file as a _cabi.Fasta (bases back to back + offsets + names)."""
+def open_fasta(path, pinned=False, qualities=False):
+    """The whole file as a _cabi.Fasta (bases back to back + offsets + names; a FASTQ file's qualities in .quals when
+    `qualities`)."""
     if not os.path.isfile(path):
         raise FileNotFoundError(path)
-    return _cabi.Fasta(path, pinned=pinned)
+    return _cabi.Fasta(path, pinned=pinned, qualities=qualities)
 
 
 def read_fasta(path):
-    """All records of a FASTA file, in file order, as (name, bytes) records."""
+    """All records of a FASTA or FASTQ file, in file order, as (name, bytes) records."""
     with open_fasta(path) as fa:
         return [FastaRecord(name, fa.record(i).tobytes()) for i, name in enumerate(fa.names)]

@@ -1,4 +1,4 @@
-// Native FASTA ingest (host only): file -> one contiguous byte-per-base buffer + record table.
+// Native FASTA / FASTQ ingest (host only): file -> one contiguous byte-per-base buffer + record table.
 //
 // Stands in for what the reference takes from pyfastx (perfect_repeat_finder.py:117-137: iterate the records,
 // `.name` = first whitespace-delimited token of the header, `.seq` = the record's lines joined, case preserved).
@@ -34,6 +34,8 @@ struct crf_fasta {
     bool planes_pinned = false;
     bool want_pinned_planes = false;                     // crf_fasta_open(pinned & 3): page-lock the planes crf_fasta_packed makes
     std::vector<uint64_t> exotic;
+    int format = 0;                                      // 0 = FASTA, 1 = FASTQ
+    uint8_t *quals = nullptr;                            // FASTQ, crf_fasta_open(pinned & 4): laid out like bases
 };
 
 namespace fasta_detail {
@@ -242,6 +244,242 @@ static bool inflate_bgzf(const FileBytes &in, unsigned n_threads, crf_inflate::O
     return true;
 }
 
+static bool is_space(uint8_t c) { return c == ' ' || c == '\t' || c == '\r' || c == '\n' || c == '\v' || c == '\f'; }
+
+// The record name: the first whitespace-delimited token [*a, returned end) of the header text [*a, h1).
+static uint64_t name_token(const uint8_t *t, uint64_t *a, uint64_t h1) {
+    while (*a < h1 && is_space(t[*a])) ++*a;
+    uint64_t b = *a;
+    while (b < h1 && !is_space(t[b])) ++b;
+    return b;
+}
+
+// The base buffer: page-locked with pinned & 1 when a device is present, else plain pages (2 MB ones when large).
+static bool alloc_bases(crf_fasta *fa, uint64_t total, int pinned) {
+    const size_t alloc = std::max<uint64_t>(total, 1);
+    fa->want_pinned_planes = (pinned & 3) != 0;
+    if (pinned & 1) {
+        void *p = nullptr;
+        if (cudaHostAlloc(&p, alloc, cudaHostAllocDefault) == cudaSuccess) {
+            fa->bases = (uint8_t *)p;
+            fa->pinned = true;
+        } else {
+            cudaGetLastError();                         // no device / no pinned memory left: plain pages
+        }
+    }
+    if (!fa->bases) fa->bases = (uint8_t *)malloc(alloc);
+    if (!fa->bases) return false;
+#if defined(__linux__) && defined(MADV_HUGEPAGE)
+    if (!fa->pinned && alloc >= ((size_t)8 << 20)) {    // gigabytes touched for the first time by the compaction below: 2 MB pages
+        const uintptr_t lo = ((uintptr_t)fa->bases + 4095) & ~(uintptr_t)4095, hi = ((uintptr_t)fa->bases + alloc) & ~(uintptr_t)4095;
+        if (hi > lo) madvise((void *)lo, hi - lo, MADV_HUGEPAGE);              // (advice only; the block is never realloc'ed)
+    }
+#endif
+    return true;
+}
+
+// ---- FASTQ ----
+// A record is a header line '@name ...', sequence lines up to a line starting with '+' (the rest of that line is ignored),
+// then quality lines until they hold as many bytes as the sequence (which makes quality lines starting with '@' or '+'
+// unambiguous).  A line is its bytes up to '\n' or the end of the text, without one trailing '\r'.  Whitespace between
+// records is skipped.  Quality bytes are '!'..'~'.
+//
+// Threaded path: the text is cut into pieces; every piece but the first starts at its first line that begins with '@' and
+// whose line after next begins with '+', and parses 4-line records (header, one sequence line not starting with '+', '+'
+// line, quality line as long as the sequence) while they start inside the piece.  The result is taken only if every piece
+// parsed that way and starts exactly where the previous one's last record ended (the last one ending at the end of the
+// text); then it is what the general rules give.  Anything else goes to the serial parser of the general rules, the only
+// place that reports errors.
+
+struct Line { uint64_t a, b; };                         // content [a, b)
+
+static inline uint64_t next_line(const uint8_t *t, uint64_t n, uint64_t p, Line &ln) {
+    const uint8_t *e = (const uint8_t *)memchr(t + p, '\n', n - p);
+    const uint64_t end = e ? (uint64_t)(e - t) : n;
+    ln.a = p;
+    ln.b = end > p && t[end - 1] == '\r' ? end - 1 : end;
+    return e ? end + 1 : n;
+}
+
+static inline bool quality_bytes_ok(const uint8_t *q, uint64_t len) {
+    uint8_t bad = 0;
+    for (uint64_t i = 0; i < len; ++i) bad |= (uint8_t)(q[i] - '!') > ('~' - '!');
+    return !bad;
+}
+
+// What a parse pass does with the records it finds: count them, or write them into the handle.
+struct FastqCount {
+    uint64_t records = 0, bases = 0, name_bytes = 0;
+    void record(const uint8_t *t, uint64_t a, uint64_t h1) {
+        const uint64_t b = name_token(t, &a, h1);
+        ++records;
+        name_bytes += b - a + 1;
+    }
+    void seq(const uint8_t *, const Line &ln) { bases += ln.b - ln.a; }
+    void qual(const uint8_t *, const Line &) {}
+};
+
+struct FastqWrite {
+    crf_fasta *fa;
+    uint64_t rec, base, name, qbase;                    // cursors: record, base, name byte, quality byte
+    void record(const uint8_t *t, uint64_t a, uint64_t h1) {
+        const uint64_t e = name_token(t, &a, h1);
+        fa->offsets[rec] = base;
+        fa->name_off[rec++] = name;
+        memcpy(fa->names.data() + name, t + a, e - a);
+        name += e - a;
+        fa->names[name++] = '\0';
+    }
+    void seq(const uint8_t *t, const Line &ln) {
+        memcpy(fa->bases + base, t + ln.a, ln.b - ln.a);
+        base += ln.b - ln.a;
+    }
+    void qual(const uint8_t *t, const Line &ln) {
+        if (fa->quals) memcpy(fa->quals + qbase, t + ln.a, ln.b - ln.a);
+        qbase += ln.b - ln.a;
+    }
+};
+
+// 4-line records from p while they start before stop.  *end = where the last one ends.  false: a record without that shape.
+template <class Sink>
+static bool fastq_4line(const uint8_t *t, uint64_t n, uint64_t p, uint64_t stop, uint64_t *end, Sink &sink) {
+    while (p < stop) {
+        Line h, s, plus, q;
+        if (t[p] != '@') return false;
+        p = next_line(t, n, p, h);
+        if (p >= n) return false;
+        p = next_line(t, n, p, s);
+        if (p >= n || (s.b > s.a && t[s.a] == '+')) return false;
+        p = next_line(t, n, p, plus);
+        if (p >= n || t[plus.a] != '+') return false;
+        p = next_line(t, n, p, q);
+        if (q.b - q.a != s.b - s.a || !quality_bytes_ok(t + q.a, q.b - q.a)) return false;
+        sink.record(t, h.a + 1, h.b);
+        sink.seq(t, s);
+        sink.qual(t, q);
+    }
+    *end = p;
+    return true;
+}
+
+// The general rules, from p to the end of the text.  Returns 0, or the 1-based number of the record at fault with *why set.
+template <class Sink>
+static uint64_t fastq_serial(const uint8_t *t, uint64_t n, uint64_t p, Sink &sink, const char **why) {
+    for (uint64_t rec = 1;; ++rec) {
+        while (p < n && is_space(t[p])) ++p;
+        if (p == n) return 0;
+        if (t[p] != '@') { *why = "text that is not whitespace before its '@' header"; return rec; }
+        Line ln;
+        p = next_line(t, n, p, ln);
+        sink.record(t, ln.a + 1, ln.b);
+        uint64_t len = 0;
+        for (;;) {                                      // sequence lines up to the '+' line
+            if (p >= n) { *why = "the file ends inside the record"; return rec; }
+            p = next_line(t, n, p, ln);
+            if (ln.b > ln.a && t[ln.a] == '+') break;
+            sink.seq(t, ln);
+            len += ln.b - ln.a;
+        }
+        for (uint64_t got = 0; got < len;) {            // quality lines until they hold len bytes
+            if (p >= n) { *why = "the file ends inside the record"; return rec; }
+            p = next_line(t, n, p, ln);
+            if (got + (ln.b - ln.a) > len) { *why = "its quality is longer than its sequence"; return rec; }
+            if (!quality_bytes_ok(t + ln.a, ln.b - ln.a)) { *why = "a quality byte outside '!'..'~'"; return rec; }
+            sink.qual(t, ln);
+            got += ln.b - ln.a;
+        }
+    }
+}
+
+// The FASTQ text t[lead, n) (t[lead] == '@') into fa.  piece: bytes of text per piece of the threaded path.
+// *serial: whether the serial parser made the result.
+static int parse_fastq(const char *path, const uint8_t *t, uint64_t n, uint64_t lead, unsigned n_threads, uint64_t piece,
+                       int pinned, crf_fasta *fa, bool *serial) {
+    fa->format = 1;
+    const uint64_t n_pieces = (n - lead + piece - 1) / piece;
+    struct Part { uint64_t begin, end; FastqCount count; bool ok; };
+    std::vector<Part> parts(n_pieces);
+    run_parallel(n_threads, n_pieces, [&](size_t i) {
+        Part &pt = parts[i];
+        const uint64_t lo = lead + i * piece, hi = std::min(n, lo + piece);
+        pt.ok = false;
+        pt.begin = pt.end = hi;                         // (no record starts in the piece)
+        uint64_t p = lo;
+        if (i > 0) {                                    // the first line start at or after lo that looks like a header
+            if (t[p - 1] != '\n') {
+                const uint8_t *e = (const uint8_t *)memchr(t + p, '\n', n - p);
+                p = e ? (uint64_t)(e - t) + 1 : n;
+            }
+            for (; p < hi; ) {
+                Line l1, l2;
+                const uint64_t p1 = next_line(t, n, p, l1);
+                if (t[p] == '@' && p1 < n) {
+                    const uint64_t p2 = next_line(t, n, p1, l2);
+                    if (p2 < n && t[p2] == '+') break;
+                }
+                p = p1;
+            }
+            if (p >= hi) { pt.ok = true; return; }
+        }
+        pt.begin = p;
+        pt.ok = fastq_4line(t, n, p, hi, &pt.end, pt.count);
+    });
+    uint64_t at = lead;
+    bool chained = true;
+    for (const Part &pt : parts) {
+        if (!pt.ok) { chained = false; break; }
+        if (pt.count.records == 0) continue;            // no record starts in it (text skipped here breaks the chain later)
+        if (pt.begin != at) { chained = false; break; }
+        at = pt.end;
+    }
+    chained = chained && at == n;
+    *serial = !chained;
+
+    FastqCount total;
+    if (chained) {
+        for (const Part &pt : parts) {
+            total.records += pt.count.records;
+            total.bases += pt.count.bases;
+            total.name_bytes += pt.count.name_bytes;
+        }
+    } else {
+        const char *why = nullptr;
+        if (const uint64_t bad = fastq_serial(t, n, lead, total, &why)) {
+            set_err("crf_fasta_open: %s: FASTQ record %llu: %s", path, (unsigned long long)bad, why);
+            return CRF_ERR_ARG;
+        }
+    }
+    fa->offsets.assign(total.records + 1, 0);
+    fa->name_off.assign(total.records, 0);
+    fa->names.assign(total.name_bytes, 0);
+    fa->offsets[total.records] = fa->total = total.bases;
+    if (!alloc_bases(fa, total.bases, pinned) || ((pinned & 4) && !(fa->quals = (uint8_t *)malloc(std::max<uint64_t>(total.bases, 1))))) {
+        set_err("crf_fasta_open: out of host memory (%llu bases)", (unsigned long long)total.bases);
+        return CRF_ERR_NOMEM;
+    }
+    if (chained) {
+        std::vector<FastqWrite> sinks(n_pieces, FastqWrite{fa, 0, 0, 0, 0});
+        FastqWrite cur{fa, 0, 0, 0, 0};
+        for (uint64_t i = 0; i < n_pieces; ++i) {
+            sinks[i] = cur;
+            sinks[i].qbase = cur.base;
+            cur.rec += parts[i].count.records;
+            cur.base += parts[i].count.bases;
+            cur.name += parts[i].count.name_bytes;
+        }
+        run_parallel(n_threads, n_pieces, [&](size_t i) {
+            const Part &pt = parts[i];
+            uint64_t end;
+            if (pt.count.records) (void)fastq_4line(t, n, pt.begin, std::min(n, lead + (i + 1) * piece), &end, sinks[i]);
+        });
+    } else {
+        FastqWrite sink{fa, 0, 0, 0, 0};
+        const char *why = nullptr;
+        fastq_serial(t, n, lead, sink, &why);
+    }
+    return CRF_OK;
+}
+
 }  // namespace fasta_detail
 
 static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf_fasta **out);
@@ -297,8 +535,20 @@ static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf
     } guard{new crf_fasta};
     crf_fasta *fa = guard.p;
 
-    // headers: a '>' at the start of a line
     const uint64_t PIECE = 8u << 20;
+    uint64_t lead = 0;                                  // a FASTQ file: '@' is its first byte that is not whitespace
+    while (lead < n && is_space(t[lead])) ++lead;
+    if (lead < n && t[lead] == '@') {
+        bool serial = false;
+        const int rc = parse_fastq(path, t, n, lead, n_threads, PIECE, pinned, fa, &serial);
+        if (rc != CRF_OK) return rc;
+        lap(serial ? "fastq-serial" : "fastq");
+        guard.p = nullptr;
+        *out = fa;
+        return CRF_OK;
+    }
+
+    // headers: a '>' at the start of a line
     std::vector<std::vector<uint64_t>> hdr_in((n + PIECE - 1) / PIECE);
     run_parallel(n_threads, hdr_in.size(), [&](size_t i) {
         const uint64_t hi = std::min<uint64_t>(n, (i + 1) * PIECE);
@@ -321,10 +571,7 @@ static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf
         body_lo[r] = eol ? h1 + 1 : stop;
         body_hi[r] = stop;
         uint64_t a = hdr[r] + 1;
-        auto is_space = [](uint8_t c) { return c == ' ' || c == '\t' || c == '\r' || c == '\n' || c == '\v' || c == '\f'; };
-        while (a < h1 && is_space(t[a])) ++a;
-        uint64_t b = a;
-        while (b < h1 && !is_space(t[b])) ++b;
+        const uint64_t b = name_token(t, &a, h1);
         fa->name_off.push_back(fa->names.size());
         fa->names.insert(fa->names.end(), t + a, t + b);
         fa->names.push_back('\0');
@@ -358,25 +605,7 @@ static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf
     fa->offsets[n_rec] = total;
     fa->total = total;
 
-    const size_t alloc = std::max<uint64_t>(total, 1);
-    fa->want_pinned_planes = (pinned & 3) != 0;
-    if (pinned & 1) {
-        void *p = nullptr;
-        if (cudaHostAlloc(&p, alloc, cudaHostAllocDefault) == cudaSuccess) {
-            fa->bases = (uint8_t *)p;
-            fa->pinned = true;
-        } else {
-            cudaGetLastError();                         // no device / no pinned memory left: plain pages
-        }
-    }
-    if (!fa->bases) fa->bases = (uint8_t *)malloc(alloc);
-    if (!fa->bases) { set_err("crf_fasta_open: out of host memory (%llu bases)", (unsigned long long)total); return CRF_ERR_NOMEM; }
-#if defined(__linux__) && defined(MADV_HUGEPAGE)
-    if (!fa->pinned && alloc >= ((size_t)8 << 20)) {    // gigabytes touched for the first time by the compaction below: 2 MB pages
-        const uintptr_t lo = ((uintptr_t)fa->bases + 4095) & ~(uintptr_t)4095, hi = ((uintptr_t)fa->bases + alloc) & ~(uintptr_t)4095;
-        if (hi > lo) madvise((void *)lo, hi - lo, MADV_HUGEPAGE);              // (advice only; the block is never realloc'ed)
-    }
-#endif
+    if (!alloc_bases(fa, total, pinned)) { set_err("crf_fasta_open: out of host memory (%llu bases)", (unsigned long long)total); return CRF_ERR_NOMEM; }
 
     lap("alloc");
     uint8_t *dst = fa->bases;
@@ -461,10 +690,23 @@ extern "C" int crf_fasta_data(const crf_fasta *fa, const uint8_t **bases, const 
     return CRF_OK;
 }
 
+extern "C" int crf_fasta_format(const crf_fasta *fa, int *format) {
+    if (!fa || !format) { set_err("crf_fasta_format: null argument"); return CRF_ERR_ARG; }
+    *format = fa->format;
+    return CRF_OK;
+}
+
+extern "C" int crf_fasta_quals(const crf_fasta *fa, const uint8_t **quals) {
+    if (!fa || !quals) { set_err("crf_fasta_quals: null argument"); return CRF_ERR_ARG; }
+    *quals = fa->quals;
+    return CRF_OK;
+}
+
 extern "C" int crf_fasta_close(crf_fasta *fa) {
     if (!fa) return CRF_OK;
     if (fa->pinned) cudaFreeHost(fa->bases);
     else free(fa->bases);
+    free(fa->quals);
     if (fa->planes_pinned) cudaFreeHost(fa->planes);
     else free(fa->planes);
     delete fa;

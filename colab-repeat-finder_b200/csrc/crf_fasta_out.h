@@ -1,6 +1,6 @@
-// Masked FASTA writer (host only): the records as read, with the bases a mask marks lower-cased (soft) or replaced by N
-// (hard) -- what TRF's -m output, dustmasker or a soft-masked reference give.  Formatted on several threads, in waves of
-// equal slices of the bases written in order, as crf_rows.h writes rows.
+// Masked FASTA / FASTQ writer (host only): the records as read, with the bases a mask marks lower-cased (soft) or replaced
+// by N (hard) -- what TRF's -m output, dustmasker or a soft-masked reference give.  Formatted on several threads, in waves
+// of equal slices of the bases written in order, as crf_rows.h writes rows.
 //
 // Included at the end of crf_api.cu after crf_rows.h (shares set_err()); tests/fuzz_mask_writer.cpp compiles it without
 // the CUDA runtime.
@@ -18,9 +18,12 @@
 
 // Formats the part of the file that stands for bases [p0, p1) into buf: the header of every record that starts there
 // (`last`: also those that start at p1, the empty records at the very end) and the bases with their line breaks.
+// quals != NULL: FASTQ, the bases on one line, and the slice that ends a record (or starts it, when it is empty) writes its
+// "+" line and qualities.
 static size_t fasta_out_slice(const char *const *name_ptr, const size_t *name_len, const uint8_t *bases,
-                              const uint64_t *offsets, uint64_t n_records, const uint32_t *mask, int hard, uint32_t width,
-                              uint64_t p0, uint64_t p1, bool last, std::vector<char> &buf) {
+                              const uint8_t *quals, const uint64_t *offsets, uint64_t n_records, const uint32_t *mask,
+                              int hard, uint32_t width, uint64_t p0, uint64_t p1, bool last, std::vector<char> &buf) {
+    auto ends_here = [&](uint64_t rs, uint64_t re) { return re <= p1 && (re > p0 || (rs == re && rs >= p0)); };
     uint64_t r = (uint64_t)(std::lower_bound(offsets, offsets + n_records, p0) - offsets);
     if (r > 0 && (r == n_records || offsets[r] > p0)) --r;   // the slice starts inside record r - 1
     const uint64_t r_begin = r;
@@ -29,13 +32,14 @@ static size_t fasta_out_slice(const char *const *name_ptr, const size_t *name_le
         const uint64_t a = std::max(offsets[q], p0), b = std::min(offsets[q + 1], p1);
         if (offsets[q] >= p0) need += name_len[q] + 2;
         if (b > a) need += (b - a) + (b - a) / width + 2;
+        if (quals && ends_here(offsets[q], offsets[q + 1])) need += offsets[q + 1] - offsets[q] + 4;
     }
     if (buf.size() < need) buf.resize(need);
     char *out = buf.data();
     for (; r < n_records && (offsets[r] < p1 || (last && offsets[r] == p1)); ++r) {
         const uint64_t rs = offsets[r], re = offsets[r + 1];
         if (rs >= p0) {
-            *out++ = '>';
+            *out++ = quals ? '@' : '>';
             memcpy(out, name_ptr[r], name_len[r]);
             out += name_len[r];
             *out++ = '\n';
@@ -43,7 +47,7 @@ static size_t fasta_out_slice(const char *const *name_ptr, const size_t *name_le
         uint64_t p = std::max(rs, p0);
         const uint64_t stop = std::min(re, p1);
         while (p < stop) {                                   // one line, or the part of it inside the slice
-            const uint64_t line_end = rs + ((p - rs) / width + 1) * width;
+            const uint64_t line_end = quals ? re : rs + ((p - rs) / width + 1) * width;
             const uint64_t q = std::min(line_end, stop);
             memcpy(out, bases + p, q - p);
             for (uint64_t w = p >> 5; w <= (q - 1) >> 5; ++w) {
@@ -61,14 +65,24 @@ static size_t fasta_out_slice(const char *const *name_ptr, const size_t *name_le
             if (q == line_end || q == re) *out++ = '\n';
             p = q;
         }
+        if (quals && ends_here(rs, re)) {
+            if (rs == re) *out++ = '\n';
+            *out++ = '+';
+            *out++ = '\n';
+            memcpy(out, quals + rs, re - rs);
+            out += re - rs;
+            *out++ = '\n';
+        }
     }
     return (size_t)(out - buf.data());
 }
 
-static int write_fasta_masked_impl(const char *path, const char *names, const uint8_t *bases, const uint64_t *offsets,
-                                   uint64_t n_records, const uint32_t *mask, int hard, uint32_t width, uint64_t *bytes) {
+// fn: the caller's name, for messages
+static int write_fasta_masked_impl(const char *fn, const char *path, const char *names, const uint8_t *bases,
+                                   const uint8_t *quals, const uint64_t *offsets, uint64_t n_records, const uint32_t *mask,
+                                   int hard, uint32_t width, uint64_t *bytes) {
     FILE *f = fopen(path, "wb");
-    if (!f) { set_err("crf_write_fasta_masked: cannot open %s", path); return CRF_ERR_ARG; }
+    if (!f) { set_err("%s: cannot open %s", fn, path); return CRF_ERR_ARG; }
     struct Closer {                                  // the file is closed on every way out (bad_alloc included)
         FILE *f;
         ~Closer() { if (f) fclose(f); }
@@ -106,8 +120,8 @@ static int write_fasta_masked_impl(const char *path, const char *names, const ui
             if (j >= n_slices) continue;
             auto job = [&, t, p0, p1, last]() {
                 try {
-                    used[t] = fasta_out_slice(name_ptr.data(), name_len.data(), bases, offsets, n_records, mask, hard, width,
-                                              p0, p1, last, bufs[t]);
+                    used[t] = fasta_out_slice(name_ptr.data(), name_len.data(), bases, quals, offsets, n_records, mask, hard,
+                                              width, p0, p1, last, bufs[t]);
                 } catch (const std::bad_alloc &) { no_memory = true; }
             };
             if (n_thr == 1) { job(); continue; }
@@ -123,29 +137,48 @@ static int write_fasta_masked_impl(const char *path, const char *names, const ui
     if (fclose(f) != 0) ok = false;
     if (bytes) *bytes = total;
     if (!ok) {
-        set_err("crf_write_fasta_masked: write to %s failed (after %llu bytes)", path, (unsigned long long)total);
+        set_err("%s: write to %s failed (after %llu bytes)", fn, path, (unsigned long long)total);
         return CRF_ERR_IO;
     }
     return CRF_OK;
 }
 
-extern "C" int crf_write_fasta_masked(const char *path, const char *names, const uint8_t *bases, const uint64_t *offsets,
-                                      uint64_t n_records, const uint32_t *mask, int hard, uint32_t line_width,
-                                      uint64_t *bytes) {
+// The checks and the call both writers share.  quals: NULL for FASTA.
+static int write_masked(const char *fn, const char *path, const char *names, const uint8_t *bases, const uint8_t *quals,
+                        const uint64_t *offsets, uint64_t n_records, const uint32_t *mask, int hard, uint32_t line_width,
+                        uint64_t *bytes) {
     if (!path || (n_records && (!names || !offsets)) || line_width == 0) {
-        set_err("crf_write_fasta_masked: null argument or zero line width");
+        set_err("%s: null argument or zero line width", fn);
         return CRF_ERR_ARG;
     }
     if (n_records && offsets[n_records] > offsets[0] && (!bases || !mask)) {
-        set_err("crf_write_fasta_masked: null bases or mask");
+        set_err("%s: null bases or mask", fn);
         return CRF_ERR_ARG;
     }
     for (uint64_t r = 0; r < n_records; ++r)
-        if (offsets[r + 1] < offsets[r]) { set_err("crf_write_fasta_masked: offsets decrease at record %llu", (unsigned long long)r); return CRF_ERR_ARG; }
+        if (offsets[r + 1] < offsets[r]) { set_err("%s: offsets decrease at record %llu", fn, (unsigned long long)r); return CRF_ERR_ARG; }
     try {                                            // no exception crosses the C boundary
-        return write_fasta_masked_impl(path, names, bases, offsets, n_records, mask, hard, line_width, bytes);
+        return write_fasta_masked_impl(fn, path, names, bases, quals, offsets, n_records, mask, hard, line_width, bytes);
     } catch (const std::bad_alloc &) {
-        set_err("crf_write_fasta_masked: out of host memory");
+        set_err("%s: out of host memory", fn);
         return CRF_ERR_NOMEM;
     }
+}
+
+extern "C" int crf_write_fasta_masked(const char *path, const char *names, const uint8_t *bases, const uint64_t *offsets,
+                                      uint64_t n_records, const uint32_t *mask, int hard, uint32_t line_width,
+                                      uint64_t *bytes) {
+    return write_masked("crf_write_fasta_masked", path, names, bases, nullptr, offsets, n_records, mask, hard, line_width,
+                        bytes);
+}
+
+extern "C" int crf_write_fastq_masked(const char *path, const char *names, const uint8_t *bases, const uint8_t *quals,
+                                      const uint64_t *offsets, uint64_t n_records, const uint32_t *mask, int hard,
+                                      uint64_t *bytes) {
+    if (n_records && !quals) {                       // (an empty read too has a quality line)
+        set_err("crf_write_fastq_masked: null qualities");
+        return CRF_ERR_ARG;
+    }
+    return write_masked("crf_write_fastq_masked", path, names, bases, quals, offsets, n_records, mask, hard, UINT32_MAX,
+                        bytes);
 }

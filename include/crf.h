@@ -312,21 +312,34 @@ int crf_write_rows_at(const char *path, int append, int tsv, const char *names, 
  * threads.  *bytes = bytes written; a short write is CRF_ERR_IO. */
 int crf_write_fasta_masked(const char *path, const char *names, const uint8_t *bases, const uint64_t *offsets,
                            uint64_t n_records, const uint32_t *mask, int hard, uint32_t line_width, uint64_t *bytes);
+/* The same as a FASTQ file: per record "@name\n", its bases on one line (masked as above), "+\n" and quals[offsets[r] ..
+ * offsets[r+1]) on one line, written as they are (quals is indexed like bases, as crf_fasta_quals gives it). */
+int crf_write_fastq_masked(const char *path, const char *names, const uint8_t *bases, const uint8_t *quals,
+                           const uint64_t *offsets, uint64_t n_records, const uint32_t *mask, int hard, uint64_t *bytes);
 
 /* ---- input (host only, no GPU) ---------------------------------------------------------------
  * Native FASTA ingest, replacing what the reference takes from pyfastx (prf:117-137: the records in file
  * order, .name = first whitespace-delimited header token, .seq = the lines joined, case preserved).  Plain or
- * gzip (concatenated members too; BGZF/bgzip blocks are inflated in parallel).  The result is laid out as crf_seq_load_ascii and crf_write_rows
+ * gzip (concatenated members too; BGZF/bgzip blocks are inflated in parallel).
+ * FASTQ too: a text whose first byte that is not whitespace is '@' is read as FASTQ (records '@name ...', sequence
+ * lines up to a line starting with '+', quality lines until they hold as many bytes as the sequence; multi-line records
+ * and CRLF line ends are read; a malformed record is CRF_ERR_ARG naming its 1-based number), with the same layout.  The result is laid out as crf_seq_load_ascii and crf_write_rows
  * take it: all records back to back, n_records+1 offsets, NUL-separated names.  n_threads = 0: up to 16.
  * pinned: bit 0 = page-locked base buffer (cudaHostAlloc, when a device is present: a faster upload of the text), bit 1 =
  * page-locked planes only (crf_fasta_packed; bit 0 implies it) -- what a caller that uploads the planes and keeps the text
- * on the host for the motif column wants: page-locking gigabytes it never uploads costs seconds.
- * The pointers of crf_fasta_data stay valid until crf_fasta_close. */
+ * on the host for the motif column wants: page-locking gigabytes it never uploads costs seconds.  Bit 2 (value 4): keep
+ * a FASTQ file's qualities (crf_fasta_quals); without it they are checked and dropped.
+ * The pointers of crf_fasta_data and crf_fasta_quals stay valid until crf_fasta_close. */
 typedef struct crf_fasta crf_fasta;
 int crf_fasta_open(const char *path, uint32_t n_threads, int pinned, crf_fasta **fasta);
 int crf_fasta_info(const crf_fasta *fasta, uint64_t *n_records, uint64_t *total_bases, int *pinned);
 int crf_fasta_data(const crf_fasta *fasta, const uint8_t **bases, const uint64_t **offsets, const char **names,
                    uint64_t *names_bytes);
+/* *format = 0 for a FASTA file, 1 for a FASTQ file. */
+int crf_fasta_format(const crf_fasta *fasta, int *format);
+/* A FASTQ file's qualities, laid out like the bases (record r = quals[offsets[r] .. offsets[r+1])); NULL for a FASTA
+ * file or when crf_fasta_open was not given pinned bit 2. */
+int crf_fasta_quals(const crf_fasta *fasta, const uint8_t **quals);
 /* Packed planes of the whole file (all records back to back, as crf_seq_load_packed takes them), made on first call
  * and owned by the handle; page-locked when the base buffer is. */
 int crf_fasta_packed(crf_fasta *fasta, uint32_t n_threads, const uint32_t **H, const uint32_t **L, const uint32_t **NM,
