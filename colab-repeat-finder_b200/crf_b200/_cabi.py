@@ -29,10 +29,11 @@ EXPORTS = [
     "crf_last_error", "crf_abi_version", "crf_ctx_create", "crf_ctx_destroy", "crf_ctx_set_stream",
     "crf_ctx_synchronize", "crf_load_limit", "crf_seq_load_packed", "crf_seq_load_packed_ranges", "crf_pack_ascii",
     "crf_seq_load_packed_runs", "crf_seq_load_packed_runs_ranges", "crf_mask_runs",
-    "crf_fasta_packed", "crf_seq_load_ascii", "crf_seq_load_ascii_ranges", "crf_seq_set_output_map", "crf_seq_destroy", "crf_seq_info", "crf_scan", "crf_fetch",
+    "crf_fasta_packed", "crf_seq_load_2bit", "crf_seq_load_ascii", "crf_seq_load_ascii_ranges", "crf_seq_set_output_map", "crf_seq_destroy", "crf_seq_info", "crf_scan", "crf_fetch",
     "crf_scan_stats", "crf_run_end", "crf_interval_stop", "crf_fetch_open", "crf_patch_end", "crf_write_rows",
-    "crf_write_rows_at", "crf_mask_rows", "crf_write_fasta_masked", "crf_write_fastq_masked",
-    "crf_fasta_open", "crf_fasta_info", "crf_fasta_data", "crf_fasta_format", "crf_fasta_quals", "crf_fasta_close",
+    "crf_write_rows_at", "crf_write_rows_twobit", "crf_mask_rows", "crf_write_fasta_masked", "crf_write_fastq_masked",
+    "crf_fasta_open", "crf_fasta_info", "crf_fasta_data", "crf_fasta_format", "crf_fasta_quals", "crf_fasta_index",
+    "crf_fasta_twobit", "crf_fasta_close",
     "crf_gunzip",
     "crf_xchg_create", "crf_xchg_destroy", "crf_xchg_export", "crf_xchg_connect_ipc", "crf_xchg_connect_local",
     "crf_xchg_set_timeout", "crf_xchg_set_compact", "crf_scan_gather", "crf_xchg_push", "crf_xchg_wait", "crf_xchg_step_result", "crf_xchg_fetch",
@@ -106,6 +107,7 @@ def lib():
         L.crf_seq_load_packed_runs_ranges.argtypes = [vp, vp, vp, vp, u64, vp, u64, vp, vp, vp, vp, u32, u32, i, P(vp)]
         L.crf_mask_runs.argtypes = [vp, u64, u32, vp, u64, P(u64)]
         L.crf_fasta_packed.argtypes = [vp, u32, P(vp), P(vp), P(vp), P(vp), P(u64)]
+        L.crf_seq_load_2bit.argtypes = [vp, vp, vp, vp, u32, vp, u64, u32, i, P(vp)]
         L.crf_seq_set_output_map.argtypes = [vp, vp, vp, vp]
         L.crf_seq_destroy.argtypes = [vp]
         L.crf_seq_info.argtypes = [vp, P(SeqInfo)]
@@ -118,6 +120,7 @@ def lib():
         L.crf_patch_end.argtypes = [vp, u64, u32]
         L.crf_write_rows.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
         L.crf_write_rows_at.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
+        L.crf_write_rows_twobit.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
         L.crf_mask_rows.argtypes = [vp, vp, vp, vp, u64, i, vp, u32, vp, u64, i]
         L.crf_write_fasta_masked.argtypes = [ctypes.c_char_p, vp, vp, vp, u64, vp, i, u32, P(u64)]
         L.crf_write_fastq_masked.argtypes = [ctypes.c_char_p, vp, vp, vp, vp, u64, vp, i, P(u64)]
@@ -126,6 +129,8 @@ def lib():
         L.crf_fasta_data.argtypes = [vp, P(vp), P(vp), P(vp), P(u64)]
         L.crf_fasta_format.argtypes = [vp, P(i)]
         L.crf_fasta_quals.argtypes = [vp, P(vp)]
+        L.crf_fasta_index.argtypes = [vp, P(vp), P(vp), P(u64)]
+        L.crf_fasta_twobit.argtypes = [vp, P(vp), P(vp), P(vp), P(u64)]
         L.crf_fasta_close.argtypes = [vp]
         L.crf_gunzip.argtypes = [vp, ctypes.c_uint64, vp, ctypes.c_uint64, ctypes.POINTER(ctypes.c_uint64), ctypes.c_int]
         L.crf_xchg_create.argtypes = [vp, u32, u32, u64, P(vp)]
@@ -213,6 +218,14 @@ class Context:
             offsets = np.array([0, planes.n_bases], dtype=np.uint64)
         return Sequence(self, None, offsets, max_motif_cap, False, ranges=ranges, packed=planes)
 
+    def load_2bit(self, source, max_motif_cap=50, on_device=False):
+        """crf_seq_load_2bit: the records of a .2bit file, loaded from its packed bytes.  source: a .2bit Fasta, or a
+        TwoBitSource (Fasta.twobit(), .records(first, last) for some of them) whose dna may also be a CUDA uint8 tensor
+        holding the file's bytes, or a device pointer (int) with on_device=True."""
+        if isinstance(source, Fasta):
+            source = source.twobit()
+        return Sequence(self, None, None, max_motif_cap, on_device, twobit=source)
+
     @_serialised
     def mask_rows(self, record, start, end, dst_offset, mask_bits, n_rows=None, mask=None):
         """crf_mask_rows: the union of the rows [dst_offset[record] + start, dst_offset[record] + end) as a bit mask.
@@ -251,10 +264,39 @@ class Sequence:
     """Records resident in HBM as packed planes (crf_seq)."""
 
     @_serialised
-    def __init__(self, ctx, bases, offsets, max_motif_cap, on_device, ranges=None, packed=None):
+    def __init__(self, ctx, bases, offsets, max_motif_cap, on_device, ranges=None, packed=None, twobit=None):
         self.ctx = ctx
         self._h = ctypes.c_void_p()
         keep = None
+        if twobit is not None:
+            src = twobit
+            dna = src.dna
+            if hasattr(dna, "data_ptr"):                  # a torch tensor holding the file's bytes
+                if str(dna.dtype) != "torch.uint8" or not dna.is_contiguous():
+                    raise ValueError("dna must be a contiguous torch.uint8 tensor")
+                if dna.is_cuda:
+                    import torch
+                    torch.cuda.current_stream(dna.device).synchronize()     # its bytes are written before the upload
+                    on_device = True
+                ptr = dna.data_ptr()
+            elif isinstance(dna, int):
+                if not on_device:
+                    raise ValueError("a pointer as dna needs on_device=True")
+                ptr = dna
+            else:
+                ptr, _ = _host_bytes("dna", dna)
+            offsets = np.ascontiguousarray(src.offsets, dtype=np.uint64)
+            rec_byte = np.ascontiguousarray(src.rec_byte, dtype=np.uint64)
+            runs = np.ascontiguousarray(src.runs, dtype=np.uint64).reshape(-1, 2)
+            if offsets.ndim != 1 or offsets.size < 2 or rec_byte.shape != (offsets.size - 1,):
+                raise ValueError("a .2bit source needs n_records + 1 offsets and n_records rec_byte entries")
+            self.offsets = offsets
+            self.n_records = offsets.size - 1
+            _check(lib().crf_seq_load_2bit(ctx._h, ctypes.c_void_p(ptr), ctypes.c_void_p(rec_byte.ctypes.data),
+                                           ctypes.c_void_p(offsets.ctypes.data), self.n_records,
+                                           ctypes.c_void_p(runs.ctypes.data if runs.size else 0), runs.shape[0],
+                                           int(max_motif_cap), int(bool(on_device)), ctypes.byref(self._h)))
+            return
         if packed is not None:
             pk = packed
             ex_ptr = pk.exotic.ctypes.data if pk.exotic.size else 0
@@ -613,11 +655,25 @@ class Xchg:
             pass
 
 
+class TwoBitSource:
+    """The packed form of a .2bit file's records, what crf_seq_load_2bit and crf_write_rows_twobit take: dna (the file's
+    bytes: a host uint8 array, a CUDA torch.uint8 tensor, or a device pointer), rec_byte[r] (the byte where record r's
+    packed bases start), offsets (n_records + 1, the records' position space) and runs ((n, 2) N blocks in that space)."""
+
+    def __init__(self, dna, rec_byte, offsets, runs, keep=None):
+        self.dna, self.rec_byte, self.offsets, self.runs = dna, rec_byte, offsets, runs
+        self._keep = keep
+
+    def records(self, first, last):
+        """Records [first, last) (the run list stays whole: a load ignores runs outside its records)."""
+        return TwoBitSource(self.dna, self.rec_byte[first:last], self.offsets[first:last + 1], self.runs, self._keep)
+
+
 class Fasta:
-    """A FASTA or FASTQ file read by the native reader (crf_fasta_open): `bases` (uint8 view of all records back to
-    back, owned by the library until close()), `offsets` (n_records+1, uint64), `names` (list of str),
-    `names_blob` (NUL-separated, as crf_write_rows takes them), `format` ("fasta" / "fastq") and `quals` (a FASTQ file's
-    qualities as a uint8 view laid out like `bases`, or None)."""
+    """A FASTA, FASTQ or .2bit file read by the native reader (crf_fasta_open): `bases` (uint8 view of all records back
+    to back, owned by the library until close(); a .2bit file's text is decoded on first use), `offsets` (n_records+1,
+    uint64), `names` (list of str), `names_blob` (NUL-separated, as crf_write_rows takes them), `format` ("fasta" /
+    "fastq" / "2bit") and `quals` (a FASTQ file's qualities as a uint8 view laid out like `bases`, or None)."""
 
     def __init__(self, path, n_threads=0, pinned=False, qualities=False):
         """pinned: False / True (page-locked base buffer and planes) / 2 (page-locked planes only: the text stays pageable).
@@ -627,12 +683,10 @@ class Fasta:
                                     ctypes.byref(self._h)))
         n_rec, total, pin = ctypes.c_uint64(), ctypes.c_uint64(), ctypes.c_int()
         _check(lib().crf_fasta_info(self._h, ctypes.byref(n_rec), ctypes.byref(total), ctypes.byref(pin)))
-        bases, offsets, names, nbytes = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_uint64()
-        _check(lib().crf_fasta_data(self._h, ctypes.byref(bases), ctypes.byref(offsets), ctypes.byref(names),
-                                    ctypes.byref(nbytes)))
+        offsets, names, nbytes = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_uint64()
+        _check(lib().crf_fasta_index(self._h, ctypes.byref(offsets), ctypes.byref(names), ctypes.byref(nbytes)))
         self.n_records, self.total_bases, self.pinned = n_rec.value, total.value, bool(pin.value)
-        self.bases = np.ctypeslib.as_array(ctypes.cast(bases, ctypes.POINTER(ctypes.c_uint8)),
-                                           shape=(max(self.total_bases, 1),))[:self.total_bases]
+        self._bases = None
         self.offsets = np.ctypeslib.as_array(ctypes.cast(offsets, ctypes.POINTER(ctypes.c_uint64)),
                                              shape=(self.n_records + 1,)).copy()
         self.names_blob = ctypes.string_at(names, nbytes.value) if nbytes.value else b""
@@ -640,9 +694,36 @@ class Fasta:
         fmt, quals = ctypes.c_int(), ctypes.c_void_p()
         _check(lib().crf_fasta_format(self._h, ctypes.byref(fmt)))
         _check(lib().crf_fasta_quals(self._h, ctypes.byref(quals)))
-        self.format = "fastq" if fmt.value == 1 else "fasta"
+        self.format = {1: "fastq", 2: "2bit"}.get(fmt.value, "fasta")
         self.quals = np.ctypeslib.as_array(ctypes.cast(quals, ctypes.POINTER(ctypes.c_uint8)),
                                            shape=(max(self.total_bases, 1),))[:self.total_bases] if quals.value else None
+
+    @property
+    def bases(self):
+        """uint8 view of all records back to back (crf_fasta_data; a .2bit file's text is decoded on the first call)."""
+        if self._bases is None and self._h:
+            bases = ctypes.c_void_p()
+            _check(lib().crf_fasta_data(self._h, ctypes.byref(bases), None, None, None))
+            self._bases = np.ctypeslib.as_array(ctypes.cast(bases, ctypes.POINTER(ctypes.c_uint8)),
+                                                shape=(max(self.total_bases, 1),))[:self.total_bases]
+        return self._bases
+
+    def twobit(self):
+        """TwoBitSource of a .2bit file (crf_fasta_twobit; ValueError for any other format).  dna is a view of the handle's
+        bytes, valid until close()."""
+        dna, rec_byte, runs, n_runs = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_uint64()
+        _check(lib().crf_fasta_twobit(self._h, ctypes.byref(dna), ctypes.byref(rec_byte), ctypes.byref(runs),
+                                      ctypes.byref(n_runs)))
+        def u64s(ptr, n):
+            return np.ctypeslib.as_array(ctypes.cast(ptr, ctypes.POINTER(ctypes.c_uint64)), shape=(n,)).copy() \
+                if n else np.zeros(0, np.uint64)
+        rb = u64s(rec_byte, self.n_records)
+        rn = u64s(runs, 2 * n_runs.value).reshape(-1, 2)
+        lengths = np.diff(self.offsets.astype(np.int64))
+        size = int((rb.astype(np.int64) + (lengths + 3) // 4).max()) if self.n_records else 0
+        view = np.ctypeslib.as_array(ctypes.cast(dna, ctypes.POINTER(ctypes.c_uint8)), shape=(max(size, 1),))[:size] \
+            if dna.value else np.zeros(0, np.uint8)
+        return TwoBitSource(view, rb, self.offsets, rn, keep=self)
 
     @property
     def names(self):
@@ -667,7 +748,7 @@ class Fasta:
 
     def close(self):
         if self._h:
-            self.bases = self.quals = None
+            self._bases = self.quals = None
             lib().crf_fasta_close(self._h)
             self._h = ctypes.c_void_p()
 
@@ -708,6 +789,24 @@ def write_rows(path, names, bases, offsets, record, start, end, k, tsv=False, ap
     else:
         origin = np.ascontiguousarray(origin, dtype=np.uint64)
         _check(lib().crf_write_rows_at(*head, ctypes.c_void_p(origin.ctypes.data), *tail))
+    return nbytes.value
+
+
+def write_rows_twobit(path, names, dna, rec_byte, record, start, end, k, tsv=False, append=False):
+    """crf_write_rows_twobit: write_rows for records of a .2bit file, the motif read from the packed bytes (dna: host uint8
+    array of the file's bytes, rec_byte[r]: where record r's bases start, as TwoBitSource has them)."""
+    if isinstance(names, (bytes, bytearray)):
+        blob = bytes(names)
+    else:
+        blob = b"".join(n.encode("utf-8") + b"\0" for n in names) if names is not None else None
+    arrs = [np.ascontiguousarray(a, dtype=np.uint32) for a in (record, start, end, k)]
+    rec_byte = np.ascontiguousarray(rec_byte, dtype=np.uint64)
+    dptr, _ = _host_bytes("dna", dna)
+    nbytes = ctypes.c_uint64()
+    _check(lib().crf_write_rows_twobit(os.fsencode(path), int(append), int(tsv),
+                                       ctypes.cast(ctypes.c_char_p(blob), ctypes.c_void_p) if blob is not None else None,
+                                       ctypes.c_void_p(dptr), ctypes.c_void_p(rec_byte.ctypes.data),
+                                       *(ctypes.c_void_p(a.ctypes.data) for a in arrs), len(arrs[0]), ctypes.byref(nbytes)))
     return nbytes.value
 
 

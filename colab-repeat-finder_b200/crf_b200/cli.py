@@ -4,7 +4,7 @@ Same flags, defaults, stdout lines and output files as the reference's main()
 (the reference's perfect_repeat_finder.py:83-179), re-organised around two code paths:
 
   FASTA file  -> <basename(prefix)>.bed in the working directory (chrom, start_0based, end, motif); a FASTQ file is
-                 read the same way, its read names as chrom
+                 read the same way, its read names as chrom; a .2bit file too, loaded from its packed bytes
   raw string  -> <prefix>.tsv with a header line (start_0based, end, motif)
 
 Deliberate deviations (SURVEY.md section 8b):
@@ -63,7 +63,8 @@ def build_parser():
         filters.add_argument(*flags, **kw)
     for flags, kw in _OTHER_OPTIONS:
         parser.add_argument(*flags, **kw)
-    parser.add_argument("input_sequence", help="A nucleotide string, or the path of a FASTA or FASTQ file (plain or .gz)")
+    parser.add_argument("input_sequence", help="A nucleotide string, or the path of a FASTA or FASTQ file (plain or .gz) "
+                                               "or of a UCSC .2bit file")
     return parser
 
 
@@ -123,11 +124,30 @@ def _whole_fasta_to_bed(fa, args, bed_path, mask_rows=None):
     lengths = np.diff(fa.offsets.astype(np.int64))
     counts = np.zeros(fa.n_records, dtype=np.int64)
     open(bed_path, "wb").close()
+    limit = _cabi.load_limit(args.max_motif_size)
+    groups = group_records(lengths, args.max_motif_size)
+    # a .2bit file on one GPU: each group is loaded from the file's packed bytes (0.25 B/bp, packed into the layout on the
+    # device) and its motifs are read from them; the text is never decoded
+    twobit = fa.twobit() if fa.format == "2bit" and len(devices) == 1 else None
+    if twobit is not None and all(not lengths[f:l].size or int(lengths[f:l].max()) + args.max_motif_size <= limit
+                                  for f, l in groups):
+        for first, last in groups:
+            if not int(lengths[first:last].sum()):
+                continue
+            with api.get_context(devices[0]).load_2bit(twobit.records(first, last), max_motif_cap=args.max_motif_size) as seq:
+                n = seq.scan(args.min_motif_size, args.max_motif_size, args.min_repeats, args.min_span)
+                rec, start, end, k = seq.fetch(n)
+            whole_file = first == 0 and last == fa.n_records
+            _cabi.write_rows_twobit(bed_path, fa.names_blob if whole_file else fa.names[first:last], twobit.dna,
+                                    twobit.rec_byte[first:last], rec, start, end, k, append=True)
+            if mask_rows is not None:
+                mask_rows.append((rec, start, end, fa.offsets[first:last]))
+            counts[first:last] += np.bincount(rec.astype(np.int64, copy=False), minlength=last - first)
+        return counts
     # the text is packed to 2-bit planes + mask on the host (threaded, at ingest) and uploaded at 0.375 B/bp; the ASCII
     # buffer stays on the host for the motif column
     planes = fa.packed() if fa.total_bases else None
-    limit = _cabi.load_limit(args.max_motif_size)
-    for first, last in group_records(lengths, args.max_motif_size):
+    for first, last in groups:
         total = int(lengths[first:last].sum())
         base0 = int(fa.offsets[first])
         blob = fa.bases[base0:base0 + total]
@@ -261,7 +281,10 @@ def _intervals_to_bed(parser, fa, args, bed_path):
 
 def default_prefix(path, fmt):
     """The output prefix when -o is not given.  FASTA: the (unanchored) regex of prf:114, as the reference has it.  FASTQ:
-    the path without a trailing .fastq / .fq, optionally followed by .gz / .bgz (reads.fq.gz -> reads)."""
+    the path without a trailing .fastq / .fq, optionally followed by .gz / .bgz (reads.fq.gz -> reads).  .2bit: the path
+    without a trailing .2bit."""
+    if fmt == "2bit":
+        return re.sub(r"\.2bit$", "", path)
     if fmt == "fastq":
         return re.sub(r"\.(fastq|fq)(\.(gz|bgz))?$", "", path)
     return re.sub(".fa(sta)?(.gz)?", "", path)

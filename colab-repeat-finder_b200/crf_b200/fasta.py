@@ -1,7 +1,8 @@
 """FASTA input through the library's native reader (crf_fasta_open), standing in for pyfastx
 (perfect_repeat_finder.py:117-137 uses only `.name` -- the first whitespace-delimited token of the header --
 and `.seq`, the record's lines joined without line ends, case preserved).  Plain or gzip input.  A FASTQ file (first
-byte that is not whitespace: '@') is read too: read names and sequences in the same layout, qualities on request."""
+byte that is not whitespace: '@') is read too: read names and sequences in the same layout, qualities on request.  So is a
+UCSC .2bit file, whose text (what twoBitToFa writes) is decoded on first use of `bases`."""
 import os
 
 from . import _cabi

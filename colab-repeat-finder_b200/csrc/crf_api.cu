@@ -356,7 +356,7 @@ static uint64_t layout_limit(uint32_t max_motif_cap) {
 // One load holds at most this many layout positions: sum over records of (length + max_motif_cap).
 extern "C" uint64_t crf_load_limit(uint32_t max_motif_cap) { return layout_limit(max_motif_cap); }
 
-// What a load reads: ASCII bytes (one per base) or planes packed on the host (crf_pack_ascii).
+// What a load reads: ASCII bytes (one per base), planes packed on the host (crf_pack_ascii), or the bytes of a .2bit file.
 struct LoadSource {
     const uint8_t *bases = nullptr;                     // ASCII
     const uint32_t *pH = nullptr, *pL = nullptr, *pN = nullptr;   // packed: source position p = bit p & 31 of word p >> 5
@@ -365,7 +365,8 @@ struct LoadSource {
     const uint64_t *nm_runs = nullptr;                  // packed, instead of pN: the masked positions as sorted runs
     uint64_t n_runs = 0;                                //   [runs[2i], runs[2i+1]) -- 0.25 B/bp cross PCIe instead of 0.375
     bool runs_mode = false;
-    bool packed() const { return pH != nullptr; }
+    const uint8_t *twobit = nullptr;                    // .2bit (runs mode): source position p = base p & 3 of byte p >> 2
+    bool packed() const { return pH != nullptr || twobit != nullptr; }
 };
 
 // The two passes over the per-record arrays of a load run on a few threads when there are millions of records.
@@ -402,7 +403,7 @@ struct LoadTrace {
 static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, const uint64_t *lengths,
                      const uint64_t *own_lo, const uint64_t *own_hi, uint32_t n_records, uint32_t max_motif_cap,
                      int on_device, crf_seq *s) {
-    const char *who = src.packed() ? "crf_seq_load_packed" : "crf_seq_load_ascii";
+    const char *who = src.twobit ? "crf_seq_load_2bit" : src.packed() ? "crf_seq_load_packed" : "crf_seq_load_ascii";
     LoadTrace trace;
     cudaStream_t st = c->stream;
     s->ctx = c;
@@ -486,7 +487,8 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
     // The source span the records cover (units may overlap) goes up in chunks on a second stream while the pack kernel
     // works on the layout words whose source has already arrived (the PCIe copy is ~10x longer than the packing, which
     // then hides behind it).  Unit of the span: bytes (ASCII) or positions rounded out to whole 32-bit words (packed).
-    const bool packed = src.packed();
+    const bool packed = src.packed(), twobit = src.twobit != nullptr;
+    const uint64_t src_end = src_hi;                                     // .2bit: bytes up to (src_end + 3) / 4 are the caller's
     if (packed) { src_lo &= ~31ull; src_hi = (src_hi + 31) & ~31ull; }
     const uint64_t span = src_hi - src_lo;                               // positions
     const uint64_t UPLOAD_CHUNK = packed ? (512ull << 20) : (64ull << 20);   // positions per chunk (64 MB either way)
@@ -537,6 +539,11 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
     trace.mark("source allocs + runs_rel");
     auto copy_span = [&](uint64_t lo, uint64_t n, cudaStream_t cs) -> cudaError_t {    // source positions [src_lo + lo, + n)
         if (!n) return cudaSuccess;
+        if (twobit) {                                                    // (lo is a multiple of 32: whole bytes)
+            const uint64_t b0 = (src_lo + lo) / 4, b1 = std::min((src_lo + lo + n + 3) / 4, (src_end + 3) / 4);
+            if (b1 <= b0) return cudaSuccess;
+            return cudaMemcpyAsync((uint8_t *)d_planes_own + lo / 4, src.twobit + b0, b1 - b0, cudaMemcpyHostToDevice, cs);
+        }
         if (!packed) return cudaMemcpyAsync(d_src_own + lo, src.bases + src_lo + lo, n, cudaMemcpyHostToDevice, cs);
         const uint64_t w0 = lo / 32, nw = (n + 31) / 32, h0 = src_lo / 32 + w0;
         cudaError_t e = cudaMemcpyAsync(d_planes_own + w0, src.pH + h0, nw * 4, cudaMemcpyHostToDevice, cs);
@@ -647,7 +654,16 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
     // one launch of the packer over layout words [w_lo, w_hi)
     auto launch_pack = [&](uint32_t w_lo, uint32_t w_hi) -> cudaError_t {
         if (w_hi <= w_lo) return cudaSuccess;
-        if (packed) {
+        if (twobit) {
+            TwoBitParams tp;
+            tp.dna = on_device ? src.twobit : (const uint8_t *)d_planes_own;
+            tp.n_bytes = (src_end + 3) / 4 - (on_device ? 0 : src_lo / 4);
+            tp.sN = d_pN; tp.src_base = src_base;
+            tp.rec_src_start = d_src_start; tp.rec_len = s->d_rec_len; tp.rec_dev_off = s->d_rec_dev_off;
+            tp.n_records = n_records; tp.w_lo = w_lo; tp.w_hi = w_hi;
+            tp.H = s->H; tp.L = s->L; tp.NM = s->NM; tp.X = s->X;
+            twobit_pack_kernel<<<(w_hi - w_lo + 255) / 256, 256, 0, st>>>(tp);
+        } else if (packed) {
             RepackParams rp;
             rp.sH = d_pH; rp.sL = d_pL; rp.sN = d_pN; rp.src_base = src_base;
             rp.rec_src_start = d_src_start; rp.rec_len = s->d_rec_len; rp.rec_dev_off = s->d_rec_dev_off;
@@ -790,7 +806,7 @@ static int load_checked(crf_ctx *c, const LoadSource &src, const uint64_t *start
         set_err("%s: max_motif_cap %u not in [1, %u]", who, max_motif_cap, MAX_K);
         return max_motif_cap < 1 ? CRF_ERR_ARG : CRF_ERR_UNSUPPORTED;
     }
-    const bool have_src = src.packed() ? (src.pL && src.pN) : (src.bases != nullptr);
+    const bool have_src = src.twobit ? true : src.packed() ? (src.pL && src.pN) : (src.bases != nullptr);
     if (!have_src) {
         for (uint32_t r = 0; r < n_records; ++r)
             if (lengths ? lengths[r] : starts[r + 1] - starts[r]) { set_err("%s: null %s", who, src.packed() ? "plane" : "bases"); return CRF_ERR_ARG; }
@@ -891,6 +907,68 @@ extern "C" int crf_seq_load_packed_runs(crf_ctx *c, const uint32_t *H, const uin
     CHECK(check_offsets(offsets, n_records, "crf_seq_load_packed_runs"));
     return packed_runs_load(c, H, L, runs, n_runs, exotic, n_exotic, offsets, nullptr, nullptr, nullptr, n_records, max_motif_cap,
                             planes_on_device, out);
+}
+
+// .2bit records: record r = offsets[r + 1] - offsets[r] bases packed from byte rec_byte[r] of dna (the file's bytes), its
+// N blocks among the runs of offsets' position space.  The load sees record r at source position 4 rec_byte[r] (the
+// position of its first base in the bytes) and the runs moved there, split at record ends.
+extern "C" int crf_seq_load_2bit(crf_ctx *c, const uint8_t *dna, const uint64_t *rec_byte, const uint64_t *offsets,
+                                 uint32_t n_records, const uint64_t *runs, uint64_t n_runs, uint32_t max_motif_cap,
+                                 int dna_on_device, crf_seq **out) {
+    const char *who = "crf_seq_load_2bit";
+    CHECK(check_offsets(offsets, n_records, who));
+    if (!dna || !rec_byte || (n_runs && !runs)) { set_err("%s: null argument", who); return CRF_ERR_ARG; }
+    for (uint32_t r = 0; r < n_records; ++r)
+        if (offsets[r + 1] < offsets[r]) { set_err("%s: offsets must be non-decreasing", who); return CRF_ERR_ARG; }
+    for (uint64_t i = 0; i < n_runs; ++i)
+        if (runs[2 * i] >= runs[2 * i + 1] || (i && runs[2 * i] < runs[2 * i - 1])) {
+            set_err("%s: runs must be non-empty, ascending and disjoint (run %llu)", who, (unsigned long long)i);
+            return CRF_ERR_ARG;
+        }
+    std::vector<uint64_t> starts, lengths, moved;
+    try {
+        starts.resize(n_records);
+        lengths.resize(n_records);
+        for (uint32_t r = 0; r < n_records; ++r) {
+            starts[r] = 4 * rec_byte[r];
+            lengths[r] = offsets[r + 1] - offsets[r];
+        }
+        const uint64_t pos0 = offsets[0], pos1 = offsets[n_records];
+        uint64_t a_i = 0, b_i = n_runs;                                  // first run that ends after pos0
+        while (a_i < b_i) { const uint64_t m = (a_i + b_i) / 2; if (runs[2 * m + 1] <= pos0) a_i = m + 1; else b_i = m; }
+        bool sorted = true;
+        uint32_t r = 0;
+        for (uint64_t k = a_i; k < n_runs && runs[2 * k] < pos1; ++k) {
+            uint64_t a = std::max(runs[2 * k], pos0);
+            const uint64_t b = std::min(runs[2 * k + 1], pos1);
+            while (a < b) {
+                while (offsets[r + 1] <= a) ++r;
+                const uint64_t e = std::min(b, offsets[r + 1]);
+                const uint64_t m0 = starts[r] + (a - offsets[r]), m1 = starts[r] + (e - offsets[r]);
+                if (!moved.empty() && m0 < moved.back()) sorted = false;
+                moved.push_back(m0);
+                moved.push_back(m1);
+                a = e;
+            }
+        }
+        if (!sorted) {                                                   // records not in file order
+            std::vector<std::pair<uint64_t, uint64_t>> pairs(moved.size() / 2);
+            for (size_t j = 0; j < pairs.size(); ++j) pairs[j] = {moved[2 * j], moved[2 * j + 1]};
+            std::sort(pairs.begin(), pairs.end());
+            for (size_t j = 0; j < pairs.size(); ++j) {
+                moved[2 * j] = pairs[j].first;
+                moved[2 * j + 1] = pairs[j].second;
+                if (j && pairs[j].first < pairs[j - 1].second) { set_err("%s: records share bytes of dna", who); return CRF_ERR_ARG; }
+            }
+        }
+    } catch (const std::bad_alloc &) {
+        set_err("out of host memory");
+        return CRF_ERR_NOMEM;
+    }
+    LoadSource src;
+    src.twobit = dna;
+    src.nm_runs = moved.data(); src.n_runs = moved.size() / 2; src.runs_mode = true;
+    return load_checked(c, src, starts.data(), lengths.data(), nullptr, nullptr, n_records, max_motif_cap, dna_on_device, out, who);
 }
 
 extern "C" int crf_seq_load_packed(crf_ctx *c, const uint32_t *H, const uint32_t *L, const uint32_t *NM,
@@ -1910,6 +1988,7 @@ static cudaError_t preload_kernels() {
     if (e == cudaSuccess) e = preload(scan_kernel<16>);
     if (e == cudaSuccess) e = preload(pack_kernel);
     if (e == cudaSuccess) e = preload(repack_kernel);
+    if (e == cudaSuccess) e = preload(twobit_pack_kernel);
     if (e == cudaSuccess) e = preload(mask_runs_kernel);
     if (e == cudaSuccess) e = preload(exotic_apply_kernel);
     if (e == cudaSuccess) e = preload(tile_offsets_kernel);

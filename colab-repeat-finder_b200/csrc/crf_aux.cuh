@@ -139,6 +139,100 @@ __global__ void __launch_bounds__(256) repack_kernel(const RepackParams p) {
     p.X[w] = 0;
 }
 
+// ---- .2bit: the packed bases of a .2bit file -> the device layout.  Source position q is base q & 3 of byte q >> 2, the
+// first base in the top two bits, T=0 C=1 A=2 G=3: with (h, l) its two bits, the planes are H = ~(h ^ l), L = ~h.  The
+// N blocks arrive as the mask plane of the source positions (runs mode).  Same structure and result as repack_kernel, with
+// the source planes of a word made from its 8 bytes; X = 0 (a .2bit file holds only A, C, G, T and N). ---------------------
+struct TwoBitParams {
+    const uint8_t *dna;             // byte 0 holds source positions [src_base, src_base + 4)
+    uint64_t n_bytes;               // bytes of dna that may be read
+    const uint32_t *sN;             // mask plane; word 0 = source positions [src_base, src_base + 32)
+    uint64_t src_base;              // multiple of 32
+    const uint64_t *rec_src_start;  // source position of each record's first base
+    const uint32_t *rec_len;
+    const uint32_t *rec_dev_off;
+    uint32_t n_records;
+    uint32_t w_lo, w_hi;            // layout words this launch packs
+    uint32_t *H, *L, *NM, *X;
+};
+
+__device__ __forceinline__ uint32_t even_bits(uint64_t v) {     // bits 0, 2, 4, ... of v -> bits 0, 1, 2, ...
+    v &= 0x5555555555555555ull;
+    v = (v | (v >> 1)) & 0x3333333333333333ull;
+    v = (v | (v >> 2)) & 0x0F0F0F0F0F0F0F0Full;
+    v = (v | (v >> 4)) & 0x00FF00FF00FF00FFull;
+    v = (v | (v >> 8)) & 0x0000FFFF0000FFFFull;
+    return (uint32_t)(v | (v >> 16));
+}
+
+// the H / L planes of source word wi (bytes 8 wi .. 8 wi + 7)
+__device__ __forceinline__ void twobit_planes(const TwoBitParams &p, uint64_t wi, uint32_t &H, uint32_t &L) {
+    const uint64_t b0 = 8 * wi;
+    const uint8_t *s = p.dna + b0;
+    uint64_t x = 0;
+    if (b0 + 8 <= p.n_bytes && ((uintptr_t)s & 7) == 0) {
+        x = *reinterpret_cast<const uint64_t *>(s);
+    } else {
+        for (uint32_t j = 0; j < 8; ++j)
+            if (b0 + j < p.n_bytes) x |= (uint64_t)s[j] << (8 * j);
+    }
+    x = ((x >> 4) & 0x0F0F0F0F0F0F0F0Full) | ((x & 0x0F0F0F0F0F0F0F0Full) << 4);   // base j of the word -> bits 2j + 1, 2j
+    x = ((x >> 2) & 0x3333333333333333ull) | ((x & 0x3333333333333333ull) << 2);
+    const uint32_t h = even_bits(x >> 1), l = even_bits(x);
+    H = ~(h ^ l);
+    L = ~h;
+}
+
+__global__ void __launch_bounds__(256) twobit_pack_kernel(const TwoBitParams p) {
+    const uint32_t w = p.w_lo + blockIdx.x * blockDim.x + threadIdx.x;
+    if (w >= p.w_hi) return;
+    const uint32_t p0 = w << 5;
+    uint32_t h = 0, l = 0, nm = 0xFFFFFFFFu;                 // gaps and pads are masked
+    if (p.n_records) {
+        uint32_t lo = 0, hi = p.n_records - 1;               // last record that starts at or before p0
+        while (lo < hi) {
+            const uint32_t mid = (lo + hi + 1) >> 1;
+            if (p.rec_dev_off[mid] <= p0) lo = mid; else hi = mid - 1;
+        }
+        const uint64_t p1 = (uint64_t)p0 + 32;
+        for (uint32_t r = lo; r < p.n_records; ++r) {
+            const uint32_t dev0 = p.rec_dev_off[r];
+            if ((uint64_t)dev0 >= p1) break;
+            const uint64_t rec_end = (uint64_t)dev0 + p.rec_len[r];
+            const uint64_t a = max((uint64_t)p0, (uint64_t)dev0), b = min(p1, rec_end);
+            if (a >= b) continue;
+            const uint32_t nbits = (uint32_t)(b - a), place = (uint32_t)(a - p0);
+            const uint64_t sbit = p.rec_src_start[r] - p.src_base + (a - dev0);
+            const uint64_t wi = sbit >> 5;
+            const uint32_t sh = (uint32_t)sbit & 31u;
+            const uint32_t mask = nbits == 32 ? 0xFFFFFFFFu : ((1u << nbits) - 1u);
+            const uint64_t wj = (sh && nbits > 32u - sh) ? wi + 1 : wi;
+            uint32_t hi_, li_, hj, lj;
+            twobit_planes(p, wi, hi_, li_);
+            if (wj != wi) twobit_planes(p, wj, hj, lj); else { hj = hi_; lj = li_; }
+            const uint32_t eh = __funnelshift_r(hi_, hj, sh) & mask;
+            const uint32_t el = __funnelshift_r(li_, lj, sh) & mask;
+            const uint32_t en = __funnelshift_r(p.sN[wi], p.sN[wj], sh) & mask;
+            h |= eh << place;
+            l |= el << place;
+            nm = (nm & ~(mask << place)) | (en << place);
+        }
+    }
+    h &= ~nm;
+    l &= ~nm;
+    for (uint32_t m = nm; m;) {                               // aperiodic filler at masked positions (see pack_kernel)
+        const uint32_t b = __ffs(m) - 1;
+        m &= m - 1;
+        const uint32_t code = hash32(p0 + b) & 3;
+        h |= (code >> 1) << b;
+        l |= (code & 1) << b;
+    }
+    p.H[w] = h;
+    p.L[w] = l;
+    p.NM[w] = nm;
+    p.X[w] = 0;
+}
+
 // runs mode of a packed load: the mask plane from the sorted runs of masked positions [runs[2i], runs[2i+1]); one warp per
 // run (its lanes stride over the run's words; a genome has a few hundred long N blocks, a read set millions of single N's)
 __global__ void __launch_bounds__(256) mask_runs_kernel(const uint64_t *runs, uint32_t n_runs, uint32_t *NM) {

@@ -19,6 +19,7 @@
 #include <exception>
 #include <chrono>
 #include <functional>
+#include <mutex>
 #include <thread>
 
 struct crf_fasta {
@@ -34,8 +35,19 @@ struct crf_fasta {
     bool planes_pinned = false;
     bool want_pinned_planes = false;                     // crf_fasta_open(pinned & 3): page-lock the planes crf_fasta_packed makes
     std::vector<uint64_t> exotic;
-    int format = 0;                                      // 0 = FASTA, 1 = FASTQ
+    int format = 0;                                      // 0 = FASTA, 1 = FASTQ, 2 = .2bit
     uint8_t *quals = nullptr;                            // FASTQ, crf_fasta_open(pinned & 4): laid out like bases
+    // .2bit: the file's bytes as they are (mapped, or page-locked with pinned & 3), where each record's packed bases
+    // start, its N blocks and mask blocks as sorted disjoint runs of concatenated positions; the text (bases) is decoded
+    // on the first crf_fasta_data
+    const uint8_t *dna = nullptr;
+    uint64_t dna_size = 0;
+    void *dna_map = nullptr;
+    bool dna_pinned = false;
+    std::vector<uint64_t> rec_byte, n_runs, mask_runs;
+    std::mutex decode_mu;
+    int text_pinned = 0;                                 // the pinned argument of crf_fasta_open, for the decoded text
+    uint32_t n_threads = 1;
 };
 
 namespace fasta_detail {
@@ -480,6 +492,170 @@ static int parse_fastq(const char *path, const uint8_t *t, uint64_t n, uint64_t 
     return CRF_OK;
 }
 
+// ---- .2bit (UCSC) ----
+// Header: signature 0x1A412743, version (0: 32-bit index offsets, 1: 64-bit ones, faToTwoBit -long), record count,
+// reserved; a file with the signature in the other byte order has every integer swapped.  Index: per record a name size
+// byte, the name and the offset of the record.  A record: dnaSize, N block count, starts, sizes, mask block count, starts,
+// sizes, a reserved word, then (dnaSize + 3) / 4 bytes of packed bases, T=0 C=1 A=2 G=3, the first base in the top two
+// bits of its byte.  The bases stay packed in the file's bytes; the text is decoded only when a caller asks for it.
+static const uint32_t TWOBIT_SIG = 0x1A412743u;
+
+static bool is_twobit(const uint8_t *t, uint64_t n) {
+    if (n < 4) return false;
+    uint32_t v;
+    memcpy(&v, t, 4);
+    return v == TWOBIT_SIG || __builtin_bswap32(v) == TWOBIT_SIG;
+}
+
+// One record's blocks [start, start + size) as sorted, merged runs shifted by base (empty blocks dropped).
+static void merge_blocks(std::vector<std::pair<uint64_t, uint64_t>> &blk, uint64_t base, std::vector<uint64_t> &out) {
+    std::sort(blk.begin(), blk.end());
+    bool open = false;
+    uint64_t a = 0, b = 0;
+    for (const auto &x : blk) {
+        if (x.first == x.second) continue;
+        if (open && x.first <= b) { b = std::max(b, x.second); continue; }
+        if (open) { out.push_back(base + a); out.push_back(base + b); }
+        a = x.first; b = x.second; open = true;
+    }
+    if (open) { out.push_back(base + a); out.push_back(base + b); }
+}
+
+// Index, record headers and blocks of the .2bit file t[0, n) into fa, every count, offset and block checked against the
+// file size and dnaSize.  The bases are not touched.
+static int parse_twobit(const char *path, const uint8_t *t, uint64_t n, crf_fasta *fa) {
+    fa->format = 2;
+    uint32_t sig;
+    memcpy(&sig, t, 4);
+    const bool swap = sig != TWOBIT_SIG;
+    auto u32 = [&](uint64_t p) { uint32_t v; memcpy(&v, t + p, 4); return swap ? __builtin_bswap32(v) : v; };
+    auto u64 = [&](uint64_t p) { uint64_t v; memcpy(&v, t + p, 8); return swap ? __builtin_bswap64(v) : v; };
+    auto fail = [&](uint64_t rec, const char *why) {
+        set_err("crf_fasta_open: %s: .2bit record %llu: %s", path, (unsigned long long)rec, why);
+        return CRF_ERR_ARG;
+    };
+    if (n < 16) { set_err("crf_fasta_open: %s: the .2bit header is truncated", path); return CRF_ERR_ARG; }
+    const uint32_t version = u32(4), count = u32(8);
+    if (version > 1) { set_err("crf_fasta_open: %s: .2bit version %u (0 or 1 expected)", path, version); return CRF_ERR_ARG; }
+    const uint64_t off_bytes = version ? 8 : 4;
+    std::vector<uint64_t> rec_off;
+    rec_off.reserve(std::min<uint64_t>(count, n / 5));
+    uint64_t p = 16;
+    for (uint64_t r = 0; r < count; ++r) {
+        if (p >= n || n - p - 1 < t[p] + off_bytes) return fail(r + 1, "the index is truncated");
+        const uint32_t ns = t[p++];
+        fa->name_off.push_back(fa->names.size());
+        fa->names.insert(fa->names.end(), t + p, t + p + ns);
+        fa->names.push_back('\0');
+        p += ns;
+        rec_off.push_back(version ? u64(p) : u32(p));
+        p += off_bytes;
+    }
+    fa->offsets.assign((size_t)count + 1, 0);
+    fa->rec_byte.assign(count, 0);
+    std::vector<std::pair<uint64_t, uint64_t>> blk;
+    uint64_t total = 0;
+    for (uint64_t r = 0; r < count; ++r) {
+        const uint64_t off = rec_off[r];
+        if (off >= n) return fail(r + 1, "its offset is past the end of the file");
+        if (n - off < 8) return fail(r + 1, "its header runs past the end of the file");
+        const uint64_t dna_size = u32(off), nb = u32(off + 4);
+        uint64_t q = off + 8;
+        for (int kind = 0; kind < 2; ++kind) {                    // N blocks, then mask blocks
+            uint64_t cnt = nb;
+            if (kind) {
+                if (n - q < 4) return fail(r + 1, "its header runs past the end of the file");
+                cnt = u32(q);
+                q += 4;
+            }
+            if ((n - q) / 8 < cnt) return fail(r + 1, kind ? "its mask blocks run past the end of the file"
+                                                           : "its N blocks run past the end of the file");
+            blk.clear();
+            for (uint64_t i = 0; i < cnt; ++i) {
+                const uint64_t s = u32(q + 4 * i), z = u32(q + 4 * (cnt + i));
+                if (s + z > dna_size) return fail(r + 1, kind ? "a mask block ends past its dnaSize" : "an N block ends past its dnaSize");
+                blk.push_back({s, s + z});
+            }
+            merge_blocks(blk, total, kind ? fa->mask_runs : fa->n_runs);
+            q += 8 * cnt;
+        }
+        if (n - q < 4) return fail(r + 1, "its header runs past the end of the file");
+        q += 4;                                                   // reserved
+        if (n - q < (dna_size + 3) / 4) return fail(r + 1, "the file is shorter than its DNA");
+        fa->rec_byte[r] = q;
+        fa->offsets[r] = total;
+        total += dna_size;
+    }
+    fa->offsets[count] = fa->total = total;
+    // the records' bases may not share bytes: a load masks the N blocks by byte position
+    std::vector<uint32_t> order;
+    for (uint32_t r = 0; r < count; ++r)
+        if (fa->offsets[r + 1] > fa->offsets[r]) order.push_back(r);
+    std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return fa->rec_byte[a] < fa->rec_byte[b]; });
+    for (size_t i = 1; i < order.size(); ++i) {
+        const uint32_t a = order[i - 1], b = order[i];
+        if (fa->rec_byte[a] + (fa->offsets[a + 1] - fa->offsets[a] + 3) / 4 > fa->rec_byte[b]) {
+            set_err("crf_fasta_open: %s: .2bit record %u: its bases overlap those of record %u", path, std::max(a, b) + 1,
+                    std::min(a, b) + 1);
+            return CRF_ERR_ARG;
+        }
+    }
+    return CRF_OK;
+}
+
+// The text of a .2bit handle, what twoBitToFa writes: T/C/A/G, N blocks as 'N', mask blocks lower-cased ('n' inside
+// both).  Decoded once, on the reader's threads, in pieces of concatenated positions.
+static int twobit_decode(crf_fasta *fa) {
+    std::lock_guard<std::mutex> lock(fa->decode_mu);
+    if (fa->bases || fa->format != 2) return CRF_OK;
+    static const struct Lut {                                     // a byte -> its four letters
+        uint32_t v[256];
+        Lut() {
+            for (uint32_t b = 0; b < 256; ++b) {
+                uint8_t c[4];
+                for (int j = 0; j < 4; ++j) c[j] = (uint8_t)"TCAG"[(b >> (6 - 2 * j)) & 3];
+                memcpy(&v[b], c, 4);
+            }
+        }
+    } lut;
+    try {
+        if (!alloc_bases(fa, fa->total, fa->text_pinned)) {
+            set_err("crf_fasta_data: out of host memory (%llu bases)", (unsigned long long)fa->total);
+            return CRF_ERR_NOMEM;
+        }
+        const uint64_t PIECE = 4u << 20, total = fa->total;
+        const std::vector<uint64_t> &off = fa->offsets, &nr = fa->n_runs, &mr = fa->mask_runs;
+        uint8_t *out = fa->bases;
+        run_parallel(fa->n_threads, (total + PIECE - 1) / PIECE, [&](size_t i) {
+            const uint64_t lo = i * PIECE, hi = std::min(total, lo + PIECE);
+            uint64_t r = (uint64_t)(std::upper_bound(off.begin(), off.end(), lo) - off.begin()) - 1;
+            for (uint64_t pos = lo; pos < hi; ++r) {
+                if (off[r + 1] <= pos) continue;
+                const uint64_t i1 = std::min(hi, off[r + 1]) - off[r];
+                const uint8_t *d = fa->dna + fa->rec_byte[r];
+                uint8_t *o = out + off[r];
+                uint64_t j = pos - off[r];
+                for (; j < i1 && (j & 3); ++j) o[j] = (uint8_t)"TCAG"[(d[j >> 2] >> (6 - 2 * (j & 3))) & 3];
+                for (; j + 4 <= i1; j += 4) memcpy(o + j, &lut.v[d[j >> 2]], 4);
+                for (; j < i1; ++j) o[j] = (uint8_t)"TCAG"[(d[j >> 2] >> (6 - 2 * (j & 3))) & 3];
+                pos = off[r] + i1;
+            }
+            for (int kind = 0; kind < 2; ++kind) {                // mask blocks lower-case, then N blocks keep the case
+                const std::vector<uint64_t> &runs = kind ? nr : mr;
+                uint64_t a = 0, b = runs.size() / 2;              // first run that ends after lo
+                while (a < b) { const uint64_t m = (a + b) / 2; if (runs[2 * m + 1] <= lo) a = m + 1; else b = m; }
+                for (; a < runs.size() / 2 && runs[2 * a] < hi; ++a)
+                    for (uint64_t q = std::max(lo, runs[2 * a]), e = std::min(hi, runs[2 * a + 1]); q < e; ++q)
+                        out[q] = kind ? (uint8_t)((out[q] & 0x20) | 'N') : (uint8_t)(out[q] | 0x20);
+            }
+        });
+    } catch (const std::bad_alloc &) {
+        set_err("crf_fasta_data: out of host memory");
+        return CRF_ERR_NOMEM;
+    }
+    return CRF_OK;
+}
+
 }  // namespace fasta_detail
 
 static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf_fasta **out);
@@ -516,6 +692,44 @@ static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf
     const uint8_t *t = file.data;
     uint64_t n = file.size;
     if (n_threads == 0) n_threads = std::min(16u, std::max(1u, std::thread::hardware_concurrency()));
+    if (is_twobit(t, n)) {                              // (the raw file: a .2bit file is never compressed)
+        struct Guard {
+            crf_fasta *p;
+            ~Guard() { if (p) crf_fasta_close(p); }
+        } guard{new crf_fasta};
+        crf_fasta *fa = guard.p;
+        fa->n_threads = n_threads;
+        fa->text_pinned = pinned;
+        const int rc = parse_twobit(path, t, n, fa);
+        if (rc != CRF_OK) return rc;
+        lap("2bit-index");
+        void *p = nullptr;                              // pinned & 3: the bytes that get uploaded, page-locked
+        if ((pinned & 3) && cudaHostAlloc(&p, n, cudaHostAllocDefault) == cudaSuccess) {
+            const uint64_t PIECE = 64u << 20;
+            run_parallel(n_threads, (n + PIECE - 1) / PIECE, [&](size_t i) {
+                memcpy((uint8_t *)p + i * PIECE, t + i * PIECE, std::min(PIECE, n - i * PIECE));
+            });
+            fa->dna = (const uint8_t *)p;
+            fa->dna_pinned = true;
+            lap("2bit-pin");
+        } else {
+            if (pinned & 3) cudaGetLastError();
+            if (file.map) {                             // the mapping goes to the handle
+                fa->dna_map = file.map;
+                file.map = nullptr;
+                fa->dna = t;
+            } else {
+                uint8_t *own = (uint8_t *)malloc(std::max<uint64_t>(n, 1));
+                if (!own) throw std::bad_alloc();
+                memcpy(own, t, n);
+                fa->dna = own;
+            }
+        }
+        fa->dna_size = n;
+        guard.p = nullptr;
+        *out = fa;
+        return CRF_OK;
+    }
     if (n >= 2 && t[0] == 0x1f && t[1] == 0x8b) {
         bool bad = false;
         const bool bgzf = inflate_bgzf(file, n_threads, inflated, &bad);
@@ -683,10 +897,33 @@ extern "C" int crf_fasta_info(const crf_fasta *fa, uint64_t *n_records, uint64_t
 extern "C" int crf_fasta_data(const crf_fasta *fa, const uint8_t **bases, const uint64_t **offsets, const char **names,
                               uint64_t *names_bytes) {
     if (!fa) { set_err("null fasta handle"); return CRF_ERR_ARG; }
+    if (bases && fa->format == 2) {                     // a .2bit file's text: decoded once, under the handle's lock
+        const int rc = fasta_detail::twobit_decode(const_cast<crf_fasta *>(fa));
+        if (rc != CRF_OK) return rc;
+    }
     if (bases) *bases = fa->bases;
     if (offsets) *offsets = fa->offsets.data();
     if (names) *names = fa->names.data();
     if (names_bytes) *names_bytes = fa->names.size();
+    return CRF_OK;
+}
+
+extern "C" int crf_fasta_index(const crf_fasta *fa, const uint64_t **offsets, const char **names, uint64_t *names_bytes) {
+    if (!fa) { set_err("crf_fasta_index: null fasta handle"); return CRF_ERR_ARG; }
+    if (offsets) *offsets = fa->offsets.data();
+    if (names) *names = fa->names.data();
+    if (names_bytes) *names_bytes = fa->names.size();
+    return CRF_OK;
+}
+
+extern "C" int crf_fasta_twobit(const crf_fasta *fa, const uint8_t **dna, const uint64_t **rec_byte, const uint64_t **runs,
+                                uint64_t *n_runs) {
+    if (!fa || !dna || !rec_byte || !runs || !n_runs) { set_err("crf_fasta_twobit: null argument"); return CRF_ERR_ARG; }
+    if (fa->format != 2) { set_err("crf_fasta_twobit: not a .2bit file"); return CRF_ERR_ARG; }
+    *dna = fa->dna;
+    *rec_byte = fa->rec_byte.data();
+    *runs = fa->n_runs.data();
+    *n_runs = fa->n_runs.size() / 2;
     return CRF_OK;
 }
 
@@ -707,6 +944,9 @@ extern "C" int crf_fasta_close(crf_fasta *fa) {
     if (fa->pinned) cudaFreeHost(fa->bases);
     else free(fa->bases);
     free(fa->quals);
+    if (fa->dna_pinned) cudaFreeHost((void *)fa->dna);
+    else if (fa->dna_map) munmap(fa->dna_map, fa->dna_size);
+    else free((void *)fa->dna);
     if (fa->planes_pinned) cudaFreeHost(fa->planes);
     else free(fa->planes);
     delete fa;

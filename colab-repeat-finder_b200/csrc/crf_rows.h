@@ -1,6 +1,6 @@
 // Native BED / TSV row writer (host only): result rows -> text, replacing the per-row Python of
 // perfect_repeat_finder.py:148-149 (BED: chrom, start, end, motif) and :166-170 (TSV with header).  Rows are formatted on
-// several threads, the motif column read back from the host copy of the text.
+// several threads, the motif column read back from the host copy of the text (or from a .2bit file's packed bases).
 //
 // Included at the end of crf_api.cu (shares set_err()); tests/fuzz_reader.cpp compiles it without the CUDA runtime.
 #pragma once
@@ -23,9 +23,37 @@ static inline char *put_u64(char *p, uint64_t v) {
     return p;
 }
 
-// origin (may be null): per record, added to the printed start and end (the motif is still read at offsets[r] + start)
-static int write_rows_impl(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
-                           const uint64_t *offsets, const uint64_t *origin, const uint32_t *record, const uint32_t *start,
+// Where the motif column comes from: the text (one byte per base, upper-cased here) ...
+struct TextMotif {
+    const uint8_t *bases;
+    const uint64_t *offsets;
+    char *operator()(char *p, uint32_t r, uint32_t start, uint32_t k) const {
+        const uint8_t *m = bases + offsets[r] + start;
+        for (uint32_t j = 0; j < k; ++j) {
+            uint8_t c = m[j];
+            if (c >= 'a' && c <= 'z') c -= 32;
+            *p++ = (char)c;
+        }
+        return p;
+    }
+};
+
+// ... or a .2bit file's packed bases (record r's base i: bits 7-6 of byte rec_byte[r] + i / 4 for i % 4 == 0, then 5-4, ...;
+// T=0 C=1 A=2 G=3).  A motif never holds an N, so the codes alone give the letters the text has, upper-cased.
+struct TwoBitMotif {
+    const uint8_t *dna;
+    const uint64_t *rec_byte;
+    char *operator()(char *p, uint32_t r, uint32_t start, uint32_t k) const {
+        const uint8_t *d = dna + rec_byte[r];
+        for (uint64_t i = start, e = (uint64_t)start + k; i < e; ++i) *p++ = "TCAG"[(d[i >> 2] >> (6 - 2 * (i & 3))) & 3];
+        return p;
+    }
+};
+
+// origin (may be null): per record, added to the printed start and end (the motif is still read at start)
+template <class Motif>
+static int write_rows_impl(const char *path, int append, int tsv, const char *names, const Motif &motif,
+                           const uint64_t *origin, const uint32_t *record, const uint32_t *start,
                            const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
     FILE *f = fopen(path, append ? "ab" : "wb");
     if (!f) { set_err("crf_write_rows: cannot open %s", path); return CRF_ERR_ARG; }
@@ -69,12 +97,7 @@ static int write_rows_impl(const char *path, int append, int tsv, const char *na
             if (!tsv) { memcpy(p, name_ptr[r], name_len[r]); p += name_len[r]; *p++ = '\t'; }
             p = put_u64(p, o + start[i]); *p++ = '\t';
             p = put_u64(p, o + end[i]); *p++ = '\t';
-            const uint8_t *m = bases + offsets[r] + start[i];
-            for (uint32_t j = 0; j < k; ++j) {
-                uint8_t c = m[j];
-                if (c >= 'a' && c <= 'z') c -= 32;
-                *p++ = (char)c;
-            }
+            p = motif(p, r, start[i], k);
             *p++ = '\n';
         }
         return (size_t)(p - buf.data());
@@ -117,7 +140,8 @@ extern "C" int crf_write_rows_at(const char *path, int append, int tsv, const ch
         return CRF_ERR_ARG;
     }
     try {                                            // no exception crosses the C boundary
-        return write_rows_impl(path, append, tsv, names, bases, offsets, origin, record, start, end, motif_size, n_rows, bytes);
+        return write_rows_impl(path, append, tsv, names, TextMotif{bases, offsets}, origin, record, start, end, motif_size, n_rows,
+                               bytes);
     } catch (const std::bad_alloc &) {
         set_err("crf_write_rows: out of host memory");
         return CRF_ERR_NOMEM;
@@ -128,4 +152,22 @@ extern "C" int crf_write_rows(const char *path, int append, int tsv, const char 
                               const uint64_t *offsets, const uint32_t *record, const uint32_t *start,
                               const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
     return crf_write_rows_at(path, append, tsv, names, bases, offsets, nullptr, record, start, end, motif_size, n_rows, bytes);
+}
+
+// The rows of records read from a .2bit file (crf_fasta_twobit: dna, rec_byte), the motif read from the packed bases: the
+// same bytes crf_write_rows writes from the file's decoded text, without that text.
+extern "C" int crf_write_rows_twobit(const char *path, int append, int tsv, const char *names, const uint8_t *dna,
+                                     const uint64_t *rec_byte, const uint32_t *record, const uint32_t *start,
+                                     const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
+    if (!path || (n_rows && (!dna || !rec_byte || !record || !start || !end || !motif_size)) || (!tsv && !names)) {
+        set_err("crf_write_rows: null argument");
+        return CRF_ERR_ARG;
+    }
+    try {
+        return write_rows_impl(path, append, tsv, names, TwoBitMotif{dna, rec_byte}, nullptr, record, start, end, motif_size,
+                               n_rows, bytes);
+    } catch (const std::bad_alloc &) {
+        set_err("crf_write_rows: out of host memory");
+        return CRF_ERR_NOMEM;
+    }
 }

@@ -91,6 +91,15 @@ int crf_seq_load_packed_runs_ranges(crf_ctx *ctx, const uint32_t *H, const uint3
                                     const uint64_t *exotic, uint64_t n_exotic, const uint64_t *starts,
                                     const uint64_t *lengths, const uint64_t *own_lo, const uint64_t *own_hi,
                                     uint32_t n_records, uint32_t max_motif_cap, int planes_on_device, crf_seq **seq);
+/* Records of a .2bit file (crf_fasta_twobit), loaded from the file's packed bytes: record r holds offsets[r + 1] -
+ * offsets[r] bases packed from byte rec_byte[r] of dna, its N blocks among the ascending, disjoint runs [runs[2i],
+ * runs[2i+1]) of the position space of offsets (runs outside [offsets[0], offsets[n_records]) are ignored, so a load of
+ * some of the records takes the whole file's list).  The byte span the records cover (headers between them included) goes
+ * up at 0.25 B/bp, in chunks on a second stream while twobit_pack_kernel lays out the words whose bytes have arrived; the
+ * records may not share bytes.  The rows equal those of crf_seq_load_ascii on the decoded text (crf_fasta_data).
+ * dna_on_device != 0: dna is a device pointer to the file's bytes (rec_byte, offsets and runs stay host arrays). */
+int crf_seq_load_2bit(crf_ctx *ctx, const uint8_t *dna, const uint64_t *rec_byte, const uint64_t *offsets, uint32_t n_records,
+                      const uint64_t *runs, uint64_t n_runs, uint32_t max_motif_cap, int dna_on_device, crf_seq **seq);
 /* Host only: the maximal runs of set bits of an NM plane over [0, n_bases) (threaded).  *n_runs = how many there are
  * (CRF_ERR_CAPACITY if more than cap pairs: call again with a longer list). */
 int crf_mask_runs(const uint32_t *NM, uint64_t n_bases, uint32_t n_threads, uint64_t *runs, uint64_t cap, uint64_t *n_runs);
@@ -305,6 +314,13 @@ int crf_write_rows(const char *path, int append, int tsv, const char *names, con
 int crf_write_rows_at(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
                       const uint64_t *offsets, const uint64_t *origin, const uint32_t *record, const uint32_t *start,
                       const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes);
+/* crf_write_rows for records read from a .2bit file: the motif is read from the file's packed bases (dna and rec_byte as
+ * crf_fasta_twobit gives them: record r's base i is bits 7-6 of byte rec_byte[r] + i / 4 for i % 4 == 0, then 5-4, 3-2,
+ * 1-0; T=0 C=1 A=2 G=3) as upper-case A/C/G/T.  A motif never holds an N, so the output is byte-identical to
+ * crf_write_rows on the file's decoded text (crf_fasta_data). */
+int crf_write_rows_twobit(const char *path, int append, int tsv, const char *names, const uint8_t *dna,
+                          const uint64_t *rec_byte, const uint32_t *record, const uint32_t *start, const uint32_t *end,
+                          const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes);
 /* A repeat-masked FASTA file: per record a header line ">name" (names NUL-separated, as crf_write_rows takes them), then
  * its bases, line_width per line.  Mask bit p (as crf_mask_rows lays it out) stands for bases[p], with the indexing of
  * offsets (record r = bases[offsets[r] .. offsets[r+1])).  A masked byte is lower-cased when it is an ASCII letter A-Z
@@ -335,11 +351,24 @@ int crf_fasta_open(const char *path, uint32_t n_threads, int pinned, crf_fasta *
 int crf_fasta_info(const crf_fasta *fasta, uint64_t *n_records, uint64_t *total_bases, int *pinned);
 int crf_fasta_data(const crf_fasta *fasta, const uint8_t **bases, const uint64_t **offsets, const char **names,
                    uint64_t *names_bytes);
-/* *format = 0 for a FASTA file, 1 for a FASTQ file. */
+/* UCSC .2bit too: a file that starts with the signature 0x1A412743 (either byte order; version 0, or 1 with 64-bit index
+ * offsets) is read as .2bit.  Only its index and record headers are parsed at open: every count, offset and block is
+ * checked against the file size and dnaSize, and a bad file is CRF_ERR_ARG naming the 1-based record.  N blocks and mask
+ * blocks may be unsorted or overlap; they are merged per record.  crf_fasta_data then decodes the text on first call (on the
+ * reader's threads): what twoBitToFa writes, T/C/A/G, N blocks as 'N', mask blocks lower-cased ('n' inside both).
+ * *format = 0 for a FASTA file, 1 for a FASTQ file, 2 for a .2bit file. */
 int crf_fasta_format(const crf_fasta *fasta, int *format);
 /* A FASTQ file's qualities, laid out like the bases (record r = quals[offsets[r] .. offsets[r+1])); NULL for a FASTA
  * file or when crf_fasta_open was not given pinned bit 2. */
 int crf_fasta_quals(const crf_fasta *fasta, const uint8_t **quals);
+/* Offsets (n_records + 1) and NUL-separated names of any handle, without decoding a .2bit file's bases. */
+int crf_fasta_index(const crf_fasta *fasta, const uint64_t **offsets, const char **names, uint64_t *names_bytes);
+/* A .2bit handle's packed form (CRF_ERR_ARG for any other): dna = the file's bytes (page-locked when crf_fasta_open had
+ * pinned & 3, else mapped), rec_byte[r] = the byte where record r's packed bases start, runs = its N blocks as n_runs
+ * ascending, disjoint runs [runs[2i], runs[2i+1]) of the position space of the offsets (merged within a record, not across
+ * records) -- what crf_seq_load_2bit and crf_write_rows_twobit take. */
+int crf_fasta_twobit(const crf_fasta *fasta, const uint8_t **dna, const uint64_t **rec_byte, const uint64_t **runs,
+                     uint64_t *n_runs);
 /* Packed planes of the whole file (all records back to back, as crf_seq_load_packed takes them), made on first call
  * and owned by the handle; page-locked when the base buffer is. */
 int crf_fasta_packed(crf_fasta *fasta, uint32_t n_threads, const uint32_t **H, const uint32_t **L, const uint32_t **NM,
