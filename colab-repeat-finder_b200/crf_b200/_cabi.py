@@ -29,11 +29,11 @@ EXPORTS = [
     "crf_last_error", "crf_abi_version", "crf_ctx_create", "crf_ctx_destroy", "crf_ctx_set_stream",
     "crf_ctx_synchronize", "crf_load_limit", "crf_seq_load_packed", "crf_seq_load_packed_ranges", "crf_pack_ascii",
     "crf_seq_load_packed_runs", "crf_seq_load_packed_runs_ranges", "crf_mask_runs",
-    "crf_fasta_packed", "crf_seq_load_2bit", "crf_seq_load_ascii", "crf_seq_load_ascii_ranges", "crf_seq_set_output_map", "crf_seq_destroy", "crf_seq_info", "crf_scan", "crf_fetch",
+    "crf_fasta_packed", "crf_seq_load_2bit", "crf_seq_load_nibbles", "crf_seq_load_ascii", "crf_seq_load_ascii_ranges", "crf_seq_set_output_map", "crf_seq_destroy", "crf_seq_info", "crf_scan", "crf_fetch",
     "crf_scan_stats", "crf_run_end", "crf_interval_stop", "crf_fetch_open", "crf_patch_end", "crf_write_rows",
-    "crf_write_rows_at", "crf_write_rows_twobit", "crf_mask_rows", "crf_write_fasta_masked", "crf_write_fastq_masked",
+    "crf_write_rows_at", "crf_write_rows_twobit", "crf_write_rows_nibbles", "crf_mask_rows", "crf_write_fasta_masked", "crf_write_fastq_masked",
     "crf_fasta_open", "crf_fasta_info", "crf_fasta_data", "crf_fasta_format", "crf_fasta_quals", "crf_fasta_index",
-    "crf_fasta_twobit", "crf_fasta_close",
+    "crf_fasta_twobit", "crf_fasta_nibbles", "crf_fasta_close",
     "crf_gunzip",
     "crf_xchg_create", "crf_xchg_destroy", "crf_xchg_export", "crf_xchg_connect_ipc", "crf_xchg_connect_local",
     "crf_xchg_set_timeout", "crf_xchg_set_compact", "crf_scan_gather", "crf_xchg_push", "crf_xchg_wait", "crf_xchg_step_result", "crf_xchg_fetch",
@@ -108,6 +108,7 @@ def lib():
         L.crf_mask_runs.argtypes = [vp, u64, u32, vp, u64, P(u64)]
         L.crf_fasta_packed.argtypes = [vp, u32, P(vp), P(vp), P(vp), P(vp), P(u64)]
         L.crf_seq_load_2bit.argtypes = [vp, vp, vp, vp, u32, vp, u64, u32, i, P(vp)]
+        L.crf_seq_load_nibbles.argtypes = [vp, vp, vp, vp, u32, vp, u64, u32, i, P(vp)]
         L.crf_seq_set_output_map.argtypes = [vp, vp, vp, vp]
         L.crf_seq_destroy.argtypes = [vp]
         L.crf_seq_info.argtypes = [vp, P(SeqInfo)]
@@ -121,6 +122,7 @@ def lib():
         L.crf_write_rows.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
         L.crf_write_rows_at.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
         L.crf_write_rows_twobit.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
+        L.crf_write_rows_nibbles.argtypes = [ctypes.c_char_p, i, i, vp, vp, vp, vp, vp, vp, vp, u64, P(u64)]
         L.crf_mask_rows.argtypes = [vp, vp, vp, vp, u64, i, vp, u32, vp, u64, i]
         L.crf_write_fasta_masked.argtypes = [ctypes.c_char_p, vp, vp, vp, u64, vp, i, u32, P(u64)]
         L.crf_write_fastq_masked.argtypes = [ctypes.c_char_p, vp, vp, vp, vp, u64, vp, i, P(u64)]
@@ -131,6 +133,7 @@ def lib():
         L.crf_fasta_quals.argtypes = [vp, P(vp)]
         L.crf_fasta_index.argtypes = [vp, P(vp), P(vp), P(u64)]
         L.crf_fasta_twobit.argtypes = [vp, P(vp), P(vp), P(vp), P(u64)]
+        L.crf_fasta_nibbles.argtypes = [vp, P(vp), P(vp), P(vp), P(u64)]
         L.crf_fasta_close.argtypes = [vp]
         L.crf_gunzip.argtypes = [vp, ctypes.c_uint64, vp, ctypes.c_uint64, ctypes.POINTER(ctypes.c_uint64), ctypes.c_int]
         L.crf_xchg_create.argtypes = [vp, u32, u32, u64, P(vp)]
@@ -226,6 +229,14 @@ class Context:
             source = source.twobit()
         return Sequence(self, None, None, max_motif_cap, on_device, twobit=source)
 
+    def load_nibbles(self, source, max_motif_cap=50, on_device=False):
+        """crf_seq_load_nibbles: the reads of a BAM file, loaded from their 4-bit codes.  source: a BAM Fasta, or a
+        NibbleSource (Fasta.nibbles(), .records(first, last) for some of them) whose nib may also be a CUDA uint8 tensor
+        holding the codes, or a device pointer (int) with on_device=True."""
+        if isinstance(source, Fasta):
+            source = source.nibbles()
+        return Sequence(self, None, None, max_motif_cap, on_device, nibbles=source)
+
     @_serialised
     def mask_rows(self, record, start, end, dst_offset, mask_bits, n_rows=None, mask=None):
         """crf_mask_rows: the union of the rows [dst_offset[record] + start, dst_offset[record] + end) as a bit mask.
@@ -264,32 +275,36 @@ class Sequence:
     """Records resident in HBM as packed planes (crf_seq)."""
 
     @_serialised
-    def __init__(self, ctx, bases, offsets, max_motif_cap, on_device, ranges=None, packed=None, twobit=None):
+    def __init__(self, ctx, bases, offsets, max_motif_cap, on_device, ranges=None, packed=None, twobit=None,
+                 nibbles=None):
         self.ctx = ctx
         self._h = ctypes.c_void_p()
         keep = None
+        if nibbles is not None:
+            src = nibbles
+            ptr, on_device = _source_bytes("nib", src.nib, on_device)
+            offsets = np.ascontiguousarray(src.offsets, dtype=np.uint64)
+            rec_byte = np.ascontiguousarray(src.rec_byte, dtype=np.uint64)
+            exotic = np.ascontiguousarray(src.exotic, dtype=np.uint64)
+            if offsets.ndim != 1 or offsets.size < 2 or rec_byte.shape != (offsets.size - 1,):
+                raise ValueError("a BAM source needs n_records + 1 offsets and n_records rec_byte entries")
+            _check_extent("nib", src.nib, rec_byte, offsets, 2)
+            self.offsets = offsets
+            self.n_records = offsets.size - 1
+            _check(lib().crf_seq_load_nibbles(ctx._h, ctypes.c_void_p(ptr), ctypes.c_void_p(rec_byte.ctypes.data),
+                                              ctypes.c_void_p(offsets.ctypes.data), self.n_records,
+                                              ctypes.c_void_p(exotic.ctypes.data if exotic.size else 0), exotic.size,
+                                              int(max_motif_cap), int(bool(on_device)), ctypes.byref(self._h)))
+            return
         if twobit is not None:
             src = twobit
-            dna = src.dna
-            if hasattr(dna, "data_ptr"):                  # a torch tensor holding the file's bytes
-                if str(dna.dtype) != "torch.uint8" or not dna.is_contiguous():
-                    raise ValueError("dna must be a contiguous torch.uint8 tensor")
-                if dna.is_cuda:
-                    import torch
-                    torch.cuda.current_stream(dna.device).synchronize()     # its bytes are written before the upload
-                    on_device = True
-                ptr = dna.data_ptr()
-            elif isinstance(dna, int):
-                if not on_device:
-                    raise ValueError("a pointer as dna needs on_device=True")
-                ptr = dna
-            else:
-                ptr, _ = _host_bytes("dna", dna)
+            ptr, on_device = _source_bytes("dna", src.dna, on_device)
             offsets = np.ascontiguousarray(src.offsets, dtype=np.uint64)
             rec_byte = np.ascontiguousarray(src.rec_byte, dtype=np.uint64)
             runs = np.ascontiguousarray(src.runs, dtype=np.uint64).reshape(-1, 2)
             if offsets.ndim != 1 or offsets.size < 2 or rec_byte.shape != (offsets.size - 1,):
                 raise ValueError("a .2bit source needs n_records + 1 offsets and n_records rec_byte entries")
+            _check_extent("dna", src.dna, rec_byte, offsets, 4)
             self.offsets = offsets
             self.n_records = offsets.size - 1
             _check(lib().crf_seq_load_2bit(ctx._h, ctypes.c_void_p(ptr), ctypes.c_void_p(rec_byte.ctypes.data),
@@ -669,15 +684,31 @@ class TwoBitSource:
         return TwoBitSource(self.dna, self.rec_byte[first:last], self.offsets[first:last + 1], self.runs, self._keep)
 
 
+class NibbleSource:
+    """The packed form of a BAM file's reads, what crf_seq_load_nibbles and crf_write_rows_nibbles take: nib (4-bit codes
+    =ACMGRSVTWYHKDBN, high nibble first: a host uint8 array, a CUDA torch.uint8 tensor, or a device pointer), rec_byte[r]
+    (the byte where record r's codes start), offsets (n_records + 1, the records' position space) and exotic (codes other
+    than A, C, G, T, N as position << 8 | letter, ascending, in that space)."""
+
+    def __init__(self, nib, rec_byte, offsets, exotic, keep=None):
+        self.nib, self.rec_byte, self.offsets, self.exotic = nib, rec_byte, offsets, exotic
+        self._keep = keep
+
+    def records(self, first, last):
+        """Records [first, last) (the exotic list stays whole: a load ignores entries outside its records)."""
+        return NibbleSource(self.nib, self.rec_byte[first:last], self.offsets[first:last + 1], self.exotic, self._keep)
+
+
 class Fasta:
-    """A FASTA, FASTQ or .2bit file read by the native reader (crf_fasta_open): `bases` (uint8 view of all records back
-    to back, owned by the library until close(); a .2bit file's text is decoded on first use), `offsets` (n_records+1,
-    uint64), `names` (list of str), `names_blob` (NUL-separated, as crf_write_rows takes them), `format` ("fasta" /
-    "fastq" / "2bit") and `quals` (a FASTQ file's qualities as a uint8 view laid out like `bases`, or None)."""
+    """A FASTA, FASTQ, .2bit or BAM file read by the native reader (crf_fasta_open): `bases` (uint8 view of all records
+    back to back, owned by the library until close(); a .2bit or BAM file's text is decoded on first use), `offsets`
+    (n_records+1, uint64), `names` (list of str), `names_blob` (NUL-separated, as crf_write_rows takes them), `format`
+    ("fasta" / "fastq" / "2bit" / "bam") and `quals` (a FASTQ or BAM file's qualities as a uint8 view laid out like
+    `bases`, or None)."""
 
     def __init__(self, path, n_threads=0, pinned=False, qualities=False):
         """pinned: False / True (page-locked base buffer and planes) / 2 (page-locked planes only: the text stays pageable).
-        qualities: keep a FASTQ file's qualities (else they are checked and dropped: no host memory for them)."""
+        qualities: keep a FASTQ or BAM file's qualities (else they are dropped: no host memory for them)."""
         self._h = ctypes.c_void_p()
         _check(lib().crf_fasta_open(os.fsencode(path), n_threads, int(pinned) | (4 if qualities else 0),
                                     ctypes.byref(self._h)))
@@ -694,13 +725,14 @@ class Fasta:
         fmt, quals = ctypes.c_int(), ctypes.c_void_p()
         _check(lib().crf_fasta_format(self._h, ctypes.byref(fmt)))
         _check(lib().crf_fasta_quals(self._h, ctypes.byref(quals)))
-        self.format = {1: "fastq", 2: "2bit"}.get(fmt.value, "fasta")
+        self.format = {1: "fastq", 2: "2bit", 3: "bam"}.get(fmt.value, "fasta")
         self.quals = np.ctypeslib.as_array(ctypes.cast(quals, ctypes.POINTER(ctypes.c_uint8)),
                                            shape=(max(self.total_bases, 1),))[:self.total_bases] if quals.value else None
 
     @property
     def bases(self):
-        """uint8 view of all records back to back (crf_fasta_data; a .2bit file's text is decoded on the first call)."""
+        """uint8 view of all records back to back (crf_fasta_data; a .2bit or BAM file's text is decoded on the first
+        call)."""
         if self._bases is None and self._h:
             bases = ctypes.c_void_p()
             _check(lib().crf_fasta_data(self._h, ctypes.byref(bases), None, None, None))
@@ -724,6 +756,22 @@ class Fasta:
         view = np.ctypeslib.as_array(ctypes.cast(dna, ctypes.POINTER(ctypes.c_uint8)), shape=(max(size, 1),))[:size] \
             if dna.value else np.zeros(0, np.uint8)
         return TwoBitSource(view, rb, self.offsets, rn, keep=self)
+
+    def nibbles(self):
+        """NibbleSource of a BAM file (crf_fasta_nibbles; ValueError for any other format).  nib is a view of the handle's
+        codes, valid until close()."""
+        nib, rec_byte, ex, n_ex = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_uint64()
+        _check(lib().crf_fasta_nibbles(self._h, ctypes.byref(nib), ctypes.byref(rec_byte), ctypes.byref(ex),
+                                       ctypes.byref(n_ex)))
+        def u64s(ptr, n):
+            return np.ctypeslib.as_array(ctypes.cast(ptr, ctypes.POINTER(ctypes.c_uint64)), shape=(n,)).copy() \
+                if n else np.zeros(0, np.uint64)
+        rb = u64s(rec_byte, self.n_records)
+        lengths = np.diff(self.offsets.astype(np.int64))
+        size = int((rb.astype(np.int64) + (lengths + 1) // 2).max()) if self.n_records else 0
+        view = np.ctypeslib.as_array(ctypes.cast(nib, ctypes.POINTER(ctypes.c_uint8)), shape=(max(size, 1),))[:size] \
+            if nib.value else np.zeros(0, np.uint8)
+        return NibbleSource(view, rb, self.offsets, u64s(ex, n_ex.value), keep=self)
 
     @property
     def names(self):
@@ -808,6 +856,58 @@ def write_rows_twobit(path, names, dna, rec_byte, record, start, end, k, tsv=Fal
                                        ctypes.c_void_p(dptr), ctypes.c_void_p(rec_byte.ctypes.data),
                                        *(ctypes.c_void_p(a.ctypes.data) for a in arrs), len(arrs[0]), ctypes.byref(nbytes)))
     return nbytes.value
+
+
+def write_rows_nibbles(path, names, nib, rec_byte, record, start, end, k, tsv=False, append=False):
+    """crf_write_rows_nibbles: write_rows for reads of a BAM file, the motif read from the 4-bit codes (nib: host uint8
+    array, rec_byte[r]: where record r's codes start, as NibbleSource has them)."""
+    if isinstance(names, (bytes, bytearray)):
+        blob = bytes(names)
+    else:
+        blob = b"".join(n.encode("utf-8") + b"\0" for n in names) if names is not None else None
+    arrs = [np.ascontiguousarray(a, dtype=np.uint32) for a in (record, start, end, k)]
+    rec_byte = np.ascontiguousarray(rec_byte, dtype=np.uint64)
+    nptr, _ = _host_bytes("nib", nib)
+    nbytes = ctypes.c_uint64()
+    _check(lib().crf_write_rows_nibbles(os.fsencode(path), int(append), int(tsv),
+                                        ctypes.cast(ctypes.c_char_p(blob), ctypes.c_void_p) if blob is not None else None,
+                                        ctypes.c_void_p(nptr), ctypes.c_void_p(rec_byte.ctypes.data),
+                                        *(ctypes.c_void_p(a.ctypes.data) for a in arrs), len(arrs[0]), ctypes.byref(nbytes)))
+    return nbytes.value
+
+
+def _check_extent(what, buf, rec_byte, offsets, per_byte):
+    """ValueError unless every non-empty record's packed bytes, rec_byte[r] .. rec_byte[r] + ceil(length / per_byte), lie
+    inside buf (not checked for a device pointer given as an int: its size is unknown)."""
+    if isinstance(buf, int):
+        return
+    size = buf.numel() if hasattr(buf, "numel") else len(buf)
+    lengths = np.diff(offsets.astype(np.int64))
+    if (lengths < 0).any():
+        raise ValueError("offsets must be non-decreasing")
+    full = lengths > 0
+    if full.any():
+        end = rec_byte.astype(np.int64)[full] + (lengths[full] + per_byte - 1) // per_byte
+        if int(end.max()) > size:
+            raise ValueError(f"a record's bytes run past the end of {what} ({int(end.max())} > {size} bytes)")
+
+
+def _source_bytes(what, buf, on_device):
+    """(address, on_device) of the bytes a .2bit or BAM load reads: a torch uint8 tensor (a CUDA one is read on the
+    device), a device pointer (int, with on_device=True), or host bytes / a uint8 array."""
+    if hasattr(buf, "data_ptr"):
+        if str(buf.dtype) != "torch.uint8" or not buf.is_contiguous():
+            raise ValueError(f"{what} must be a contiguous torch.uint8 tensor")
+        if buf.is_cuda:
+            import torch
+            torch.cuda.current_stream(buf.device).synchronize()     # its bytes are written before the upload
+            on_device = True
+        return buf.data_ptr(), on_device
+    if isinstance(buf, int):
+        if not on_device:
+            raise ValueError(f"a pointer as {what} needs on_device=True")
+        return buf, on_device
+    return _host_bytes(what, buf)[0], on_device
 
 
 def _host_bytes(what, buf):

@@ -4,7 +4,8 @@ Same flags, defaults, stdout lines and output files as the reference's main()
 (the reference's perfect_repeat_finder.py:83-179), re-organised around two code paths:
 
   FASTA file  -> <basename(prefix)>.bed in the working directory (chrom, start_0based, end, motif); a FASTQ file is
-                 read the same way, its read names as chrom; a .2bit file too, loaded from its packed bytes
+                 read the same way, its read names as chrom; a .2bit file too, loaded from its packed bytes, and an
+                 unaligned BAM file, loaded from its 4-bit codes
   raw string  -> <prefix>.tsv with a header line (start_0based, end, motif)
 
 Deliberate deviations (SURVEY.md section 8b):
@@ -51,7 +52,8 @@ _OTHER_OPTIONS = [
     (("--mask",), dict(choices=("soft", "hard"), help="Also write <basename(prefix)>.masked.fa (FASTA input only, not with "
                                                       "--interval / --intervals): the records with every base inside a "
                                                       "reported repeat lower-cased (soft) or replaced by N (hard).  For "
-                                                      "FASTQ input: <basename(prefix)>.masked.fq, qualities unchanged.")),
+                                                      "FASTQ or BAM input: <basename(prefix)>.masked.fq, qualities "
+                                                      "unchanged.")),
 ]
 
 
@@ -63,8 +65,9 @@ def build_parser():
         filters.add_argument(*flags, **kw)
     for flags, kw in _OTHER_OPTIONS:
         parser.add_argument(*flags, **kw)
-    parser.add_argument("input_sequence", help="A nucleotide string, or the path of a FASTA or FASTQ file (plain or .gz) "
-                                               "or of a UCSC .2bit file")
+    parser.add_argument("input_sequence", help="A nucleotide string, or the path of a FASTA or FASTQ file (plain or .gz), "
+                                               "of a UCSC .2bit file or of an unaligned BAM file (read as `samtools "
+                                               "fastq -n` writes it)")
     return parser
 
 
@@ -128,18 +131,25 @@ def _whole_fasta_to_bed(fa, args, bed_path, mask_rows=None):
     groups = group_records(lengths, args.max_motif_size)
     # a .2bit file on one GPU: each group is loaded from the file's packed bytes (0.25 B/bp, packed into the layout on the
     # device) and its motifs are read from them; the text is never decoded
-    twobit = fa.twobit() if fa.format == "2bit" and len(devices) == 1 else None
-    if twobit is not None and all(not lengths[f:l].size or int(lengths[f:l].max()) + args.max_motif_size <= limit
-                                  for f, l in groups):
+    # (a BAM file the same way, from its 4-bit codes at 0.5 B/bp)
+    packed_src = None
+    if len(devices) == 1 and fa.format == "2bit":
+        packed_src, load, write = fa.twobit(), "load_2bit", _cabi.write_rows_twobit
+    elif len(devices) == 1 and fa.format == "bam":
+        packed_src, load, write = fa.nibbles(), "load_nibbles", _cabi.write_rows_nibbles
+    if packed_src is not None and all(not lengths[f:l].size or int(lengths[f:l].max()) + args.max_motif_size <= limit
+                                      for f, l in groups):
+        data = packed_src.dna if fa.format == "2bit" else packed_src.nib
         for first, last in groups:
             if not int(lengths[first:last].sum()):
                 continue
-            with api.get_context(devices[0]).load_2bit(twobit.records(first, last), max_motif_cap=args.max_motif_size) as seq:
+            with getattr(api.get_context(devices[0]), load)(packed_src.records(first, last),
+                                                            max_motif_cap=args.max_motif_size) as seq:
                 n = seq.scan(args.min_motif_size, args.max_motif_size, args.min_repeats, args.min_span)
                 rec, start, end, k = seq.fetch(n)
             whole_file = first == 0 and last == fa.n_records
-            _cabi.write_rows_twobit(bed_path, fa.names_blob if whole_file else fa.names[first:last], twobit.dna,
-                                    twobit.rec_byte[first:last], rec, start, end, k, append=True)
+            write(bed_path, fa.names_blob if whole_file else fa.names[first:last], data, packed_src.rec_byte[first:last],
+                  rec, start, end, k, append=True)
             if mask_rows is not None:
                 mask_rows.append((rec, start, end, fa.offsets[first:last]))
             counts[first:last] += np.bincount(rec.astype(np.int64, copy=False), minlength=last - first)
@@ -282,9 +292,11 @@ def _intervals_to_bed(parser, fa, args, bed_path):
 def default_prefix(path, fmt):
     """The output prefix when -o is not given.  FASTA: the (unanchored) regex of prf:114, as the reference has it.  FASTQ:
     the path without a trailing .fastq / .fq, optionally followed by .gz / .bgz (reads.fq.gz -> reads).  .2bit: the path
-    without a trailing .2bit."""
+    without a trailing .2bit.  BAM: the path without a trailing .bam."""
     if fmt == "2bit":
         return re.sub(r"\.2bit$", "", path)
+    if fmt == "bam":
+        return re.sub(r"\.bam$", "", path)
     if fmt == "fastq":
         return re.sub(r"\.(fastq|fq)(\.(gz|bgz))?$", "", path)
     return re.sub(".fa(sta)?(.gz)?", "", path)
@@ -297,12 +309,12 @@ def _run_fasta(parser, args):
         parser.error("--mask writes whole records: it cannot be used with --interval or --intervals")
     mask_rows = [] if args.mask else None
     # (page-locked planes only: the planes are what is uploaded, the text stays on the host for the motif column; a FASTQ
-    # file's qualities are kept only for the masked FASTQ)
+    # or BAM file's qualities are kept only for the masked FASTQ)
     with fasta.open_fasta(args.input_sequence, pinned=2, qualities=bool(args.mask)) as fa:
         if not args.output_prefix:                                                 # FASTA or FASTQ: known once it is read
             args.output_prefix = default_prefix(args.input_sequence, fa.format)
         bed_path = f"{os.path.basename(args.output_prefix)}.bed"                   # always in the working directory
-        mask_path = f"{os.path.basename(args.output_prefix)}.masked.{'fq' if fa.format == 'fastq' else 'fa'}" \
+        mask_path = f"{os.path.basename(args.output_prefix)}.masked.{'fq' if fa.format in ('fastq', 'bam') else 'fa'}" \
             if args.mask else None
         if args.intervals:
             _intervals_to_bed(parser, fa, args, bed_path)
@@ -343,7 +355,7 @@ def _run_fasta(parser, args):
                     for n_, l_, c_ in zip(names[lo:lo + 65536], lengths[lo:lo + 65536], counts[lo:lo + 65536])))
         if mask_rows is not None:                                  # every record has been scanned: paint once, write
             words = _paint_mask(api.get_context(parse_devices(getattr(args, "devices", None))[0]), mask_rows, fa.total_bases)
-            if fa.format == "fastq":
+            if fa.format in ("fastq", "bam"):
                 _cabi.write_fastq_masked(mask_path, fa.names_blob, fa.bases, fa.quals, fa.offsets, words,
                                          hard=args.mask == "hard")
             else:

@@ -2,7 +2,8 @@
 (perfect_repeat_finder.py:117-137 uses only `.name` -- the first whitespace-delimited token of the header --
 and `.seq`, the record's lines joined without line ends, case preserved).  Plain or gzip input.  A FASTQ file (first
 byte that is not whitespace: '@') is read too: read names and sequences in the same layout, qualities on request.  So is a
-UCSC .2bit file, whose text (what twoBitToFa writes) is decoded on first use of `bases`."""
+UCSC .2bit file, whose text (what twoBitToFa writes) is decoded on first use of `bases`, and an unaligned BAM file (the
+reads `samtools fastq -n` writes from it, kept as 4-bit codes until `bases` is first used)."""
 import os
 
 from . import _cabi

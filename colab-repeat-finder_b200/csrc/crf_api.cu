@@ -356,7 +356,8 @@ static uint64_t layout_limit(uint32_t max_motif_cap) {
 // One load holds at most this many layout positions: sum over records of (length + max_motif_cap).
 extern "C" uint64_t crf_load_limit(uint32_t max_motif_cap) { return layout_limit(max_motif_cap); }
 
-// What a load reads: ASCII bytes (one per base), planes packed on the host (crf_pack_ascii), or the bytes of a .2bit file.
+// What a load reads: ASCII bytes (one per base), planes packed on the host (crf_pack_ascii), the bytes of a .2bit file, or
+// the 4-bit codes of BAM reads.
 struct LoadSource {
     const uint8_t *bases = nullptr;                     // ASCII
     const uint32_t *pH = nullptr, *pL = nullptr, *pN = nullptr;   // packed: source position p = bit p & 31 of word p >> 5
@@ -366,7 +367,8 @@ struct LoadSource {
     uint64_t n_runs = 0;                                //   [runs[2i], runs[2i+1]) -- 0.25 B/bp cross PCIe instead of 0.375
     bool runs_mode = false;
     const uint8_t *twobit = nullptr;                    // .2bit (runs mode): source position p = base p & 3 of byte p >> 2
-    bool packed() const { return pH != nullptr || twobit != nullptr; }
+    const uint8_t *nibbles = nullptr;                   // BAM codes: source position p = nibble p & 1 of byte p >> 1
+    bool packed() const { return pH != nullptr || twobit != nullptr || nibbles != nullptr; }
 };
 
 // The two passes over the per-record arrays of a load run on a few threads when there are millions of records.
@@ -403,7 +405,8 @@ struct LoadTrace {
 static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, const uint64_t *lengths,
                      const uint64_t *own_lo, const uint64_t *own_hi, uint32_t n_records, uint32_t max_motif_cap,
                      int on_device, crf_seq *s) {
-    const char *who = src.twobit ? "crf_seq_load_2bit" : src.packed() ? "crf_seq_load_packed" : "crf_seq_load_ascii";
+    const char *who = src.twobit ? "crf_seq_load_2bit" : src.nibbles ? "crf_seq_load_nibbles"
+                    : src.packed() ? "crf_seq_load_packed" : "crf_seq_load_ascii";
     LoadTrace trace;
     cudaStream_t st = c->stream;
     s->ctx = c;
@@ -487,11 +490,13 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
     // The source span the records cover (units may overlap) goes up in chunks on a second stream while the pack kernel
     // works on the layout words whose source has already arrived (the PCIe copy is ~10x longer than the packing, which
     // then hides behind it).  Unit of the span: bytes (ASCII) or positions rounded out to whole 32-bit words (packed).
-    const bool packed = src.packed(), twobit = src.twobit != nullptr;
-    const uint64_t src_end = src_hi;                                     // .2bit: bytes up to (src_end + 3) / 4 are the caller's
+    const bool packed = src.packed(), twobit = src.twobit != nullptr, nibbles = src.nibbles != nullptr;
+    const uint64_t src_end = src_hi;                                     // .2bit / BAM: bytes up to (src_end + 3) / 4 or
+                                                                         // (src_end + 1) / 2 are the caller's
     if (packed) { src_lo &= ~31ull; src_hi = (src_hi + 31) & ~31ull; }
     const uint64_t span = src_hi - src_lo;                               // positions
-    const uint64_t UPLOAD_CHUNK = packed ? (512ull << 20) : (64ull << 20);   // positions per chunk (64 MB either way)
+    const uint64_t UPLOAD_CHUNK = nibbles ? (128ull << 20) : packed ? (512ull << 20) : (64ull << 20);   // positions per chunk
+                                                                                                   // (64 MB of planes, bytes or codes)
     const bool pipelined = !on_device && span > 2 * UPLOAD_CHUNK;
     const uint8_t *d_src = src.bases;                                    // device views of the source
     const uint32_t *d_pH = src.pH, *d_pL = src.pL, *d_pN = src.pN;
@@ -505,7 +510,7 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
     const bool runs_mode = packed && src.runs_mode;
     if (!on_device) {
         if (packed) {
-            CHECK(dev_alloc(&d_planes_own, 3 * (size_t)span_words));
+            CHECK(dev_alloc(&d_planes_own, (nibbles ? 4 : 3) * (size_t)span_words));
             d_pH = d_planes_own; d_pL = d_planes_own + span_words; d_pN = d_planes_own + 2 * span_words;
         } else {
             CHECK(dev_alloc(&d_src_own, (size_t)span));
@@ -543,6 +548,11 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
             const uint64_t b0 = (src_lo + lo) / 4, b1 = std::min((src_lo + lo + n + 3) / 4, (src_end + 3) / 4);
             if (b1 <= b0) return cudaSuccess;
             return cudaMemcpyAsync((uint8_t *)d_planes_own + lo / 4, src.twobit + b0, b1 - b0, cudaMemcpyHostToDevice, cs);
+        }
+        if (nibbles) {
+            const uint64_t b0 = (src_lo + lo) / 2, b1 = std::min((src_lo + lo + n + 1) / 2, (src_end + 1) / 2);
+            if (b1 <= b0) return cudaSuccess;
+            return cudaMemcpyAsync((uint8_t *)d_planes_own + lo / 2, src.nibbles + b0, b1 - b0, cudaMemcpyHostToDevice, cs);
         }
         if (!packed) return cudaMemcpyAsync(d_src_own + lo, src.bases + src_lo + lo, n, cudaMemcpyHostToDevice, cs);
         const uint64_t w0 = lo / 32, nw = (n + 31) / 32, h0 = src_lo / 32 + w0;
@@ -663,6 +673,15 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
             tp.n_records = n_records; tp.w_lo = w_lo; tp.w_hi = w_hi;
             tp.H = s->H; tp.L = s->L; tp.NM = s->NM; tp.X = s->X;
             twobit_pack_kernel<<<(w_hi - w_lo + 255) / 256, 256, 0, st>>>(tp);
+        } else if (nibbles) {
+            NibbleParams np;
+            np.nib = on_device ? src.nibbles : (const uint8_t *)d_planes_own;
+            np.n_bytes = (src_end + 1) / 2 - (on_device ? 0 : src_lo / 2);
+            np.src_base = src_base;
+            np.rec_src_start = d_src_start; np.rec_len = s->d_rec_len; np.rec_dev_off = s->d_rec_dev_off;
+            np.n_records = n_records; np.w_lo = w_lo; np.w_hi = w_hi;
+            np.H = s->H; np.L = s->L; np.NM = s->NM; np.X = s->X;
+            nibble_pack_kernel<<<(w_hi - w_lo + 255) / 256, 256, 0, st>>>(np);
         } else if (packed) {
             RepackParams rp;
             rp.sH = d_pH; rp.sL = d_pL; rp.sN = d_pN; rp.src_base = src_base;
@@ -806,7 +825,7 @@ static int load_checked(crf_ctx *c, const LoadSource &src, const uint64_t *start
         set_err("%s: max_motif_cap %u not in [1, %u]", who, max_motif_cap, MAX_K);
         return max_motif_cap < 1 ? CRF_ERR_ARG : CRF_ERR_UNSUPPORTED;
     }
-    const bool have_src = src.twobit ? true : src.packed() ? (src.pL && src.pN) : (src.bases != nullptr);
+    const bool have_src = src.twobit || src.nibbles ? true : src.packed() ? (src.pL && src.pN) : (src.bases != nullptr);
     if (!have_src) {
         for (uint32_t r = 0; r < n_records; ++r)
             if (lengths ? lengths[r] : starts[r + 1] - starts[r]) { set_err("%s: null %s", who, src.packed() ? "plane" : "bases"); return CRF_ERR_ARG; }
@@ -969,6 +988,48 @@ extern "C" int crf_seq_load_2bit(crf_ctx *c, const uint8_t *dna, const uint64_t 
     src.twobit = dna;
     src.nm_runs = moved.data(); src.n_runs = moved.size() / 2; src.runs_mode = true;
     return load_checked(c, src, starts.data(), lengths.data(), nullptr, nullptr, n_records, max_motif_cap, dna_on_device, out, who);
+}
+
+// BAM reads: record r = offsets[r + 1] - offsets[r] bases coded from byte rec_byte[r] of nib, its exotic codes among the
+// list in offsets' position space.  The load sees record r at source position 2 rec_byte[r] and the exotic list moved there.
+extern "C" int crf_seq_load_nibbles(crf_ctx *c, const uint8_t *nib, const uint64_t *rec_byte, const uint64_t *offsets,
+                                    uint32_t n_records, const uint64_t *exotic, uint64_t n_exotic, uint32_t max_motif_cap,
+                                    int nib_on_device, crf_seq **out) {
+    const char *who = "crf_seq_load_nibbles";
+    CHECK(check_offsets(offsets, n_records, who));
+    if (!nib || !rec_byte || (n_exotic && !exotic)) { set_err("%s: null argument", who); return CRF_ERR_ARG; }
+    for (uint32_t r = 0; r < n_records; ++r)
+        if (offsets[r + 1] < offsets[r]) { set_err("%s: offsets must be non-decreasing", who); return CRF_ERR_ARG; }
+    for (uint64_t i = 1; i < n_exotic; ++i)
+        if (exotic[i] >> 8 <= exotic[i - 1] >> 8) { set_err("%s: the exotic list must be ascending (entry %llu)", who, (unsigned long long)i); return CRF_ERR_ARG; }
+    std::vector<uint64_t> starts, lengths, moved;
+    try {
+        starts.resize(n_records);
+        lengths.resize(n_records);
+        for (uint32_t r = 0; r < n_records; ++r) {
+            starts[r] = 2 * rec_byte[r];
+            lengths[r] = offsets[r + 1] - offsets[r];
+        }
+        const uint64_t pos0 = offsets[0], pos1 = offsets[n_records];
+        const uint64_t *e0 = std::lower_bound(exotic, exotic + n_exotic, pos0 << 8), *e1 = std::lower_bound(e0, exotic + n_exotic, pos1 << 8);
+        bool sorted = true;
+        uint32_t r = 0;
+        for (const uint64_t *e = e0; e < e1; ++e) {
+            const uint64_t q = *e >> 8;
+            while (offsets[r + 1] <= q) ++r;
+            const uint64_t m = ((starts[r] + (q - offsets[r])) << 8) | (*e & 0xFF);
+            if (!moved.empty() && m < moved.back()) sorted = false;
+            moved.push_back(m);
+        }
+        if (!sorted) std::sort(moved.begin(), moved.end());            // records not in the order of their bytes
+    } catch (const std::bad_alloc &) {
+        set_err("out of host memory");
+        return CRF_ERR_NOMEM;
+    }
+    LoadSource src;
+    src.nibbles = nib;
+    src.exotic = moved.data(); src.n_exotic = moved.size();
+    return load_checked(c, src, starts.data(), lengths.data(), nullptr, nullptr, n_records, max_motif_cap, nib_on_device, out, who);
 }
 
 extern "C" int crf_seq_load_packed(crf_ctx *c, const uint32_t *H, const uint32_t *L, const uint32_t *NM,
@@ -1989,6 +2050,7 @@ static cudaError_t preload_kernels() {
     if (e == cudaSuccess) e = preload(pack_kernel);
     if (e == cudaSuccess) e = preload(repack_kernel);
     if (e == cudaSuccess) e = preload(twobit_pack_kernel);
+    if (e == cudaSuccess) e = preload(nibble_pack_kernel);
     if (e == cudaSuccess) e = preload(mask_runs_kernel);
     if (e == cudaSuccess) e = preload(exotic_apply_kernel);
     if (e == cudaSuccess) e = preload(tile_offsets_kernel);

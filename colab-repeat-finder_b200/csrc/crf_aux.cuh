@@ -233,6 +233,111 @@ __global__ void __launch_bounds__(256) twobit_pack_kernel(const TwoBitParams p) 
     p.X[w] = 0;
 }
 
+// ---- BAM: 4-bit codes (=ACMGRSVTWYHKDBN) -> the device layout.  Source position q is nibble q & 1 of byte q >> 1, high
+// nibble first.  A code c gives H = (c & 0b1100) != 0, L = (c & 0b1010) != 0 (A = 1, C = 2, G = 4, T = 8 -> codes 0..3),
+// and NM wherever c is not 1, 2, 4 or 8, so N and the other codes are masked without a list from the host (the exotic ones
+// then get their letters from exotic_apply_kernel).  Same structure and result as twobit_pack_kernel. -------------------
+struct NibbleParams {
+    const uint8_t *nib;             // byte 0 holds source positions [src_base, src_base + 2)
+    uint64_t n_bytes;               // bytes of nib that may be read
+    uint64_t src_base;              // multiple of 32
+    const uint64_t *rec_src_start;  // source position of each record's first base
+    const uint32_t *rec_len;
+    const uint32_t *rec_dev_off;
+    uint32_t n_records;
+    uint32_t w_lo, w_hi;            // layout words this launch packs
+    uint32_t *H, *L, *NM, *X;
+};
+
+__device__ __forceinline__ uint32_t fourth_bits(uint64_t v) {   // bits 0, 4, 8, ... of v -> bits 0, 1, 2, ...
+    v &= 0x1111111111111111ull;
+    v = (v | (v >> 3)) & 0x0303030303030303ull;
+    v = (v | (v >> 6)) & 0x000F000F000F000Full;
+    v = (v | (v >> 12)) & 0x000000FF000000FFull;
+    return (uint32_t)((v | (v >> 24)) & 0xFFFFu);
+}
+
+// H, L and NM of 16 source positions from their 8 bytes (x: byte j in bits 8j..8j+7)
+__device__ __forceinline__ void nibble_planes16(uint64_t x, uint32_t &H, uint32_t &L, uint32_t &NM) {
+    x = ((x >> 4) & 0x0F0F0F0F0F0F0F0Full) | ((x & 0x0F0F0F0F0F0F0F0Full) << 4);   // position i -> bits 4i .. 4i + 3
+    const uint64_t b0 = x, b1 = x >> 1, b2 = x >> 2, b3 = x >> 3;
+    const uint64_t any = b0 | b1 | b2 | b3, two = (b0 & (b1 | b2 | b3)) | (b1 & (b2 | b3)) | (b2 & b3);
+    H = fourth_bits(b2 | b3);
+    L = fourth_bits(b1 | b3);
+    NM = fourth_bits(~(any & ~two));
+}
+
+// the H / L / NM planes of source word wi (bytes 16 wi .. 16 wi + 15); bytes past n_bytes read as code 0 (masked)
+__device__ __forceinline__ void nibble_planes(const NibbleParams &p, uint64_t wi, uint32_t &H, uint32_t &L, uint32_t &NM) {
+    const uint64_t b0 = 16 * wi;
+    const uint8_t *s = p.nib + b0;
+    uint64_t x0 = 0, x1 = 0;
+    if (b0 + 16 <= p.n_bytes && ((uintptr_t)s & 15) == 0) {
+        const uint4 v = *reinterpret_cast<const uint4 *>(s);
+        x0 = ((uint64_t)v.y << 32) | v.x;
+        x1 = ((uint64_t)v.w << 32) | v.z;
+    } else {
+        for (uint32_t j = 0; j < 16; ++j)
+            if (b0 + j < p.n_bytes) (j < 8 ? x0 : x1) |= (uint64_t)s[j] << (8 * (j & 7));
+    }
+    uint32_t h0, l0, n0, h1, l1, n1;
+    nibble_planes16(x0, h0, l0, n0);
+    nibble_planes16(x1, h1, l1, n1);
+    H = h0 | (h1 << 16);
+    L = l0 | (l1 << 16);
+    NM = n0 | (n1 << 16);
+}
+
+__global__ void __launch_bounds__(256) nibble_pack_kernel(const NibbleParams p) {
+    const uint32_t w = p.w_lo + blockIdx.x * blockDim.x + threadIdx.x;
+    if (w >= p.w_hi) return;
+    const uint32_t p0 = w << 5;
+    uint32_t h = 0, l = 0, nm = 0xFFFFFFFFu;                 // gaps and pads are masked
+    if (p.n_records) {
+        uint32_t lo = 0, hi = p.n_records - 1;               // last record that starts at or before p0
+        while (lo < hi) {
+            const uint32_t mid = (lo + hi + 1) >> 1;
+            if (p.rec_dev_off[mid] <= p0) lo = mid; else hi = mid - 1;
+        }
+        const uint64_t p1 = (uint64_t)p0 + 32;
+        for (uint32_t r = lo; r < p.n_records; ++r) {
+            const uint32_t dev0 = p.rec_dev_off[r];
+            if ((uint64_t)dev0 >= p1) break;
+            const uint64_t rec_end = (uint64_t)dev0 + p.rec_len[r];
+            const uint64_t a = max((uint64_t)p0, (uint64_t)dev0), b = min(p1, rec_end);
+            if (a >= b) continue;
+            const uint32_t nbits = (uint32_t)(b - a), place = (uint32_t)(a - p0);
+            const uint64_t sbit = p.rec_src_start[r] - p.src_base + (a - dev0);
+            const uint64_t wi = sbit >> 5;
+            const uint32_t sh = (uint32_t)sbit & 31u;
+            const uint32_t mask = nbits == 32 ? 0xFFFFFFFFu : ((1u << nbits) - 1u);
+            const uint64_t wj = (sh && nbits > 32u - sh) ? wi + 1 : wi;
+            uint32_t hi_, li_, ni_, hj, lj, nj;
+            nibble_planes(p, wi, hi_, li_, ni_);
+            if (wj != wi) nibble_planes(p, wj, hj, lj, nj); else { hj = hi_; lj = li_; nj = ni_; }
+            const uint32_t eh = __funnelshift_r(hi_, hj, sh) & mask;
+            const uint32_t el = __funnelshift_r(li_, lj, sh) & mask;
+            const uint32_t en = __funnelshift_r(ni_, nj, sh) & mask;
+            h |= eh << place;
+            l |= el << place;
+            nm = (nm & ~(mask << place)) | (en << place);
+        }
+    }
+    h &= ~nm;
+    l &= ~nm;
+    for (uint32_t m = nm; m;) {                               // aperiodic filler at masked positions (see pack_kernel)
+        const uint32_t b = __ffs(m) - 1;
+        m &= m - 1;
+        const uint32_t code = hash32(p0 + b) & 3;
+        h |= (code >> 1) << b;
+        l |= (code & 1) << b;
+    }
+    p.H[w] = h;
+    p.L[w] = l;
+    p.NM[w] = nm;
+    p.X[w] = 0;
+}
+
 // runs mode of a packed load: the mask plane from the sorted runs of masked positions [runs[2i], runs[2i+1]); one warp per
 // run (its lanes stride over the run's words; a genome has a few hundred long N blocks, a read set millions of single N's)
 __global__ void __launch_bounds__(256) mask_runs_kernel(const uint64_t *runs, uint32_t n_runs, uint32_t *NM) {

@@ -35,8 +35,8 @@ struct crf_fasta {
     bool planes_pinned = false;
     bool want_pinned_planes = false;                     // crf_fasta_open(pinned & 3): page-lock the planes crf_fasta_packed makes
     std::vector<uint64_t> exotic;
-    int format = 0;                                      // 0 = FASTA, 1 = FASTQ, 2 = .2bit
-    uint8_t *quals = nullptr;                            // FASTQ, crf_fasta_open(pinned & 4): laid out like bases
+    int format = 0;                                      // 0 = FASTA, 1 = FASTQ, 2 = .2bit, 3 = BAM
+    uint8_t *quals = nullptr;                            // FASTQ / BAM, crf_fasta_open(pinned & 4): laid out like bases
     // .2bit: the file's bytes as they are (mapped, or page-locked with pinned & 3), where each record's packed bases
     // start, its N blocks and mask blocks as sorted disjoint runs of concatenated positions; the text (bases) is decoded
     // on the first crf_fasta_data
@@ -45,6 +45,13 @@ struct crf_fasta {
     void *dna_map = nullptr;
     bool dna_pinned = false;
     std::vector<uint64_t> rec_byte, n_runs, mask_runs;
+    // BAM: the reads' 4-bit codes (=ACMGRSVTWYHKDBN, high nibble first), record r from byte rec_byte[r] with reverse
+    // complements applied; page-locked with pinned & 3, else an anonymous mapping of nib_map bytes.  nib_exotic: codes other
+    // than A, C, G, T, N as (position in the offsets' space << 8 | letter), ascending.  quals_map: the qualities' mapping size.
+    uint8_t *nib = nullptr;
+    uint64_t nib_bytes = 0, nib_map = 0, quals_map = 0;
+    bool nib_pinned = false;
+    std::vector<uint64_t> nib_exotic;
     std::mutex decode_mu;
     int text_pinned = 0;                                 // the pinned argument of crf_fasta_open, for the decoded text
     uint32_t n_threads = 1;
@@ -169,15 +176,16 @@ static void run_parallel(unsigned n_threads, size_t n_items, const std::function
 // BGZF (bgzip, what `samtools faidx` wants and the reference's Hail pipeline ships: run_hail_batch_pipeline.py:112 takes
 // the .gzi next to the FASTA): every gzip member is a self-contained block of <= 64 KiB that says its own compressed size
 // in a 'BC' extra field, so the blocks are found by hopping over the headers and inflated on all threads.
-// Returns false if the file is not BGZF from the first to the last byte (the caller then inflates it serially);
-// *bad is set if it is BGZF but a block is corrupt.
+// A file that is not BGZF from the first to the last byte is inflated serially instead.
 // Each block is decoded by the reader's own DEFLATE decoder (crf_inflate.h, ~2 x zlib on FASTA text) into a scratch buffer --
 // its copies may write a few bytes beyond a match, which in the shared output would be the next block's -- and copied to its
 // place once length and CRC-32 agree; a block it does not take (or CRF_GUNZIP_ZLIB=1) goes through zlib, which then decides.
-// The output is a mapping of its own (no zero-fill before the blocks arrive, 2 MB pages).
-static bool inflate_bgzf(const FileBytes &in, unsigned n_threads, crf_inflate::OutBuf &out, bool *bad) {
-    struct Block { uint64_t cdata, clen, out; uint32_t isize, crc; };
-    std::vector<Block> blocks;
+// The whole-file output is a mapping of its own (no zero-fill before the blocks arrive, 2 MB pages).
+struct BgzfBlock { uint64_t cdata, clen, out; uint32_t isize, crc; };
+
+// The blocks of a BGZF file (false: not BGZF from the first to the last byte); *total = the inflated size.
+static bool bgzf_index(const FileBytes &in, std::vector<BgzfBlock> &blocks, uint64_t *total_out) {
+    using Block = BgzfBlock;
     const uint8_t *d = in.data;
     const uint64_t n = in.size;
     uint64_t pos = 0, total = 0;
@@ -206,54 +214,66 @@ static bool inflate_bgzf(const FileBytes &in, unsigned n_threads, crf_inflate::O
         blocks.push_back(b);
         pos += bsize;
     }
-    if (!out.reserve(total + 64)) throw std::bad_alloc();
-    out.size = total;
-    uint8_t *const dst = out.p;
-    const bool own_decoder = getenv("CRF_GUNZIP_ZLIB") == nullptr;
-    std::atomic<bool> failed{false}, no_memory{false};
-    const size_t GROUP = 128;                             // blocks per work item (<= 8 MiB of text)
-    run_parallel(n_threads, (blocks.size() + GROUP - 1) / GROUP, [&](size_t g) {
-      try {
-        crf_inflate::OutBuf scratch;
-        crf_inflate::Tables tables;
-        z_stream zs;
-        bool zs_ready = false;
-        for (size_t i = g * GROUP; i < std::min(blocks.size(), (g + 1) * GROUP) && !failed; ++i) {
-            const Block &b = blocks[i];
-            if (b.isize == 0) continue;                   // the empty end-of-file block
-            if (own_decoder) {
-                crf_inflate::Decoder dec;
-                dec.base = dec.in = d + b.cdata;
-                dec.in_end = dec.in + b.clen;
-                dec.out = &scratch;
-                dec.op = 0;
-                if (dec.run(tables) == crf_inflate::Decoder::RUN_FINAL && dec.op == b.isize &&
-                    (uint32_t)crc32(crc32(0L, Z_NULL, 0), scratch.p, b.isize) == b.crc) {
-                    memcpy(dst + b.out, scratch.p, b.isize);
-                    continue;
-                }
+    *total_out = total;
+    return true;
+}
+
+// Inflates BGZF blocks one after the other on one thread (a worker's state: scratch output, tables, a zlib stream).
+struct BgzfInflater {
+    const uint8_t *d;                                     // the file's bytes
+    bool own_decoder = getenv("CRF_GUNZIP_ZLIB") == nullptr;
+    crf_inflate::OutBuf scratch;
+    crf_inflate::Tables tables;
+    z_stream zs;
+    bool zs_ready = false;
+    explicit BgzfInflater(const uint8_t *data) : d(data) {}
+    ~BgzfInflater() { if (zs_ready) inflateEnd(&zs); }
+    // block b -> dst[0, b.isize); false if it is corrupt (length or CRC-32)
+    bool run(const BgzfBlock &b, uint8_t *dst) {
+        if (b.isize == 0) return true;                    // the empty end-of-file block
+        if (own_decoder) {
+            crf_inflate::Decoder dec;
+            dec.base = dec.in = d + b.cdata;
+            dec.in_end = dec.in + b.clen;
+            dec.out = &scratch;
+            dec.op = 0;
+            if (dec.run(tables) == crf_inflate::Decoder::RUN_FINAL && dec.op == b.isize &&
+                (uint32_t)crc32(crc32(0L, Z_NULL, 0), scratch.p, b.isize) == b.crc) {
+                memcpy(dst, scratch.p, b.isize);
+                return true;
             }
-            if (!zs_ready) {
-                memset(&zs, 0, sizeof zs);
-                if (inflateInit2(&zs, -15) != Z_OK) { failed = true; return; }
-                zs_ready = true;
-            }
-            zs.next_in = const_cast<Bytef *>(d + b.cdata);
-            zs.avail_in = (uInt)b.clen;
-            zs.next_out = dst + b.out;
-            zs.avail_out = b.isize;
-            const int rc = inflate(&zs, Z_FINISH);
-            if (rc != Z_STREAM_END || zs.avail_out != 0 ||
-                (uint32_t)crc32(crc32(0L, Z_NULL, 0), dst + b.out, b.isize) != b.crc)
-                failed = true;
-            inflateReset(&zs);
         }
-        if (zs_ready) inflateEnd(&zs);
+        if (!zs_ready) {
+            memset(&zs, 0, sizeof zs);
+            if (inflateInit2(&zs, -15) != Z_OK) return false;
+            zs_ready = true;
+        }
+        zs.next_in = const_cast<Bytef *>(d + b.cdata);
+        zs.avail_in = (uInt)b.clen;
+        zs.next_out = dst;
+        zs.avail_out = b.isize;
+        const int rc = inflate(&zs, Z_FINISH);
+        const bool ok = rc == Z_STREAM_END && zs.avail_out == 0 && (uint32_t)crc32(crc32(0L, Z_NULL, 0), dst, b.isize) == b.crc;
+        inflateReset(&zs);
+        return ok;
+    }
+};
+
+// Blocks [first, last) on the reader's threads into dst (block i at dst + blocks[i].out - blocks[first].out); false if one
+// is corrupt.
+static bool inflate_blocks(const uint8_t *d, const std::vector<BgzfBlock> &blocks, size_t first, size_t last,
+                           unsigned n_threads, uint8_t *dst, size_t GROUP = 128) {   // GROUP: blocks per work item
+    std::atomic<bool> failed{false}, no_memory{false};
+    const uint64_t out0 = first < last ? blocks[first].out : 0;
+    run_parallel(n_threads, (last - first + GROUP - 1) / GROUP, [&](size_t g) {
+      try {
+        BgzfInflater inf(d);
+        for (size_t i = first + g * GROUP; i < std::min(last, first + (g + 1) * GROUP) && !failed; ++i)
+            if (!inf.run(blocks[i], dst + blocks[i].out - out0)) failed = true;
       } catch (const std::bad_alloc &) { no_memory = true; failed = true; }      // (nothing leaves a worker thread)
     });
     if (no_memory) throw std::bad_alloc();
-    *bad = failed;
-    return true;
+    return !failed;
 }
 
 static bool is_space(uint8_t c) { return c == ' ' || c == '\t' || c == '\r' || c == '\n' || c == '\v' || c == '\f'; }
@@ -656,6 +676,294 @@ static int twobit_decode(crf_fasta *fa) {
     return CRF_OK;
 }
 
+// ---- BAM (unaligned reads) ----
+// A BGZF stream that starts with "BAM\1": l_text, the header text, n_ref and the reference list, then the records.  A
+// record is block_size and block_size bytes: refID, pos, l_read_name (u8), mapq, bin, n_cigar_op (u16), flag (u16), l_seq,
+// next_refID, next_pos, tlen (32 bytes in all), read_name (NUL-terminated), cigar (4 n_cigar_op bytes), seq ((l_seq + 1) / 2
+// bytes, 4-bit codes =ACMGRSVTWYHKDBN, high nibble first), qual (l_seq bytes, 0xFF... when absent), tags.
+// What is kept is what `samtools fastq -n` writes: records with (flag & 0x900) == 0 in file order, the name up to its NUL,
+// the bases reverse-complemented when flag & 0x10 (the complement of a code is its 4-bit bit-reversal), qualities + 33 (or
+// '"' when absent), reversed with the bases.  The stream is inflated a window of blocks at a time; the bases stay codes.
+static const uint64_t BAM_WINDOW = 32u << 20;             // inflated bytes per window (CRF_BAM_WINDOW overrides it)
+static const char BAM_LETTERS[] = "=ACMGRSVTWYHKDBN";
+
+static bool is_bam_magic(const uint8_t *t, uint64_t n) { return n >= 4 && memcmp(t, "BAM\1", 4) == 0; }
+
+// A growable anonymous mapping: it grows with mremap (the pages are not copied) and nothing is zero-filled by hand.
+struct GrowBuf {
+    uint8_t *p = nullptr;
+    size_t cap = 0;
+    ~GrowBuf() { if (p) munmap(p, cap); }
+    void reserve(size_t need) {
+        if (need <= cap) return;
+        size_t nc = std::max<size_t>(std::max<size_t>(need, cap + cap / 2), (size_t)1 << 21);
+        nc = (nc + 4095) & ~(size_t)4095;
+        void *q = p ? mremap(p, cap, nc, MREMAP_MAYMOVE) : mmap(nullptr, nc, PROT_READ | PROT_WRITE, MAP_PRIVATE | MAP_ANONYMOUS, -1, 0);
+        if (q == MAP_FAILED) throw std::bad_alloc();
+        p = (uint8_t *)q;
+        cap = nc;
+    }
+    uint8_t *release() { uint8_t *q = p; p = nullptr; return q; }
+};
+
+// The inflated stream, a window of blocks at a time: bytes [pos, end) of buf are inflated and not yet consumed.
+struct BamStream {
+    const uint8_t *file;
+    const std::vector<BgzfBlock> &blocks;
+    unsigned n_threads;
+    size_t next = 0;                                      // first block not inflated
+    uint64_t left;                                        // inflated bytes of the blocks from next on
+    uint64_t window;
+    GrowBuf buf;
+    uint64_t pos = 0, end = 0;
+    uint64_t avail() const { return end - pos; }
+    // At least one more window, more while fewer than `need` bytes are available and blocks remain.  false: a corrupt block.
+    bool fill(uint64_t need) {
+        if (pos) { memmove(buf.p, buf.p + pos, end - pos); end -= pos; pos = 0; }
+        do {
+            if (next == blocks.size()) return true;
+            size_t last = next;
+            uint64_t bytes = 0;
+            while (last < blocks.size() && (last == next || bytes + blocks[last].isize <= window)) bytes += blocks[last++].isize;
+            buf.reserve(end + bytes);
+            if (!inflate_blocks(file, blocks, next, last, n_threads, buf.p + end, 16)) return false;
+            end += bytes;
+            left -= bytes;
+            next = last;
+        } while (end - pos < need);
+        return true;
+    }
+};
+
+static inline uint32_t rd32(const uint8_t *p) { uint32_t v; memcpy(&v, p, 4); return v; }
+static inline uint16_t rd16(const uint8_t *p) { uint16_t v; memcpy(&v, p, 2); return v; }
+
+struct BamRec {                                           // a kept record of the current window
+    uint64_t at;                                          // its block_size field, in the stream buffer
+    uint64_t base, name;                                  // where its bases and name go
+};
+
+// Record number `rec` (1-based) at q (its block_size field) of a buffer holding n >= 4 bytes from q on, complete when
+// n >= 4 + block_size.  Returns nullptr if it is well-formed (*kept, *l_seq, *name_len set), else why not.
+static const char *bam_check(const uint8_t *q, uint32_t bs, bool *kept, uint64_t *l_seq, uint64_t *name_len) {
+    const uint8_t *f = q + 4;
+    const uint32_t lrn = f[8], ncig = rd16(f + 12), flag = rd16(f + 14);
+    const int32_t ls = (int32_t)rd32(f + 16);
+    if (lrn == 0) return "l_read_name is 0";
+    if (ls < 0) return "l_seq is negative";
+    if (32ull + lrn + 4ull * ncig + ((uint64_t)ls + 1) / 2 + (uint64_t)ls > bs) return "its fields run past its block_size";
+    if (f[32 + lrn - 1] != 0) return "its read_name does not end with a NUL";
+    *kept = (flag & 0x900) == 0;
+    *l_seq = (uint64_t)ls;
+    *name_len = strnlen((const char *)f + 32, lrn);
+    return nullptr;
+}
+
+// A kept record's bases (codes from byte `o` of nib, reverse-complemented when flag & 0x10, a padding nibble 0), its name,
+// its qualities (quals may be null) and its exotic codes (appended to ex, positions from `base`).
+static void bam_copy(const uint8_t *q, uint8_t *nib, uint64_t o, uint8_t *quals, uint64_t base, char *name_out,
+                     std::vector<uint64_t> &ex) {
+    static const struct Lut {
+        uint8_t comp[16], exotic[16];
+        Lut() {
+            for (int c = 0; c < 16; ++c) {
+                comp[c] = (uint8_t)(((c & 1) << 3) | ((c & 2) << 1) | ((c & 4) >> 1) | ((c & 8) >> 3));
+                exotic[c] = !(c == 1 || c == 2 || c == 4 || c == 8 || c == 15);
+            }
+        }
+    } lut;
+    const uint8_t *f = q + 4;
+    const uint32_t lrn = f[8], ncig = rd16(f + 12), flag = rd16(f + 14);
+    const uint64_t n = rd32(f + 16);
+    const uint8_t *seq = f + 32 + lrn + 4 * ncig, *qual = seq + (n + 1) / 2;
+    const size_t nl = strnlen((const char *)f + 32, lrn);
+    memcpy(name_out, f + 32, nl);
+    name_out[nl] = '\0';
+    uint8_t *d = nib + o;
+    const bool rev = flag & 0x10;
+    if (!rev) {
+        memcpy(d, seq, n / 2);
+        if (n & 1) d[n / 2] = seq[n / 2] & 0xF0;
+    } else if (n) {                                        // base i = complement of base n - 1 - i, a byte at a time
+        const uint64_t last = (n - 1) / 2;
+        if (n & 1) {                                       // byte j: high nibble of byte last - j, low of the one before
+            for (uint64_t j = 0; j <= last; ++j) {
+                const uint64_t k = last - j;
+                d[j] = (uint8_t)((lut.comp[seq[k] >> 4] << 4) | (k ? lut.comp[seq[k - 1] & 15] : 0));
+            }
+        } else {                                           // byte j: byte last - j with its nibbles swapped
+            for (uint64_t j = 0; j <= last; ++j) {
+                const uint8_t b = seq[last - j];
+                d[j] = (uint8_t)((lut.comp[b & 15] << 4) | lut.comp[b >> 4]);
+            }
+        }
+    }
+    for (uint64_t i = 0; i < n; i += 2) {                  // exotic codes: rare, found a byte at a time
+        const uint8_t b = d[i >> 1];
+        if (!lut.exotic[b >> 4] && (i + 1 == n || !lut.exotic[b & 15])) continue;
+        for (uint64_t k = i; k < std::min(n, i + 2); ++k) {
+            const uint8_t c = k & 1 ? b & 15 : b >> 4;
+            if (lut.exotic[c]) ex.push_back(((base + k) << 8) | (uint8_t)BAM_LETTERS[c]);
+        }
+    }
+    if (!quals) return;
+    uint8_t *qo = quals + base;
+    if (n && qual[0] == 0xFF) memset(qo, '"', n);
+    else if (!rev) for (uint64_t i = 0; i < n; ++i) qo[i] = (uint8_t)(qual[i] + 33);
+    else for (uint64_t i = 0; i < n; ++i) qo[i] = (uint8_t)(qual[n - 1 - i] + 33);
+}
+
+// The BAM stream of the BGZF blocks into fa.  Every count and length is checked against the record and the stream.
+static int parse_bam(const char *path, const uint8_t *file, const std::vector<BgzfBlock> &blocks, uint64_t total,
+                     unsigned n_threads, int pinned, crf_fasta *fa) {
+    fa->format = 3;
+    const char *w = getenv("CRF_BAM_WINDOW");
+    BamStream s{file, blocks, n_threads, 0, total, w ? std::max<uint64_t>(strtoull(w, nullptr, 10), 1) : BAM_WINDOW};
+    auto corrupt = [&]() { set_err("crf_fasta_open: %s has a corrupt BGZF block", path); return CRF_ERR_ARG; };
+    auto header_fail = [&](const char *why) { set_err("crf_fasta_open: %s: BAM header: %s", path, why); return CRF_ERR_ARG; };
+    auto rec_fail = [&](uint64_t rec, const char *why) {
+        set_err("crf_fasta_open: %s: BAM record %llu: %s", path, (unsigned long long)rec, why);
+        return CRF_ERR_ARG;
+    };
+    // header: the first h bytes of the stream, pulled in as needed (false: shorter than that)
+    int bad_block = 0;
+    auto have = [&](uint64_t h) {
+        if (h <= s.avail()) return true;
+        if (h > s.avail() + s.left) return false;
+        if (!s.fill(h)) { bad_block = 1; return false; }
+        return true;
+    };
+    if (!have(12)) return bad_block ? corrupt() : header_fail("it is truncated");
+    const int32_t l_text = (int32_t)rd32(s.buf.p + s.pos + 4);
+    if (l_text < 0) return header_fail("l_text is negative");
+    uint64_t h = 8 + (uint64_t)l_text;
+    if (!have(h + 4)) return bad_block ? corrupt() : header_fail("the text runs past the end of the data");
+    const int32_t n_ref = (int32_t)rd32(s.buf.p + s.pos + h);
+    if (n_ref < 0) return header_fail("n_ref is negative");
+    h += 4;
+    for (int32_t i = 0; i < n_ref; ++i) {
+        if (!have(h + 4)) return bad_block ? corrupt() : header_fail("the reference list runs past the end of the data");
+        const int32_t l_name = (int32_t)rd32(s.buf.p + s.pos + h);
+        if (l_name < 0) return header_fail("a reference's l_name is negative");
+        h += 4 + (uint64_t)l_name + 4;
+        if (!have(h)) return bad_block ? corrupt() : header_fail("the reference list runs past the end of the data");
+    }
+    s.pos += h;
+
+    const bool want_quals = pinned & 4;
+    GrowBuf nib, quals;
+    uint64_t nib_at = 0, base_at = 0, rec = 0;              // output cursors; records seen
+    std::vector<BamRec> batch;
+    std::vector<std::vector<uint64_t>> ex_parts;
+    for (;;) {
+        batch.clear();
+        uint64_t p = s.pos, name_at = fa->names.size();
+        while (s.end - p >= 4) {                            // the complete records of the buffer
+            const uint32_t bs = rd32(s.buf.p + p);
+            if (bs < 32) return rec_fail(rec + 1, "block_size is less than 32");
+            if (s.end - p - 4 < bs) {
+                if (bs > s.end - p - 4 + s.left) return rec_fail(rec + 1, "it runs past the end of the data");
+                break;
+            }
+            bool kept;
+            uint64_t l_seq, nl;
+            if (const char *why = bam_check(s.buf.p + p, bs, &kept, &l_seq, &nl)) return rec_fail(rec + 1, why);
+            ++rec;
+            if (kept) {
+                batch.push_back({p, base_at, name_at});
+                fa->offsets.push_back(base_at);
+                fa->rec_byte.push_back(nib_at);
+                fa->name_off.push_back(name_at);
+                base_at += l_seq;
+                nib_at += (l_seq + 1) / 2;
+                name_at += nl + 1;
+            }
+            p += 4 + (uint64_t)bs;
+        }
+        if (!batch.empty()) {                                // copy the window's kept records on the reader's threads
+            nib.reserve(nib_at + 16);
+            if (want_quals) quals.reserve(base_at + 16);
+            fa->names.resize(name_at);
+            // (work items of a few records for long reads, thousands for short ones)
+            const size_t first = fa->rec_byte.size() - batch.size(), GROUP = (batch.size() + 8 * n_threads - 1) / (8 * n_threads);
+            ex_parts.assign((batch.size() + GROUP - 1) / GROUP, {});
+            run_parallel(n_threads, ex_parts.size(), [&](size_t g) {
+                for (size_t i = g * GROUP; i < std::min(batch.size(), (g + 1) * GROUP); ++i)
+                    bam_copy(s.buf.p + batch[i].at, nib.p, fa->rec_byte[first + i], want_quals ? quals.p : nullptr,
+                             batch[i].base, fa->names.data() + batch[i].name, ex_parts[g]);
+            });
+            for (const auto &v : ex_parts) fa->nib_exotic.insert(fa->nib_exotic.end(), v.begin(), v.end());
+        }
+        s.pos = p;
+        if (s.next == blocks.size()) {
+            if (s.avail()) return rec_fail(rec + 1, "the data ends inside the record");
+            break;
+        }
+        if (!s.fill(s.avail() >= 4 ? 4 + (uint64_t)rd32(s.buf.p + s.pos) : 4)) return corrupt();
+    }
+    fa->offsets.push_back(base_at);
+    fa->total = base_at;
+    fa->nib_bytes = nib_at;
+    nib.reserve(1);
+    void *pin = nullptr;                                     // pinned & 3: the codes that get uploaded, page-locked
+    if ((pinned & 3) && cudaHostAlloc(&pin, std::max<uint64_t>(nib_at, 1), cudaHostAllocDefault) == cudaSuccess) {
+        const uint64_t PIECE = 64u << 20;                    // copied a piece at a time, each piece's pages handed back
+        run_parallel(n_threads, (nib_at + PIECE - 1) / PIECE, [&](size_t i) {
+            const uint64_t a = i * PIECE, z = std::min(PIECE, nib_at - a);
+            memcpy((uint8_t *)pin + a, nib.p + a, z);
+            madvise(nib.p + a, z & ~(uint64_t)4095, MADV_DONTNEED);
+        });
+        fa->nib = (uint8_t *)pin;
+        fa->nib_pinned = true;
+    } else {
+        if (pinned & 3) cudaGetLastError();
+        fa->nib_map = nib.cap;
+        fa->nib = nib.release();
+    }
+    if (want_quals) {
+        quals.reserve(1);
+        fa->quals_map = quals.cap;
+        fa->quals = quals.release();
+    }
+    return CRF_OK;
+}
+
+// The text of a BAM handle (what samtools fastq writes as bases), decoded once, on the reader's threads.
+static int bam_decode(crf_fasta *fa) {
+    try {
+        if (!alloc_bases(fa, fa->total, fa->text_pinned)) {
+            set_err("crf_fasta_data: out of host memory (%llu bases)", (unsigned long long)fa->total);
+            return CRF_ERR_NOMEM;
+        }
+        const uint64_t PIECE = 4u << 20, total = fa->total;
+        const std::vector<uint64_t> &off = fa->offsets;
+        run_parallel(fa->n_threads, (total + PIECE - 1) / PIECE, [&](size_t i) {
+            const uint64_t lo = i * PIECE, hi = std::min(total, lo + PIECE);
+            uint64_t r = (uint64_t)(std::upper_bound(off.begin(), off.end(), lo) - off.begin()) - 1;
+            for (uint64_t pos = lo; pos < hi; ++r) {
+                if (off[r + 1] <= pos) continue;
+                const uint64_t i1 = std::min(hi, off[r + 1]) - off[r];
+                const uint8_t *d = fa->nib + fa->rec_byte[r];
+                uint8_t *o = fa->bases + off[r];
+                for (uint64_t j = pos - off[r]; j < i1; ++j) o[j] = (uint8_t)BAM_LETTERS[(d[j >> 1] >> (j & 1 ? 0 : 4)) & 15];
+                pos = off[r] + i1;
+            }
+        });
+    } catch (const std::bad_alloc &) {
+        set_err("crf_fasta_data: out of host memory");
+        return CRF_ERR_NOMEM;
+    }
+    return CRF_OK;
+}
+
+// The text of a .2bit or BAM handle, decoded on first use; nothing to do for the others.
+static int decode_text(crf_fasta *fa) {
+    if (fa->format == 2) return twobit_decode(fa);
+    if (fa->format != 3) return CRF_OK;
+    std::lock_guard<std::mutex> lock(fa->decode_mu);
+    return fa->bases ? CRF_OK : bam_decode(fa);
+}
+
 }  // namespace fasta_detail
 
 static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf_fasta **out);
@@ -732,13 +1040,48 @@ static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf
     }
     if (n >= 2 && t[0] == 0x1f && t[1] == 0x8b) {
         bool bad = false;
-        const bool bgzf = inflate_bgzf(file, n_threads, inflated, &bad);
+        std::vector<BgzfBlock> blocks;
+        uint64_t total = 0;
+        const bool bgzf = bgzf_index(file, blocks, &total);
+        if (bgzf) {                                     // a BAM file: its first inflated bytes are "BAM\1"
+            std::vector<uint8_t> head;                  // (the first 4 inflated bytes, from as many blocks as they span)
+            BgzfInflater inf(t);
+            bool head_ok = true;
+            for (size_t b = 0; b < blocks.size() && head.size() < 4 && head_ok; ++b) {
+                const size_t at = head.size();
+                head.resize(at + blocks[b].isize);
+                head_ok = inf.run(blocks[b], head.data() + at);
+            }
+            if (head_ok && is_bam_magic(head.data(), head.size())) {
+                struct Guard {
+                    crf_fasta *p;
+                    ~Guard() { if (p) crf_fasta_close(p); }
+                } guard{new crf_fasta};
+                crf_fasta *fa = guard.p;
+                fa->n_threads = n_threads;
+                fa->text_pinned = pinned;
+                const int rc = parse_bam(path, t, blocks, total, n_threads, pinned, fa);
+                if (rc != CRF_OK) return rc;
+                lap("bam");
+                guard.p = nullptr;
+                *out = fa;
+                return CRF_OK;
+            }
+            if (!inflated.reserve(total + 64)) throw std::bad_alloc();
+            inflated.size = total;
+            bad = !inflate_blocks(t, blocks, 0, blocks.size(), n_threads, inflated.p);
+        }
         if (bgzf && bad) { set_err("crf_fasta_open: %s has a corrupt BGZF block", path); return CRF_ERR_ARG; }
         // a plain gzip stream: the reader's own decoder (crf_inflate.h); whatever it does not take goes to zlib, which decides
         const bool own = !bgzf && getenv("CRF_GUNZIP_ZLIB") == nullptr && crf_inflate::gunzip(file.data, file.size, inflated, n_threads);
         if (!bgzf && !own && !inflate_all(file, plain)) { set_err("crf_fasta_open: %s is not a valid gzip stream", path); return CRF_ERR_ARG; }
         t = bgzf || own ? inflated.p : plain.data();
         n = bgzf || own ? inflated.size : plain.size();
+        if (is_bam_magic(t, n)) {
+            set_err("crf_fasta_open: %s is a BAM file compressed as plain gzip, not BGZF: BAM input must be BGZF "
+                    "(as samtools writes it)", path);
+            return CRF_ERR_ARG;
+        }
         lap(bgzf ? "bgzf" : own ? "gunzip" : "gzip/zlib");
     }
     lap("read");
@@ -897,8 +1240,8 @@ extern "C" int crf_fasta_info(const crf_fasta *fa, uint64_t *n_records, uint64_t
 extern "C" int crf_fasta_data(const crf_fasta *fa, const uint8_t **bases, const uint64_t **offsets, const char **names,
                               uint64_t *names_bytes) {
     if (!fa) { set_err("null fasta handle"); return CRF_ERR_ARG; }
-    if (bases && fa->format == 2) {                     // a .2bit file's text: decoded once, under the handle's lock
-        const int rc = fasta_detail::twobit_decode(const_cast<crf_fasta *>(fa));
+    if (bases) {                                        // a .2bit or BAM file's text: decoded once, under the handle's lock
+        const int rc = fasta_detail::decode_text(const_cast<crf_fasta *>(fa));
         if (rc != CRF_OK) return rc;
     }
     if (bases) *bases = fa->bases;
@@ -927,6 +1270,17 @@ extern "C" int crf_fasta_twobit(const crf_fasta *fa, const uint8_t **dna, const 
     return CRF_OK;
 }
 
+extern "C" int crf_fasta_nibbles(const crf_fasta *fa, const uint8_t **nib, const uint64_t **rec_byte, const uint64_t **exotic,
+                                 uint64_t *n_exotic) {
+    if (!fa || !nib || !rec_byte || !exotic || !n_exotic) { set_err("crf_fasta_nibbles: null argument"); return CRF_ERR_ARG; }
+    if (fa->format != 3) { set_err("crf_fasta_nibbles: not a BAM file"); return CRF_ERR_ARG; }
+    *nib = fa->nib;
+    *rec_byte = fa->rec_byte.data();
+    *exotic = fa->nib_exotic.data();
+    *n_exotic = fa->nib_exotic.size();
+    return CRF_OK;
+}
+
 extern "C" int crf_fasta_format(const crf_fasta *fa, int *format) {
     if (!fa || !format) { set_err("crf_fasta_format: null argument"); return CRF_ERR_ARG; }
     *format = fa->format;
@@ -943,7 +1297,10 @@ extern "C" int crf_fasta_close(crf_fasta *fa) {
     if (!fa) return CRF_OK;
     if (fa->pinned) cudaFreeHost(fa->bases);
     else free(fa->bases);
-    free(fa->quals);
+    if (fa->quals_map) munmap(fa->quals, fa->quals_map);
+    else free(fa->quals);
+    if (fa->nib_pinned) cudaFreeHost(fa->nib);
+    else if (fa->nib_map) munmap(fa->nib, fa->nib_map);
     if (fa->dna_pinned) cudaFreeHost((void *)fa->dna);
     else if (fa->dna_map) munmap(fa->dna_map, fa->dna_size);
     else free((void *)fa->dna);

@@ -176,7 +176,7 @@ extern "C" int crf_fasta_packed(crf_fasta *fa, uint32_t n_threads, const uint32_
     if (n_threads == 0) n_threads = std::min(16u, std::max(1u, std::thread::hardware_concurrency()));
     try {
         if (!fa->planes) {
-            const int rc = fasta_detail::twobit_decode(fa);  // (a .2bit file: its text, decoded on first use)
+            const int rc = fasta_detail::decode_text(fa);   // (a .2bit or BAM file: its text, decoded on first use)
             if (rc != CRF_OK) return rc;
             const uint64_t n_words = (fa->total + 31) / 32 + 1;
             const size_t bytes = (size_t)n_words * 12;

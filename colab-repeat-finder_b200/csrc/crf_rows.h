@@ -50,6 +50,18 @@ struct TwoBitMotif {
     }
 };
 
+// ... or a BAM file's 4-bit codes (record r's base i: nibble i & 1, high nibble first, of byte rec_byte[r] + i / 2), the
+// letters the decoded text has.
+struct NibbleMotif {
+    const uint8_t *nib;
+    const uint64_t *rec_byte;
+    char *operator()(char *p, uint32_t r, uint32_t start, uint32_t k) const {
+        const uint8_t *d = nib + rec_byte[r];
+        for (uint64_t i = start, e = (uint64_t)start + k; i < e; ++i) *p++ = "=ACMGRSVTWYHKDBN"[(d[i >> 1] >> (i & 1 ? 0 : 4)) & 15];
+        return p;
+    }
+};
+
 // origin (may be null): per record, added to the printed start and end (the motif is still read at start)
 template <class Motif>
 static int write_rows_impl(const char *path, int append, int tsv, const char *names, const Motif &motif,
@@ -165,6 +177,24 @@ extern "C" int crf_write_rows_twobit(const char *path, int append, int tsv, cons
     }
     try {
         return write_rows_impl(path, append, tsv, names, TwoBitMotif{dna, rec_byte}, nullptr, record, start, end, motif_size,
+                               n_rows, bytes);
+    } catch (const std::bad_alloc &) {
+        set_err("crf_write_rows: out of host memory");
+        return CRF_ERR_NOMEM;
+    }
+}
+
+// The rows of reads from a BAM file (crf_fasta_nibbles: nib, rec_byte), the motif read from the codes: the same bytes
+// crf_write_rows writes from the file's decoded text, without that text.
+extern "C" int crf_write_rows_nibbles(const char *path, int append, int tsv, const char *names, const uint8_t *nib,
+                                      const uint64_t *rec_byte, const uint32_t *record, const uint32_t *start,
+                                      const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
+    if (!path || (n_rows && (!nib || !rec_byte || !record || !start || !end || !motif_size)) || (!tsv && !names)) {
+        set_err("crf_write_rows: null argument");
+        return CRF_ERR_ARG;
+    }
+    try {
+        return write_rows_impl(path, append, tsv, names, NibbleMotif{nib, rec_byte}, nullptr, record, start, end, motif_size,
                                n_rows, bytes);
     } catch (const std::bad_alloc &) {
         set_err("crf_write_rows: out of host memory");

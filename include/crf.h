@@ -100,6 +100,17 @@ int crf_seq_load_packed_runs_ranges(crf_ctx *ctx, const uint32_t *H, const uint3
  * dna_on_device != 0: dna is a device pointer to the file's bytes (rec_byte, offsets and runs stay host arrays). */
 int crf_seq_load_2bit(crf_ctx *ctx, const uint8_t *dna, const uint64_t *rec_byte, const uint64_t *offsets, uint32_t n_records,
                       const uint64_t *runs, uint64_t n_runs, uint32_t max_motif_cap, int dna_on_device, crf_seq **seq);
+/* Reads of a BAM file (crf_fasta_nibbles), loaded from their 4-bit codes: record r holds offsets[r + 1] - offsets[r] bases,
+ * base i in nibble i & 1 (high nibble first) of byte rec_byte[r] + i / 2 of nib, codes =ACMGRSVTWYHKDBN (A = 1, C = 2,
+ * G = 4, T = 8, N = 15).  Every code other than A, C, G, T is masked; the exotic list (position in the space of offsets
+ * << 8 | letter, ascending; entries outside [offsets[0], offsets[n_records]) are ignored, so a load of some of the records
+ * takes the whole file's list) gives the codes other than A, C, G, T and N their letters, as crf_seq_load_packed does.  The
+ * byte span the records cover goes up at 0.5 B/bp, in chunks on a second stream while nibble_pack_kernel lays out the
+ * words whose bytes have arrived.  The rows equal those of crf_seq_load_ascii on the decoded text (crf_fasta_data).
+ * nib_on_device != 0: nib is a device pointer (rec_byte, offsets and exotic stay host arrays). */
+int crf_seq_load_nibbles(crf_ctx *ctx, const uint8_t *nib, const uint64_t *rec_byte, const uint64_t *offsets,
+                         uint32_t n_records, const uint64_t *exotic, uint64_t n_exotic, uint32_t max_motif_cap,
+                         int nib_on_device, crf_seq **seq);
 /* Host only: the maximal runs of set bits of an NM plane over [0, n_bases) (threaded).  *n_runs = how many there are
  * (CRF_ERR_CAPACITY if more than cap pairs: call again with a longer list). */
 int crf_mask_runs(const uint32_t *NM, uint64_t n_bases, uint32_t n_threads, uint64_t *runs, uint64_t cap, uint64_t *n_runs);
@@ -321,6 +332,12 @@ int crf_write_rows_at(const char *path, int append, int tsv, const char *names, 
 int crf_write_rows_twobit(const char *path, int append, int tsv, const char *names, const uint8_t *dna,
                           const uint64_t *rec_byte, const uint32_t *record, const uint32_t *start, const uint32_t *end,
                           const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes);
+/* crf_write_rows for reads of a BAM file: the motif is read from their 4-bit codes (nib and rec_byte as crf_fasta_nibbles
+ * gives them: record r's base i is nibble i & 1, high nibble first, of byte rec_byte[r] + i / 2) as the letters
+ * =ACMGRSVTWYHKDBN -- byte-identical to crf_write_rows on the file's decoded text (crf_fasta_data). */
+int crf_write_rows_nibbles(const char *path, int append, int tsv, const char *names, const uint8_t *nib,
+                           const uint64_t *rec_byte, const uint32_t *record, const uint32_t *start, const uint32_t *end,
+                           const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes);
 /* A repeat-masked FASTA file: per record a header line ">name" (names NUL-separated, as crf_write_rows takes them), then
  * its bases, line_width per line.  Mask bit p (as crf_mask_rows lays it out) stands for bases[p], with the indexing of
  * offsets (record r = bases[offsets[r] .. offsets[r+1])).  A masked byte is lower-cased when it is an ASCII letter A-Z
@@ -356,12 +373,21 @@ int crf_fasta_data(const crf_fasta *fasta, const uint8_t **bases, const uint64_t
  * checked against the file size and dnaSize, and a bad file is CRF_ERR_ARG naming the 1-based record.  N blocks and mask
  * blocks may be unsorted or overlap; they are merged per record.  crf_fasta_data then decodes the text on first call (on the
  * reader's threads): what twoBitToFa writes, T/C/A/G, N blocks as 'N', mask blocks lower-cased ('n' inside both).
- * *format = 0 for a FASTA file, 1 for a FASTQ file, 2 for a .2bit file. */
+ * BAM too: a BGZF file whose first inflated bytes are "BAM\1" is read as unaligned reads, giving what `samtools fastq -n`
+ * writes from it: the records with (flag & 0x900) == 0 in file order, named by read_name, their bases reverse-complemented
+ * when flag & 0x10, qualities + 33 (reversed with them; '"' when absent).  The blocks are inflated on the reader's threads
+ * a window of 32 MiB at a time and only the 4-bit codes (crf_fasta_nibbles), the names and, with pinned bit 2, the
+ * qualities are kept: host memory peaks at the window, plus the largest record, plus what is kept (with pinned & 3 the
+ * codes are then copied into page-locked memory, so for that moment they are held twice).  Every count and length
+ * is checked against the record and the stream; a malformed record is CRF_ERR_ARG naming its 1-based number (a missing
+ * end-of-file block is accepted), and a BAM compressed as plain gzip rather than BGZF is CRF_ERR_ARG.  crf_fasta_data
+ * decodes the text on its first call (on the reader's threads), letters of =ACMGRSVTWYHKDBN.
+ * *format = 0 for a FASTA file, 1 for a FASTQ file, 2 for a .2bit file, 3 for a BAM file. */
 int crf_fasta_format(const crf_fasta *fasta, int *format);
-/* A FASTQ file's qualities, laid out like the bases (record r = quals[offsets[r] .. offsets[r+1])); NULL for a FASTA
- * file or when crf_fasta_open was not given pinned bit 2. */
+/* A FASTQ or BAM file's qualities, laid out like the bases (record r = quals[offsets[r] .. offsets[r+1])); NULL for other
+ * formats or when crf_fasta_open was not given pinned bit 2. */
 int crf_fasta_quals(const crf_fasta *fasta, const uint8_t **quals);
-/* Offsets (n_records + 1) and NUL-separated names of any handle, without decoding a .2bit file's bases. */
+/* Offsets (n_records + 1) and NUL-separated names of any handle, without decoding a .2bit or BAM file's bases. */
 int crf_fasta_index(const crf_fasta *fasta, const uint64_t **offsets, const char **names, uint64_t *names_bytes);
 /* A .2bit handle's packed form (CRF_ERR_ARG for any other): dna = the file's bytes (page-locked when crf_fasta_open had
  * pinned & 3, else mapped), rec_byte[r] = the byte where record r's packed bases start, runs = its N blocks as n_runs
@@ -369,6 +395,12 @@ int crf_fasta_index(const crf_fasta *fasta, const uint64_t **offsets, const char
  * records) -- what crf_seq_load_2bit and crf_write_rows_twobit take. */
 int crf_fasta_twobit(const crf_fasta *fasta, const uint8_t **dna, const uint64_t **rec_byte, const uint64_t **runs,
                      uint64_t *n_runs);
+/* A BAM handle's packed form (CRF_ERR_ARG for any other): nib = the reads' 4-bit codes (page-locked when crf_fasta_open
+ * had pinned & 3), record r from byte rec_byte[r] with reverse complements applied (an odd record's last byte has a low
+ * nibble 0), exotic = the n_exotic codes other than A, C, G, T and N as (position in the space of the offsets << 8 | letter),
+ * ascending -- what crf_seq_load_nibbles and crf_write_rows_nibbles take. */
+int crf_fasta_nibbles(const crf_fasta *fasta, const uint8_t **nib, const uint64_t **rec_byte, const uint64_t **exotic,
+                      uint64_t *n_exotic);
 /* Packed planes of the whole file (all records back to back, as crf_seq_load_packed takes them), made on first call
  * and owned by the handle; page-locked when the base buffer is. */
 int crf_fasta_packed(crf_fasta *fasta, uint32_t n_threads, const uint32_t **H, const uint32_t **L, const uint32_t **NM,
