@@ -280,37 +280,25 @@ class Sequence:
         self.ctx = ctx
         self._h = ctypes.c_void_p()
         keep = None
-        if nibbles is not None:
-            src = nibbles
-            ptr, on_device = _source_bytes("nib", src.nib, on_device)
+        src = twobit if twobit is not None else nibbles
+        if src is not None:                               # a .2bit or BAM source: bytes of codes, read from rec_byte[r]
+            what, per_byte, kind, load = (("dna", 4, ".2bit", lib().crf_seq_load_2bit) if twobit is not None else
+                                          ("nib", 2, "BAM", lib().crf_seq_load_nibbles))
+            codes = getattr(src, what)
+            ptr, on_device = _source_bytes(what, codes, on_device)
             offsets = np.ascontiguousarray(src.offsets, dtype=np.uint64)
             rec_byte = np.ascontiguousarray(src.rec_byte, dtype=np.uint64)
-            exotic = np.ascontiguousarray(src.exotic, dtype=np.uint64)
+            lst = (np.ascontiguousarray(src.runs, dtype=np.uint64).reshape(-1, 2) if twobit is not None else
+                   np.ascontiguousarray(src.exotic, dtype=np.uint64))
             if offsets.ndim != 1 or offsets.size < 2 or rec_byte.shape != (offsets.size - 1,):
-                raise ValueError("a BAM source needs n_records + 1 offsets and n_records rec_byte entries")
-            _check_extent("nib", src.nib, rec_byte, offsets, 2)
+                raise ValueError(f"a {kind} source needs n_records + 1 offsets and n_records rec_byte entries")
+            _check_extent(what, codes, rec_byte, offsets, per_byte)
             self.offsets = offsets
             self.n_records = offsets.size - 1
-            _check(lib().crf_seq_load_nibbles(ctx._h, ctypes.c_void_p(ptr), ctypes.c_void_p(rec_byte.ctypes.data),
-                                              ctypes.c_void_p(offsets.ctypes.data), self.n_records,
-                                              ctypes.c_void_p(exotic.ctypes.data if exotic.size else 0), exotic.size,
-                                              int(max_motif_cap), int(bool(on_device)), ctypes.byref(self._h)))
-            return
-        if twobit is not None:
-            src = twobit
-            ptr, on_device = _source_bytes("dna", src.dna, on_device)
-            offsets = np.ascontiguousarray(src.offsets, dtype=np.uint64)
-            rec_byte = np.ascontiguousarray(src.rec_byte, dtype=np.uint64)
-            runs = np.ascontiguousarray(src.runs, dtype=np.uint64).reshape(-1, 2)
-            if offsets.ndim != 1 or offsets.size < 2 or rec_byte.shape != (offsets.size - 1,):
-                raise ValueError("a .2bit source needs n_records + 1 offsets and n_records rec_byte entries")
-            _check_extent("dna", src.dna, rec_byte, offsets, 4)
-            self.offsets = offsets
-            self.n_records = offsets.size - 1
-            _check(lib().crf_seq_load_2bit(ctx._h, ctypes.c_void_p(ptr), ctypes.c_void_p(rec_byte.ctypes.data),
-                                           ctypes.c_void_p(offsets.ctypes.data), self.n_records,
-                                           ctypes.c_void_p(runs.ctypes.data if runs.size else 0), runs.shape[0],
-                                           int(max_motif_cap), int(bool(on_device)), ctypes.byref(self._h)))
+            _check(load(ctx._h, ctypes.c_void_p(ptr), ctypes.c_void_p(rec_byte.ctypes.data),
+                        ctypes.c_void_p(offsets.ctypes.data), self.n_records,
+                        ctypes.c_void_p(lst.ctypes.data if lst.size else 0), lst.shape[0],
+                        int(max_motif_cap), int(bool(on_device)), ctypes.byref(self._h)))
             return
         if packed is not None:
             pk = packed
@@ -740,38 +728,29 @@ class Fasta:
                                                 shape=(max(self.total_bases, 1),))[:self.total_bases]
         return self._bases
 
+    def _codes(self, fn, per_byte):
+        """(codes, rec_byte, list address, list length) from crf_fasta_twobit or crf_fasta_nibbles (ValueError for any other
+        format).  codes is a view of the handle's bytes up to the end of the last record's, valid until close()."""
+        codes, rec_byte, lst, n = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_uint64()
+        _check(fn(self._h, ctypes.byref(codes), ctypes.byref(rec_byte), ctypes.byref(lst), ctypes.byref(n)))
+        rb = _u64s(rec_byte, self.n_records)
+        lengths = np.diff(self.offsets.astype(np.int64))
+        size = int((rb.astype(np.int64) + (lengths + per_byte - 1) // per_byte).max()) if self.n_records else 0
+        view = np.ctypeslib.as_array(ctypes.cast(codes, ctypes.POINTER(ctypes.c_uint8)), shape=(max(size, 1),))[:size] \
+            if codes.value else np.zeros(0, np.uint8)
+        return view, rb, lst, n.value
+
     def twobit(self):
         """TwoBitSource of a .2bit file (crf_fasta_twobit; ValueError for any other format).  dna is a view of the handle's
         bytes, valid until close()."""
-        dna, rec_byte, runs, n_runs = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_uint64()
-        _check(lib().crf_fasta_twobit(self._h, ctypes.byref(dna), ctypes.byref(rec_byte), ctypes.byref(runs),
-                                      ctypes.byref(n_runs)))
-        def u64s(ptr, n):
-            return np.ctypeslib.as_array(ctypes.cast(ptr, ctypes.POINTER(ctypes.c_uint64)), shape=(n,)).copy() \
-                if n else np.zeros(0, np.uint64)
-        rb = u64s(rec_byte, self.n_records)
-        rn = u64s(runs, 2 * n_runs.value).reshape(-1, 2)
-        lengths = np.diff(self.offsets.astype(np.int64))
-        size = int((rb.astype(np.int64) + (lengths + 3) // 4).max()) if self.n_records else 0
-        view = np.ctypeslib.as_array(ctypes.cast(dna, ctypes.POINTER(ctypes.c_uint8)), shape=(max(size, 1),))[:size] \
-            if dna.value else np.zeros(0, np.uint8)
-        return TwoBitSource(view, rb, self.offsets, rn, keep=self)
+        dna, rb, runs, n_runs = self._codes(lib().crf_fasta_twobit, 4)
+        return TwoBitSource(dna, rb, self.offsets, _u64s(runs, 2 * n_runs).reshape(-1, 2), keep=self)
 
     def nibbles(self):
         """NibbleSource of a BAM file (crf_fasta_nibbles; ValueError for any other format).  nib is a view of the handle's
         codes, valid until close()."""
-        nib, rec_byte, ex, n_ex = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_uint64()
-        _check(lib().crf_fasta_nibbles(self._h, ctypes.byref(nib), ctypes.byref(rec_byte), ctypes.byref(ex),
-                                       ctypes.byref(n_ex)))
-        def u64s(ptr, n):
-            return np.ctypeslib.as_array(ctypes.cast(ptr, ctypes.POINTER(ctypes.c_uint64)), shape=(n,)).copy() \
-                if n else np.zeros(0, np.uint64)
-        rb = u64s(rec_byte, self.n_records)
-        lengths = np.diff(self.offsets.astype(np.int64))
-        size = int((rb.astype(np.int64) + (lengths + 1) // 2).max()) if self.n_records else 0
-        view = np.ctypeslib.as_array(ctypes.cast(nib, ctypes.POINTER(ctypes.c_uint8)), shape=(max(size, 1),))[:size] \
-            if nib.value else np.zeros(0, np.uint8)
-        return NibbleSource(view, rb, self.offsets, u64s(ex, n_ex.value), keep=self)
+        nib, rb, ex, n_ex = self._codes(lib().crf_fasta_nibbles, 2)
+        return NibbleSource(nib, rb, self.offsets, _u64s(ex, n_ex), keep=self)
 
     @property
     def names(self):
@@ -790,9 +769,7 @@ class Fasta:
         n_ex = ctypes.c_uint64()
         _check(lib().crf_fasta_packed(self._h, int(n_threads), ctypes.byref(H), ctypes.byref(L), ctypes.byref(NM),
                                       ctypes.byref(ex), ctypes.byref(n_ex)))
-        exotic = np.ctypeslib.as_array(ctypes.cast(ex, ctypes.POINTER(ctypes.c_uint64)), shape=(n_ex.value,)).copy() \
-            if n_ex.value else np.zeros(0, np.uint64)
-        return PackedPlanes(self.total_bases, H.value, L.value, NM.value, exotic, keep=self).with_runs(n_threads)
+        return PackedPlanes(self.total_bases, H.value, L.value, NM.value, _u64s(ex, n_ex.value), keep=self).with_runs(n_threads)
 
     def close(self):
         if self._h:
@@ -813,67 +790,58 @@ class Fasta:
             pass
 
 
-def write_rows(path, names, bases, offsets, record, start, end, k, tsv=False, append=False, origin=None):
-    """Native BED / TSV writer (crf_write_rows).  bases: bytes or uint8 array with all records back to back;
-    names: list of str, or the NUL-separated blob.  origin: per record, a uint64 added to the printed start and end
-    (crf_write_rows_at; the rows of a record longer than 2^32 bases are written unit by unit, relative to each unit)."""
+def _u64s(ptr, n):
+    """A copy of n uint64 at a library address (an empty array when n is 0)."""
+    return np.ctypeslib.as_array(ctypes.cast(ptr, ctypes.POINTER(ctypes.c_uint64)), shape=(n,)).copy() \
+        if n else np.zeros(0, np.uint64)
+
+
+def _write_rows_with(fn, path, names, src, record, start, end, k, tsv, append):
+    """One of the native rows writers: fn(path, append, tsv, names blob, *src, record, start, end, k, n_rows, &bytes), where
+    src are the arguments that say where the motif is read.  names: list of str, or the NUL-separated blob."""
     if isinstance(names, (bytes, bytearray)):
         blob = bytes(names)
     else:
         blob = b"".join(n.encode("utf-8") + b"\0" for n in names) if names is not None else None
     arrs = [np.ascontiguousarray(a, dtype=np.uint32) for a in (record, start, end, k)]
+    nbytes = ctypes.c_uint64()
+    _check(fn(os.fsencode(path), int(append), int(tsv),
+              ctypes.cast(ctypes.c_char_p(blob), ctypes.c_void_p) if blob is not None else None, *src,
+              *(ctypes.c_void_p(a.ctypes.data) for a in arrs), len(arrs[0]), ctypes.byref(nbytes)))
+    return nbytes.value
+
+
+def write_rows(path, names, bases, offsets, record, start, end, k, tsv=False, append=False, origin=None):
+    """Native BED / TSV writer (crf_write_rows).  bases: bytes or uint8 array with all records back to back;
+    names: list of str, or the NUL-separated blob.  origin: per record, a uint64 added to the printed start and end
+    (crf_write_rows_at; the rows of a record longer than 2^32 bases are written unit by unit, relative to each unit)."""
     offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
     if isinstance(bases, np.ndarray):
         bptr = bases.ctypes.data
     else:
         bptr = ctypes.cast(ctypes.c_char_p(bases), ctypes.c_void_p).value or 0
-    nbytes = ctypes.c_uint64()
-    head = (os.fsencode(path), int(append), int(tsv),
-            ctypes.cast(ctypes.c_char_p(blob), ctypes.c_void_p) if blob is not None else None,
-            ctypes.c_void_p(bptr), ctypes.c_void_p(offsets.ctypes.data))
-    tail = (*(ctypes.c_void_p(a.ctypes.data) for a in arrs), len(arrs[0]), ctypes.byref(nbytes))
+    src = (ctypes.c_void_p(bptr), ctypes.c_void_p(offsets.ctypes.data))
     if origin is None:
-        _check(lib().crf_write_rows(*head, *tail))
-    else:
-        origin = np.ascontiguousarray(origin, dtype=np.uint64)
-        _check(lib().crf_write_rows_at(*head, ctypes.c_void_p(origin.ctypes.data), *tail))
-    return nbytes.value
+        return _write_rows_with(lib().crf_write_rows, path, names, src, record, start, end, k, tsv, append)
+    origin = np.ascontiguousarray(origin, dtype=np.uint64)
+    return _write_rows_with(lib().crf_write_rows_at, path, names, (*src, ctypes.c_void_p(origin.ctypes.data)), record, start,
+                            end, k, tsv, append)
 
 
 def write_rows_twobit(path, names, dna, rec_byte, record, start, end, k, tsv=False, append=False):
     """crf_write_rows_twobit: write_rows for records of a .2bit file, the motif read from the packed bytes (dna: host uint8
     array of the file's bytes, rec_byte[r]: where record r's bases start, as TwoBitSource has them)."""
-    if isinstance(names, (bytes, bytearray)):
-        blob = bytes(names)
-    else:
-        blob = b"".join(n.encode("utf-8") + b"\0" for n in names) if names is not None else None
-    arrs = [np.ascontiguousarray(a, dtype=np.uint32) for a in (record, start, end, k)]
     rec_byte = np.ascontiguousarray(rec_byte, dtype=np.uint64)
-    dptr, _ = _host_bytes("dna", dna)
-    nbytes = ctypes.c_uint64()
-    _check(lib().crf_write_rows_twobit(os.fsencode(path), int(append), int(tsv),
-                                       ctypes.cast(ctypes.c_char_p(blob), ctypes.c_void_p) if blob is not None else None,
-                                       ctypes.c_void_p(dptr), ctypes.c_void_p(rec_byte.ctypes.data),
-                                       *(ctypes.c_void_p(a.ctypes.data) for a in arrs), len(arrs[0]), ctypes.byref(nbytes)))
-    return nbytes.value
+    src = (ctypes.c_void_p(_host_bytes("dna", dna)[0]), ctypes.c_void_p(rec_byte.ctypes.data))
+    return _write_rows_with(lib().crf_write_rows_twobit, path, names, src, record, start, end, k, tsv, append)
 
 
 def write_rows_nibbles(path, names, nib, rec_byte, record, start, end, k, tsv=False, append=False):
     """crf_write_rows_nibbles: write_rows for reads of a BAM file, the motif read from the 4-bit codes (nib: host uint8
     array, rec_byte[r]: where record r's codes start, as NibbleSource has them)."""
-    if isinstance(names, (bytes, bytearray)):
-        blob = bytes(names)
-    else:
-        blob = b"".join(n.encode("utf-8") + b"\0" for n in names) if names is not None else None
-    arrs = [np.ascontiguousarray(a, dtype=np.uint32) for a in (record, start, end, k)]
     rec_byte = np.ascontiguousarray(rec_byte, dtype=np.uint64)
-    nptr, _ = _host_bytes("nib", nib)
-    nbytes = ctypes.c_uint64()
-    _check(lib().crf_write_rows_nibbles(os.fsencode(path), int(append), int(tsv),
-                                        ctypes.cast(ctypes.c_char_p(blob), ctypes.c_void_p) if blob is not None else None,
-                                        ctypes.c_void_p(nptr), ctypes.c_void_p(rec_byte.ctypes.data),
-                                        *(ctypes.c_void_p(a.ctypes.data) for a in arrs), len(arrs[0]), ctypes.byref(nbytes)))
-    return nbytes.value
+    src = (ctypes.c_void_p(_host_bytes("nib", nib)[0]), ctypes.c_void_p(rec_byte.ctypes.data))
+    return _write_rows_with(lib().crf_write_rows_nibbles, path, names, src, record, start, end, k, tsv, append)
 
 
 def _check_extent(what, buf, rec_byte, offsets, per_byte):

@@ -6,7 +6,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(os.path.dirname(_HERE), "csrc")
 OUT = os.path.join(_HERE, "libcrf.so")
 SOURCES = ["crf_api.cu"]
-HEADERS = ["crf_device.cuh", "crf_scan.cuh", "crf_scan_warp.cuh", "crf_aux.cuh", "crf_stop.cuh", "crf_xchg.cuh", "crf_fasta.h", "crf_pack.h", "crf_inflate.h", "crf_rows.h", "crf_mask.cuh", "crf_fasta_out.h"]
+HEADERS = ["crf_device.cuh", "crf_scan.cuh", "crf_scan_warp.cuh", "crf_aux.cuh", "crf_stop.cuh", "crf_xchg.cuh", "crf_fasta.h", "crf_codes.h", "crf_pack.h", "crf_inflate.h", "crf_rows.h", "crf_mask.cuh", "crf_fasta_out.h"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-shared", "-cudart", "shared", "-Xcompiler", "-fPIC,-pthread"]   # cudart linked dynamically: the runtime's own
                                                                                # symbol table stays out of the shipped .so

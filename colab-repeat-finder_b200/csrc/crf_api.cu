@@ -366,9 +366,9 @@ struct LoadSource {
     const uint64_t *nm_runs = nullptr;                  // packed, instead of pN: the masked positions as sorted runs
     uint64_t n_runs = 0;                                //   [runs[2i], runs[2i+1]) -- 0.25 B/bp cross PCIe instead of 0.375
     bool runs_mode = false;
-    const uint8_t *twobit = nullptr;                    // .2bit (runs mode): source position p = base p & 3 of byte p >> 2
-    const uint8_t *nibbles = nullptr;                   // BAM codes: source position p = nibble p & 1 of byte p >> 1
-    bool packed() const { return pH != nullptr || twobit != nullptr || nibbles != nullptr; }
+    const uint8_t *codes = nullptr;                     // .2bit (code_bits 2, runs mode) or BAM (4) codes, crf_codes.h: source
+    uint32_t code_bits = 0;                             //   position p = code p % (8 / code_bits) of byte p / (8 / code_bits)
+    bool packed() const { return pH != nullptr || codes != nullptr; }
 };
 
 // The two passes over the per-record arrays of a load run on a few threads when there are millions of records.
@@ -405,7 +405,7 @@ struct LoadTrace {
 static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, const uint64_t *lengths,
                      const uint64_t *own_lo, const uint64_t *own_hi, uint32_t n_records, uint32_t max_motif_cap,
                      int on_device, crf_seq *s) {
-    const char *who = src.twobit ? "crf_seq_load_2bit" : src.nibbles ? "crf_seq_load_nibbles"
+    const char *who = src.code_bits == 2 ? "crf_seq_load_2bit" : src.code_bits == 4 ? "crf_seq_load_nibbles"
                     : src.packed() ? "crf_seq_load_packed" : "crf_seq_load_ascii";
     LoadTrace trace;
     cudaStream_t st = c->stream;
@@ -490,7 +490,7 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
     // The source span the records cover (units may overlap) goes up in chunks on a second stream while the pack kernel
     // works on the layout words whose source has already arrived (the PCIe copy is ~10x longer than the packing, which
     // then hides behind it).  Unit of the span: bytes (ASCII) or positions rounded out to whole 32-bit words (packed).
-    const bool packed = src.packed(), twobit = src.twobit != nullptr, nibbles = src.nibbles != nullptr;
+    const bool packed = src.packed(), twobit = src.code_bits == 2, nibbles = src.code_bits == 4;
     const uint64_t src_end = src_hi;                                     // .2bit / BAM: bytes up to (src_end + 3) / 4 or
                                                                          // (src_end + 1) / 2 are the caller's
     if (packed) { src_lo &= ~31ull; src_hi = (src_hi + 31) & ~31ull; }
@@ -544,15 +544,11 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
     trace.mark("source allocs + runs_rel");
     auto copy_span = [&](uint64_t lo, uint64_t n, cudaStream_t cs) -> cudaError_t {    // source positions [src_lo + lo, + n)
         if (!n) return cudaSuccess;
-        if (twobit) {                                                    // (lo is a multiple of 32: whole bytes)
-            const uint64_t b0 = (src_lo + lo) / 4, b1 = std::min((src_lo + lo + n + 3) / 4, (src_end + 3) / 4);
+        if (src.codes) {                                                 // (lo is a multiple of 32: whole bytes)
+            const uint64_t per = 8 / src.code_bits;
+            const uint64_t b0 = (src_lo + lo) / per, b1 = std::min((src_lo + lo + n + per - 1) / per, (src_end + per - 1) / per);
             if (b1 <= b0) return cudaSuccess;
-            return cudaMemcpyAsync((uint8_t *)d_planes_own + lo / 4, src.twobit + b0, b1 - b0, cudaMemcpyHostToDevice, cs);
-        }
-        if (nibbles) {
-            const uint64_t b0 = (src_lo + lo) / 2, b1 = std::min((src_lo + lo + n + 1) / 2, (src_end + 1) / 2);
-            if (b1 <= b0) return cudaSuccess;
-            return cudaMemcpyAsync((uint8_t *)d_planes_own + lo / 2, src.nibbles + b0, b1 - b0, cudaMemcpyHostToDevice, cs);
+            return cudaMemcpyAsync((uint8_t *)d_planes_own + lo / per, src.codes + b0, b1 - b0, cudaMemcpyHostToDevice, cs);
         }
         if (!packed) return cudaMemcpyAsync(d_src_own + lo, src.bases + src_lo + lo, n, cudaMemcpyHostToDevice, cs);
         const uint64_t w0 = lo / 32, nw = (n + 31) / 32, h0 = src_lo / 32 + w0;
@@ -666,7 +662,7 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
         if (w_hi <= w_lo) return cudaSuccess;
         if (twobit) {
             TwoBitParams tp;
-            tp.dna = on_device ? src.twobit : (const uint8_t *)d_planes_own;
+            tp.dna = on_device ? src.codes : (const uint8_t *)d_planes_own;
             tp.n_bytes = (src_end + 3) / 4 - (on_device ? 0 : src_lo / 4);
             tp.sN = d_pN; tp.src_base = src_base;
             tp.rec_src_start = d_src_start; tp.rec_len = s->d_rec_len; tp.rec_dev_off = s->d_rec_dev_off;
@@ -675,7 +671,7 @@ static int load_impl(crf_ctx *c, const LoadSource &src, const uint64_t *starts, 
             twobit_pack_kernel<<<(w_hi - w_lo + 255) / 256, 256, 0, st>>>(tp);
         } else if (nibbles) {
             NibbleParams np;
-            np.nib = on_device ? src.nibbles : (const uint8_t *)d_planes_own;
+            np.nib = on_device ? src.codes : (const uint8_t *)d_planes_own;
             np.n_bytes = (src_end + 1) / 2 - (on_device ? 0 : src_lo / 2);
             np.src_base = src_base;
             np.rec_src_start = d_src_start; np.rec_len = s->d_rec_len; np.rec_dev_off = s->d_rec_dev_off;
@@ -825,7 +821,7 @@ static int load_checked(crf_ctx *c, const LoadSource &src, const uint64_t *start
         set_err("%s: max_motif_cap %u not in [1, %u]", who, max_motif_cap, MAX_K);
         return max_motif_cap < 1 ? CRF_ERR_ARG : CRF_ERR_UNSUPPORTED;
     }
-    const bool have_src = src.twobit || src.nibbles ? true : src.packed() ? (src.pL && src.pN) : (src.bases != nullptr);
+    const bool have_src = src.codes ? true : src.packed() ? (src.pL && src.pN) : (src.bases != nullptr);
     if (!have_src) {
         for (uint32_t r = 0; r < n_records; ++r)
             if (lengths ? lengths[r] : starts[r + 1] - starts[r]) { set_err("%s: null %s", who, src.packed() ? "plane" : "bases"); return CRF_ERR_ARG; }
@@ -872,6 +868,15 @@ extern "C" int crf_seq_load_ascii(crf_ctx *c, const uint8_t *bases, const uint64
     return load_checked(c, src, offsets, nullptr, nullptr, nullptr, n_records, max_motif_cap, bases_on_device, out, "crf_seq_load_ascii");
 }
 
+static int check_runs(const uint64_t *runs, uint64_t n_runs, const char *who) {
+    for (uint64_t i = 0; i < n_runs; ++i)
+        if (runs[2 * i] >= runs[2 * i + 1] || (i && runs[2 * i] < runs[2 * i - 1])) {
+            set_err("%s: runs must be non-empty, ascending and disjoint (run %llu)", who, (unsigned long long)i);
+            return CRF_ERR_ARG;
+        }
+    return CRF_OK;
+}
+
 static int packed_load(crf_ctx *c, const uint32_t *H, const uint32_t *L, const uint32_t *NM, const uint64_t *exotic,
                        uint64_t n_exotic, const uint64_t *starts, const uint64_t *lengths, const uint64_t *own_lo,
                        const uint64_t *own_hi, uint32_t n_records, uint32_t max_motif_cap, int planes_on_device, crf_seq **out) {
@@ -890,11 +895,7 @@ static int packed_runs_load(crf_ctx *c, const uint32_t *H, const uint32_t *L, co
                             int planes_on_device, crf_seq **out) {
     if (!H || !L) { set_err("crf_seq_load_packed_runs: null plane"); return CRF_ERR_ARG; }
     if (n_runs && !runs) { set_err("crf_seq_load_packed_runs: null run list"); return CRF_ERR_ARG; }
-    for (uint64_t i = 0; i < n_runs; ++i)
-        if (runs[2 * i] >= runs[2 * i + 1] || (i && runs[2 * i] < runs[2 * i - 1])) {
-            set_err("crf_seq_load_packed_runs: runs must be non-empty, ascending and disjoint (run %llu)", (unsigned long long)i);
-            return CRF_ERR_ARG;
-        }
+    CHECK(check_runs(runs, n_runs, "crf_seq_load_packed_runs"));
     LoadSource src;
     src.pH = H; src.pL = L; src.pN = H;      // (pN is not read in runs mode; non-null for the argument check)
     src.exotic = exotic; src.n_exotic = n_exotic;
@@ -928,30 +929,42 @@ extern "C" int crf_seq_load_packed_runs(crf_ctx *c, const uint32_t *H, const uin
                             planes_on_device, out);
 }
 
-// .2bit records: record r = offsets[r + 1] - offsets[r] bases packed from byte rec_byte[r] of dna (the file's bytes), its
-// N blocks among the runs of offsets' position space.  The load sees record r at source position 4 rec_byte[r] (the
-// position of its first base in the bytes) and the runs moved there, split at record ends.
+// What crf_seq_load_2bit and crf_seq_load_nibbles share: the checks, and record r = offsets[r + 1] - offsets[r] bases coded
+// from byte rec_byte[r] of src.codes, which the load sees at source position (8 / code_bits) rec_byte[r] (the position of its
+// first code in the bytes).  null_list: the entry point's list is missing.
+static int code_records(const LoadSource &src, const uint64_t *rec_byte, const uint64_t *offsets, uint32_t n_records,
+                        bool null_list, const char *who, std::vector<uint64_t> &starts, std::vector<uint64_t> &lengths) {
+    CHECK(check_offsets(offsets, n_records, who));
+    if (!src.codes || !rec_byte || null_list) { set_err("%s: null argument", who); return CRF_ERR_ARG; }
+    for (uint32_t r = 0; r < n_records; ++r)
+        if (offsets[r + 1] < offsets[r]) { set_err("%s: offsets must be non-decreasing", who); return CRF_ERR_ARG; }
+    try {
+        starts.resize(n_records);
+        lengths.resize(n_records);
+    } catch (const std::bad_alloc &) {
+        set_err("out of host memory");
+        return CRF_ERR_NOMEM;
+    }
+    const uint64_t per_byte = 8 / src.code_bits;
+    for (uint32_t r = 0; r < n_records; ++r) {
+        starts[r] = per_byte * rec_byte[r];
+        lengths[r] = offsets[r + 1] - offsets[r];
+    }
+    return CRF_OK;
+}
+
+// .2bit records (code_records), their N blocks among the runs of offsets' position space: the load sees the runs moved to
+// the records' source positions, split at record ends.
 extern "C" int crf_seq_load_2bit(crf_ctx *c, const uint8_t *dna, const uint64_t *rec_byte, const uint64_t *offsets,
                                  uint32_t n_records, const uint64_t *runs, uint64_t n_runs, uint32_t max_motif_cap,
                                  int dna_on_device, crf_seq **out) {
     const char *who = "crf_seq_load_2bit";
-    CHECK(check_offsets(offsets, n_records, who));
-    if (!dna || !rec_byte || (n_runs && !runs)) { set_err("%s: null argument", who); return CRF_ERR_ARG; }
-    for (uint32_t r = 0; r < n_records; ++r)
-        if (offsets[r + 1] < offsets[r]) { set_err("%s: offsets must be non-decreasing", who); return CRF_ERR_ARG; }
-    for (uint64_t i = 0; i < n_runs; ++i)
-        if (runs[2 * i] >= runs[2 * i + 1] || (i && runs[2 * i] < runs[2 * i - 1])) {
-            set_err("%s: runs must be non-empty, ascending and disjoint (run %llu)", who, (unsigned long long)i);
-            return CRF_ERR_ARG;
-        }
+    LoadSource src;
+    src.codes = dna; src.code_bits = 2;
     std::vector<uint64_t> starts, lengths, moved;
+    CHECK(code_records(src, rec_byte, offsets, n_records, n_runs && !runs, who, starts, lengths));
+    CHECK(check_runs(runs, n_runs, who));
     try {
-        starts.resize(n_records);
-        lengths.resize(n_records);
-        for (uint32_t r = 0; r < n_records; ++r) {
-            starts[r] = 4 * rec_byte[r];
-            lengths[r] = offsets[r + 1] - offsets[r];
-        }
         const uint64_t pos0 = offsets[0], pos1 = offsets[n_records];
         uint64_t a_i = 0, b_i = n_runs;                                  // first run that ends after pos0
         while (a_i < b_i) { const uint64_t m = (a_i + b_i) / 2; if (runs[2 * m + 1] <= pos0) a_i = m + 1; else b_i = m; }
@@ -984,32 +997,23 @@ extern "C" int crf_seq_load_2bit(crf_ctx *c, const uint8_t *dna, const uint64_t 
         set_err("out of host memory");
         return CRF_ERR_NOMEM;
     }
-    LoadSource src;
-    src.twobit = dna;
     src.nm_runs = moved.data(); src.n_runs = moved.size() / 2; src.runs_mode = true;
     return load_checked(c, src, starts.data(), lengths.data(), nullptr, nullptr, n_records, max_motif_cap, dna_on_device, out, who);
 }
 
-// BAM reads: record r = offsets[r + 1] - offsets[r] bases coded from byte rec_byte[r] of nib, its exotic codes among the
-// list in offsets' position space.  The load sees record r at source position 2 rec_byte[r] and the exotic list moved there.
+// BAM reads (code_records), their exotic codes among the list in offsets' position space: the load sees the list moved to
+// the records' source positions.
 extern "C" int crf_seq_load_nibbles(crf_ctx *c, const uint8_t *nib, const uint64_t *rec_byte, const uint64_t *offsets,
                                     uint32_t n_records, const uint64_t *exotic, uint64_t n_exotic, uint32_t max_motif_cap,
                                     int nib_on_device, crf_seq **out) {
     const char *who = "crf_seq_load_nibbles";
-    CHECK(check_offsets(offsets, n_records, who));
-    if (!nib || !rec_byte || (n_exotic && !exotic)) { set_err("%s: null argument", who); return CRF_ERR_ARG; }
-    for (uint32_t r = 0; r < n_records; ++r)
-        if (offsets[r + 1] < offsets[r]) { set_err("%s: offsets must be non-decreasing", who); return CRF_ERR_ARG; }
+    LoadSource src;
+    src.codes = nib; src.code_bits = 4;
+    std::vector<uint64_t> starts, lengths, moved;
+    CHECK(code_records(src, rec_byte, offsets, n_records, n_exotic && !exotic, who, starts, lengths));
     for (uint64_t i = 1; i < n_exotic; ++i)
         if (exotic[i] >> 8 <= exotic[i - 1] >> 8) { set_err("%s: the exotic list must be ascending (entry %llu)", who, (unsigned long long)i); return CRF_ERR_ARG; }
-    std::vector<uint64_t> starts, lengths, moved;
     try {
-        starts.resize(n_records);
-        lengths.resize(n_records);
-        for (uint32_t r = 0; r < n_records; ++r) {
-            starts[r] = 2 * rec_byte[r];
-            lengths[r] = offsets[r + 1] - offsets[r];
-        }
         const uint64_t pos0 = offsets[0], pos1 = offsets[n_records];
         const uint64_t *e0 = std::lower_bound(exotic, exotic + n_exotic, pos0 << 8), *e1 = std::lower_bound(e0, exotic + n_exotic, pos1 << 8);
         bool sorted = true;
@@ -1026,8 +1030,6 @@ extern "C" int crf_seq_load_nibbles(crf_ctx *c, const uint8_t *nib, const uint64
         set_err("out of host memory");
         return CRF_ERR_NOMEM;
     }
-    LoadSource src;
-    src.nibbles = nib;
     src.exotic = moved.data(); src.n_exotic = moved.size();
     return load_checked(c, src, starts.data(), lengths.data(), nullptr, nullptr, n_records, max_motif_cap, nib_on_device, out, who);
 }

@@ -13,47 +13,99 @@
 #include <unistd.h>
 #include <zlib.h>
 
+#include "crf_codes.h"
 #include "crf_inflate.h"
 
 #include <atomic>
 #include <exception>
 #include <chrono>
 #include <functional>
+#include <memory>
 #include <mutex>
 #include <thread>
+
+enum HostKind { HOST_NONE, HOST_PINNED, HOST_HEAP, HOST_MAPPED };
+
+// Gives a HostBuf's block back (a static function, so the destructor stays a one-line inline call and the library exports
+// nothing new).
+static void host_release(uint8_t *p, size_t size, HostKind kind) {
+    if (kind == HOST_PINNED) cudaFreeHost(p);
+    else if (kind == HOST_HEAP) free(p);
+    else munmap(p, size);
+}
+
+// One block of host memory, given back the way it was obtained: page-locked (cudaHostAlloc), heap (malloc) or a mapping
+// (munmap).  It uses nothing else from the CUDA runtime, so the reader builds without it (tests/fuzz_*.cpp stub these).
+struct HostBuf {
+    uint8_t *p = nullptr;
+    size_t size = 0;
+    HostKind kind = HOST_NONE;
+
+    HostBuf() = default;
+    HostBuf(const HostBuf &) = delete;
+    HostBuf &operator=(const HostBuf &) = delete;
+    HostBuf(HostBuf &&o) noexcept { *this = std::move(o); }
+    HostBuf &operator=(HostBuf &&o) noexcept {           // (what this held goes with o)
+        std::swap(p, o.p);
+        std::swap(size, o.size);
+        std::swap(kind, o.kind);
+        return *this;
+    }
+    ~HostBuf() { if (p) host_release(p, size, kind); }
+    bool pinned() const { return kind == HOST_PINNED; }
+
+    // n >= 1 bytes, page-locked; false (nothing held) when there is no device or no page-locked memory left.
+    bool pin(size_t n) {
+        void *q = nullptr;
+        if (cudaHostAlloc(&q, n, cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return false; }
+        p = (uint8_t *)q; size = n; kind = HOST_PINNED;
+        return true;
+    }
+    // n >= 1 bytes, page-locked if asked and possible, else plain pages (2 MB ones when large).  false: out of memory.
+    bool alloc(size_t n, bool page_locked) {
+        if (page_locked && pin(n)) return true;
+        if (!(p = (uint8_t *)malloc(n))) return false;
+        size = n; kind = HOST_HEAP;
+#if defined(__linux__) && defined(MADV_HUGEPAGE)
+        if (n >= ((size_t)8 << 20)) {                    // gigabytes touched for the first time by their writer: 2 MB pages
+            const uintptr_t lo = ((uintptr_t)p + 4095) & ~(uintptr_t)4095, hi = ((uintptr_t)p + n) & ~(uintptr_t)4095;
+            if (hi > lo) madvise((void *)lo, hi - lo, MADV_HUGEPAGE);   // (advice only; the block is never realloc'ed)
+        }
+#endif
+        return true;
+    }
+    // Takes over the mapping [m, m + n).
+    void adopt(void *m, size_t n) { p = (uint8_t *)m; size = n; kind = HOST_MAPPED; }
+};
+
+// What crf_fasta_format returns.
+enum FastaFormat { FORMAT_FASTA = 0, FORMAT_FASTQ = 1, FORMAT_2BIT = 2, FORMAT_BAM = 3 };
 
 struct crf_fasta {
     std::vector<uint64_t> offsets;      // n_records + 1
     std::vector<uint64_t> name_off;     // into names (NUL-separated, record order: what crf_write_rows takes)
     std::vector<char> names;
-    uint8_t *bases = nullptr;
+    // The text (total bytes) and a FASTQ / BAM file's qualities laid out like it (kept with crf_fasta_open(pinned & 4)).
+    // bases and quals are their addresses as plain pointers: always the buffers' own, whatever the buffers are reassigned.
+    HostBuf bases_buf, quals_buf;
+    uint8_t *&bases = bases_buf.p;
+    uint8_t *&quals = quals_buf.p;
     uint64_t total = 0;
-    bool pinned = false;
     // packed planes (crf_fasta_packed): H, L, NM of plane_words words each, one allocation
-    uint32_t *planes = nullptr;
+    HostBuf planes;
     uint64_t plane_words = 0;
-    bool planes_pinned = false;
-    bool want_pinned_planes = false;                     // crf_fasta_open(pinned & 3): page-lock the planes crf_fasta_packed makes
     std::vector<uint64_t> exotic;
-    int format = 0;                                      // 0 = FASTA, 1 = FASTQ, 2 = .2bit, 3 = BAM
-    uint8_t *quals = nullptr;                            // FASTQ / BAM, crf_fasta_open(pinned & 4): laid out like bases
-    // .2bit: the file's bytes as they are (mapped, or page-locked with pinned & 3), where each record's packed bases
-    // start, its N blocks and mask blocks as sorted disjoint runs of concatenated positions; the text (bases) is decoded
-    // on the first crf_fasta_data
-    const uint8_t *dna = nullptr;
-    uint64_t dna_size = 0;
-    void *dna_map = nullptr;
-    bool dna_pinned = false;
-    std::vector<uint64_t> rec_byte, n_runs, mask_runs;
-    // BAM: the reads' 4-bit codes (=ACMGRSVTWYHKDBN, high nibble first), record r from byte rec_byte[r] with reverse
-    // complements applied; page-locked with pinned & 3, else an anonymous mapping of nib_map bytes.  nib_exotic: codes other
-    // than A, C, G, T, N as (position in the offsets' space << 8 | letter), ascending.  quals_map: the qualities' mapping size.
-    uint8_t *nib = nullptr;
-    uint64_t nib_bytes = 0, nib_map = 0, quals_map = 0;
-    bool nib_pinned = false;
-    std::vector<uint64_t> nib_exotic;
+    FastaFormat format = FORMAT_FASTA;
+    // .2bit and BAM: the bases as codes (crf_codes.h), record r's from byte rec_byte[r]; page-locked with pinned & 3.  The text
+    // (bases) is decoded on the first crf_fasta_data.
+    //   .2bit: the file's bytes as they are (else mapped); n_runs, mask_runs: its N blocks and mask blocks as sorted
+    //   disjoint runs of concatenated positions.
+    //   BAM: the reads' 4-bit codes with reverse complements applied (else an anonymous mapping); nib_exotic: codes other
+    //   than A, C, G, T, N as (position in the offsets' space << 8 | letter), ascending.
+    HostBuf codes;
+    std::vector<uint64_t> rec_byte, n_runs, mask_runs, nib_exotic;
     std::mutex decode_mu;
-    int text_pinned = 0;                                 // the pinned argument of crf_fasta_open, for the decoded text
+    int pinned = 0;                                      // the pinned argument of crf_fasta_open
     uint32_t n_threads = 1;
 };
 
@@ -286,27 +338,22 @@ static uint64_t name_token(const uint8_t *t, uint64_t *a, uint64_t h1) {
     return b;
 }
 
-// The base buffer: page-locked with pinned & 1 when a device is present, else plain pages (2 MB ones when large).
+// The text buffer of total bases: page-locked with pinned & 1 when a device is present, else plain pages.
 static bool alloc_bases(crf_fasta *fa, uint64_t total, int pinned) {
-    const size_t alloc = std::max<uint64_t>(total, 1);
-    fa->want_pinned_planes = (pinned & 3) != 0;
-    if (pinned & 1) {
-        void *p = nullptr;
-        if (cudaHostAlloc(&p, alloc, cudaHostAllocDefault) == cudaSuccess) {
-            fa->bases = (uint8_t *)p;
-            fa->pinned = true;
-        } else {
-            cudaGetLastError();                         // no device / no pinned memory left: plain pages
-        }
-    }
-    if (!fa->bases) fa->bases = (uint8_t *)malloc(alloc);
-    if (!fa->bases) return false;
-#if defined(__linux__) && defined(MADV_HUGEPAGE)
-    if (!fa->pinned && alloc >= ((size_t)8 << 20)) {    // gigabytes touched for the first time by the compaction below: 2 MB pages
-        const uintptr_t lo = ((uintptr_t)fa->bases + 4095) & ~(uintptr_t)4095, hi = ((uintptr_t)fa->bases + alloc) & ~(uintptr_t)4095;
-        if (hi > lo) madvise((void *)lo, hi - lo, MADV_HUGEPAGE);              // (advice only; the block is never realloc'ed)
-    }
-#endif
+    return fa->bases_buf.alloc(std::max<uint64_t>(total, 1), pinned & 1);
+}
+
+// src[0, n) into dst, page-locked, copied 64 MiB at a time on the reader's threads; false (dst untouched) when there is no
+// page-locked memory to be had.  give_back: each piece's source pages go back to the system once copied (src is an anonymous
+// mapping nothing reads again), so the bytes are held twice only a piece at a time.
+static bool copy_page_locked(HostBuf &dst, const uint8_t *src, uint64_t n, unsigned n_threads, bool give_back) {
+    if (!dst.pin(std::max<uint64_t>(n, 1))) return false;
+    const uint64_t PIECE = 64u << 20;
+    run_parallel(n_threads, (n + PIECE - 1) / PIECE, [&](size_t i) {
+        const uint64_t a = i * PIECE, z = std::min(PIECE, n - a);
+        memcpy(dst.p + a, src + a, z);
+        if (give_back) madvise(const_cast<uint8_t *>(src) + a, z & ~(uint64_t)4095, MADV_DONTNEED);
+    });
     return true;
 }
 
@@ -427,7 +474,7 @@ static uint64_t fastq_serial(const uint8_t *t, uint64_t n, uint64_t p, Sink &sin
 // *serial: whether the serial parser made the result.
 static int parse_fastq(const char *path, const uint8_t *t, uint64_t n, uint64_t lead, unsigned n_threads, uint64_t piece,
                        int pinned, crf_fasta *fa, bool *serial) {
-    fa->format = 1;
+    fa->format = FORMAT_FASTQ;
     const uint64_t n_pieces = (n - lead + piece - 1) / piece;
     struct Part { uint64_t begin, end; FastqCount count; bool ok; };
     std::vector<Part> parts(n_pieces);
@@ -485,7 +532,7 @@ static int parse_fastq(const char *path, const uint8_t *t, uint64_t n, uint64_t 
     fa->name_off.assign(total.records, 0);
     fa->names.assign(total.name_bytes, 0);
     fa->offsets[total.records] = fa->total = total.bases;
-    if (!alloc_bases(fa, total.bases, pinned) || ((pinned & 4) && !(fa->quals = (uint8_t *)malloc(std::max<uint64_t>(total.bases, 1))))) {
+    if (!alloc_bases(fa, total.bases, pinned) || ((pinned & 4) && !fa->quals_buf.alloc(std::max<uint64_t>(total.bases, 1), false))) {
         set_err("crf_fasta_open: out of host memory (%llu bases)", (unsigned long long)total.bases);
         return CRF_ERR_NOMEM;
     }
@@ -544,7 +591,7 @@ static void merge_blocks(std::vector<std::pair<uint64_t, uint64_t>> &blk, uint64
 // Index, record headers and blocks of the .2bit file t[0, n) into fa, every count, offset and block checked against the
 // file size and dnaSize.  The bases are not touched.
 static int parse_twobit(const char *path, const uint8_t *t, uint64_t n, crf_fasta *fa) {
-    fa->format = 2;
+    fa->format = FORMAT_2BIT;
     uint32_t sig;
     memcpy(&sig, t, 4);
     const bool swap = sig != TWOBIT_SIG;
@@ -623,59 +670,6 @@ static int parse_twobit(const char *path, const uint8_t *t, uint64_t n, crf_fast
     return CRF_OK;
 }
 
-// The text of a .2bit handle, what twoBitToFa writes: T/C/A/G, N blocks as 'N', mask blocks lower-cased ('n' inside
-// both).  Decoded once, on the reader's threads, in pieces of concatenated positions.
-static int twobit_decode(crf_fasta *fa) {
-    std::lock_guard<std::mutex> lock(fa->decode_mu);
-    if (fa->bases || fa->format != 2) return CRF_OK;
-    static const struct Lut {                                     // a byte -> its four letters
-        uint32_t v[256];
-        Lut() {
-            for (uint32_t b = 0; b < 256; ++b) {
-                uint8_t c[4];
-                for (int j = 0; j < 4; ++j) c[j] = (uint8_t)"TCAG"[(b >> (6 - 2 * j)) & 3];
-                memcpy(&v[b], c, 4);
-            }
-        }
-    } lut;
-    try {
-        if (!alloc_bases(fa, fa->total, fa->text_pinned)) {
-            set_err("crf_fasta_data: out of host memory (%llu bases)", (unsigned long long)fa->total);
-            return CRF_ERR_NOMEM;
-        }
-        const uint64_t PIECE = 4u << 20, total = fa->total;
-        const std::vector<uint64_t> &off = fa->offsets, &nr = fa->n_runs, &mr = fa->mask_runs;
-        uint8_t *out = fa->bases;
-        run_parallel(fa->n_threads, (total + PIECE - 1) / PIECE, [&](size_t i) {
-            const uint64_t lo = i * PIECE, hi = std::min(total, lo + PIECE);
-            uint64_t r = (uint64_t)(std::upper_bound(off.begin(), off.end(), lo) - off.begin()) - 1;
-            for (uint64_t pos = lo; pos < hi; ++r) {
-                if (off[r + 1] <= pos) continue;
-                const uint64_t i1 = std::min(hi, off[r + 1]) - off[r];
-                const uint8_t *d = fa->dna + fa->rec_byte[r];
-                uint8_t *o = out + off[r];
-                uint64_t j = pos - off[r];
-                for (; j < i1 && (j & 3); ++j) o[j] = (uint8_t)"TCAG"[(d[j >> 2] >> (6 - 2 * (j & 3))) & 3];
-                for (; j + 4 <= i1; j += 4) memcpy(o + j, &lut.v[d[j >> 2]], 4);
-                for (; j < i1; ++j) o[j] = (uint8_t)"TCAG"[(d[j >> 2] >> (6 - 2 * (j & 3))) & 3];
-                pos = off[r] + i1;
-            }
-            for (int kind = 0; kind < 2; ++kind) {                // mask blocks lower-case, then N blocks keep the case
-                const std::vector<uint64_t> &runs = kind ? nr : mr;
-                uint64_t a = 0, b = runs.size() / 2;              // first run that ends after lo
-                while (a < b) { const uint64_t m = (a + b) / 2; if (runs[2 * m + 1] <= lo) a = m + 1; else b = m; }
-                for (; a < runs.size() / 2 && runs[2 * a] < hi; ++a)
-                    for (uint64_t q = std::max(lo, runs[2 * a]), e = std::min(hi, runs[2 * a + 1]); q < e; ++q)
-                        out[q] = kind ? (uint8_t)((out[q] & 0x20) | 'N') : (uint8_t)(out[q] | 0x20);
-            }
-        });
-    } catch (const std::bad_alloc &) {
-        set_err("crf_fasta_data: out of host memory");
-        return CRF_ERR_NOMEM;
-    }
-    return CRF_OK;
-}
-
 // ---- BAM (unaligned reads) ----
 // A BGZF stream that starts with "BAM\1": l_text, the header text, n_ref and the reference list, then the records.  A
 // record is block_size and block_size bytes: refID, pos, l_read_name (u8), mapq, bin, n_cigar_op (u16), flag (u16), l_seq,
@@ -685,7 +679,6 @@ static int twobit_decode(crf_fasta *fa) {
 // the bases reverse-complemented when flag & 0x10 (the complement of a code is its 4-bit bit-reversal), qualities + 33 (or
 // '"' when absent), reversed with the bases.  The stream is inflated a window of blocks at a time; the bases stay codes.
 static const uint64_t BAM_WINDOW = 32u << 20;             // inflated bytes per window (CRF_BAM_WINDOW overrides it)
-static const char BAM_LETTERS[] = "=ACMGRSVTWYHKDBN";
 
 static bool is_bam_magic(const uint8_t *t, uint64_t n) { return n >= 4 && memcmp(t, "BAM\1", 4) == 0; }
 
@@ -703,7 +696,12 @@ struct GrowBuf {
         p = (uint8_t *)q;
         cap = nc;
     }
-    uint8_t *release() { uint8_t *q = p; p = nullptr; return q; }
+    HostBuf release() {                                    // the mapping goes to the caller
+        HostBuf b;
+        b.adopt(p, cap);
+        p = nullptr;
+        return b;
+    }
 };
 
 // The inflated stream, a window of blocks at a time: bytes [pos, end) of buf are inflated and not yet consumed.
@@ -803,7 +801,7 @@ static void bam_copy(const uint8_t *q, uint8_t *nib, uint64_t o, uint8_t *quals,
         if (!lut.exotic[b >> 4] && (i + 1 == n || !lut.exotic[b & 15])) continue;
         for (uint64_t k = i; k < std::min(n, i + 2); ++k) {
             const uint8_t c = k & 1 ? b & 15 : b >> 4;
-            if (lut.exotic[c]) ex.push_back(((base + k) << 8) | (uint8_t)BAM_LETTERS[c]);
+            if (lut.exotic[c]) ex.push_back(((base + k) << 8) | (uint8_t)PackedCodes<4>::LETTERS[c]);
         }
     }
     if (!quals) return;
@@ -816,7 +814,7 @@ static void bam_copy(const uint8_t *q, uint8_t *nib, uint64_t o, uint8_t *quals,
 // The BAM stream of the BGZF blocks into fa.  Every count and length is checked against the record and the stream.
 static int parse_bam(const char *path, const uint8_t *file, const std::vector<BgzfBlock> &blocks, uint64_t total,
                      unsigned n_threads, int pinned, crf_fasta *fa) {
-    fa->format = 3;
+    fa->format = FORMAT_BAM;
     const char *w = getenv("CRF_BAM_WINDOW");
     BamStream s{file, blocks, n_threads, 0, total, w ? std::max<uint64_t>(strtoull(w, nullptr, 10), 1) : BAM_WINDOW};
     auto corrupt = [&]() { set_err("crf_fasta_open: %s has a corrupt BGZF block", path); return CRF_ERR_ARG; };
@@ -903,50 +901,54 @@ static int parse_bam(const char *path, const uint8_t *file, const std::vector<Bg
     }
     fa->offsets.push_back(base_at);
     fa->total = base_at;
-    fa->nib_bytes = nib_at;
     nib.reserve(1);
-    void *pin = nullptr;                                     // pinned & 3: the codes that get uploaded, page-locked
-    if ((pinned & 3) && cudaHostAlloc(&pin, std::max<uint64_t>(nib_at, 1), cudaHostAllocDefault) == cudaSuccess) {
-        const uint64_t PIECE = 64u << 20;                    // copied a piece at a time, each piece's pages handed back
-        run_parallel(n_threads, (nib_at + PIECE - 1) / PIECE, [&](size_t i) {
-            const uint64_t a = i * PIECE, z = std::min(PIECE, nib_at - a);
-            memcpy((uint8_t *)pin + a, nib.p + a, z);
-            madvise(nib.p + a, z & ~(uint64_t)4095, MADV_DONTNEED);
-        });
-        fa->nib = (uint8_t *)pin;
-        fa->nib_pinned = true;
-    } else {
-        if (pinned & 3) cudaGetLastError();
-        fa->nib_map = nib.cap;
-        fa->nib = nib.release();
-    }
+    if (!((pinned & 3) && copy_page_locked(fa->codes, nib.p, nib_at, n_threads, true))) fa->codes = nib.release();
     if (want_quals) {
         quals.reserve(1);
-        fa->quals_map = quals.cap;
-        fa->quals = quals.release();
+        fa->quals_buf = quals.release();
     }
     return CRF_OK;
 }
 
-// The text of a BAM handle (what samtools fastq writes as bases), decoded once, on the reader's threads.
-static int bam_decode(crf_fasta *fa) {
+// Record r's letters from positions [lo, hi) of the concatenated text.
+template <int BITS>
+static void decode_records(crf_fasta *fa, uint64_t lo, uint64_t hi) {
+    const std::vector<uint64_t> &off = fa->offsets;
+    uint64_t r = (uint64_t)(std::upper_bound(off.begin(), off.end(), lo) - off.begin()) - 1;
+    for (uint64_t pos = lo; pos < hi; ++r) {
+        if (off[r + 1] <= pos) continue;
+        const uint64_t i1 = std::min(hi, off[r + 1]) - off[r];
+        code_letters<BITS>(fa->codes.p + fa->rec_byte[r], pos - off[r], i1, fa->bases + off[r]);
+        pos = off[r] + i1;
+    }
+}
+
+// The text of a .2bit or BAM handle, decoded on first use (nothing to do for the others), on the reader's threads in pieces
+// of concatenated positions.  A BAM file's is what samtools fastq writes as bases; a .2bit file's what twoBitToFa writes:
+// T/C/A/G, N blocks as 'N', mask blocks lower-cased ('n' inside both).
+static int decode_text(crf_fasta *fa) {
+    if (fa->format != FORMAT_2BIT && fa->format != FORMAT_BAM) return CRF_OK;
+    std::lock_guard<std::mutex> lock(fa->decode_mu);
+    if (fa->bases) return CRF_OK;
     try {
-        if (!alloc_bases(fa, fa->total, fa->text_pinned)) {
+        if (!alloc_bases(fa, fa->total, fa->pinned)) {
             set_err("crf_fasta_data: out of host memory (%llu bases)", (unsigned long long)fa->total);
             return CRF_ERR_NOMEM;
         }
         const uint64_t PIECE = 4u << 20, total = fa->total;
-        const std::vector<uint64_t> &off = fa->offsets;
+        const bool twobit = fa->format == FORMAT_2BIT;
+        uint8_t *out = fa->bases;
         run_parallel(fa->n_threads, (total + PIECE - 1) / PIECE, [&](size_t i) {
             const uint64_t lo = i * PIECE, hi = std::min(total, lo + PIECE);
-            uint64_t r = (uint64_t)(std::upper_bound(off.begin(), off.end(), lo) - off.begin()) - 1;
-            for (uint64_t pos = lo; pos < hi; ++r) {
-                if (off[r + 1] <= pos) continue;
-                const uint64_t i1 = std::min(hi, off[r + 1]) - off[r];
-                const uint8_t *d = fa->nib + fa->rec_byte[r];
-                uint8_t *o = fa->bases + off[r];
-                for (uint64_t j = pos - off[r]; j < i1; ++j) o[j] = (uint8_t)BAM_LETTERS[(d[j >> 1] >> (j & 1 ? 0 : 4)) & 15];
-                pos = off[r] + i1;
+            if (!twobit) { decode_records<4>(fa, lo, hi); return; }
+            decode_records<2>(fa, lo, hi);
+            for (int kind = 0; kind < 2; ++kind) {                // mask blocks lower-case, then N blocks keep the case
+                const std::vector<uint64_t> &runs = kind ? fa->n_runs : fa->mask_runs;
+                uint64_t a = 0, b = runs.size() / 2;              // first run that ends after lo
+                while (a < b) { const uint64_t m = (a + b) / 2; if (runs[2 * m + 1] <= lo) a = m + 1; else b = m; }
+                for (; a < runs.size() / 2 && runs[2 * a] < hi; ++a)
+                    for (uint64_t q = std::max(lo, runs[2 * a]), e = std::min(hi, runs[2 * a + 1]); q < e; ++q)
+                        out[q] = kind ? (uint8_t)((out[q] & 0x20) | 'N') : (uint8_t)(out[q] | 0x20);
             }
         });
     } catch (const std::bad_alloc &) {
@@ -956,155 +958,23 @@ static int bam_decode(crf_fasta *fa) {
     return CRF_OK;
 }
 
-// The text of a .2bit or BAM handle, decoded on first use; nothing to do for the others.
-static int decode_text(crf_fasta *fa) {
-    if (fa->format == 2) return twobit_decode(fa);
-    if (fa->format != 3) return CRF_OK;
-    std::lock_guard<std::mutex> lock(fa->decode_mu);
-    return fa->bases ? CRF_OK : bam_decode(fa);
-}
-
-}  // namespace fasta_detail
-
-static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf_fasta **out);
-extern "C" int crf_fasta_close(crf_fasta *fa);
-
-extern "C" int crf_fasta_open(const char *path, uint32_t n_threads, int pinned, crf_fasta **out) {
-    if (!path || !out) { set_err("crf_fasta_open: null argument"); return CRF_ERR_ARG; }
-    *out = nullptr;
-    try {                                               // no exception crosses the C boundary
-        return fasta_open_impl(path, n_threads, pinned, out);
-    } catch (const std::bad_alloc &) {
-        set_err("crf_fasta_open: out of host memory reading %s", path);
-        return CRF_ERR_NOMEM;
-    } catch (const std::exception &ex) {
-        set_err("crf_fasta_open: %s", ex.what());
-        return CRF_ERR_ARG;
-    }
-}
-
-static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf_fasta **out) {
-    using namespace fasta_detail;
-    const bool trace = getenv("CRF_FASTA_TRACE") != nullptr;
-    auto t0 = std::chrono::steady_clock::now();
-    auto lap = [&](const char *what) {
-        if (!trace) return;
-        auto t1 = std::chrono::steady_clock::now();
+// CRF_FASTA_TRACE=1: the stage times of crf_fasta_open on stderr.
+struct OpenTrace {
+    bool on = getenv("CRF_FASTA_TRACE") != nullptr;
+    std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
+    void lap(const char *what) {
+        if (!on) return;
+        const auto t1 = std::chrono::steady_clock::now();
         fprintf(stderr, "[crf_fasta] %-10s %8.1f ms\n", what, std::chrono::duration<double, std::milli>(t1 - t0).count());
         t0 = t1;
-    };
-    FileBytes file;
-    std::vector<uint8_t> plain;
-    crf_inflate::OutBuf inflated;
-    if (!open_bytes(path, file)) { set_err("crf_fasta_open: cannot read %s", path); return CRF_ERR_ARG; }
-    const uint8_t *t = file.data;
-    uint64_t n = file.size;
-    if (n_threads == 0) n_threads = std::min(16u, std::max(1u, std::thread::hardware_concurrency()));
-    if (is_twobit(t, n)) {                              // (the raw file: a .2bit file is never compressed)
-        struct Guard {
-            crf_fasta *p;
-            ~Guard() { if (p) crf_fasta_close(p); }
-        } guard{new crf_fasta};
-        crf_fasta *fa = guard.p;
-        fa->n_threads = n_threads;
-        fa->text_pinned = pinned;
-        const int rc = parse_twobit(path, t, n, fa);
-        if (rc != CRF_OK) return rc;
-        lap("2bit-index");
-        void *p = nullptr;                              // pinned & 3: the bytes that get uploaded, page-locked
-        if ((pinned & 3) && cudaHostAlloc(&p, n, cudaHostAllocDefault) == cudaSuccess) {
-            const uint64_t PIECE = 64u << 20;
-            run_parallel(n_threads, (n + PIECE - 1) / PIECE, [&](size_t i) {
-                memcpy((uint8_t *)p + i * PIECE, t + i * PIECE, std::min(PIECE, n - i * PIECE));
-            });
-            fa->dna = (const uint8_t *)p;
-            fa->dna_pinned = true;
-            lap("2bit-pin");
-        } else {
-            if (pinned & 3) cudaGetLastError();
-            if (file.map) {                             // the mapping goes to the handle
-                fa->dna_map = file.map;
-                file.map = nullptr;
-                fa->dna = t;
-            } else {
-                uint8_t *own = (uint8_t *)malloc(std::max<uint64_t>(n, 1));
-                if (!own) throw std::bad_alloc();
-                memcpy(own, t, n);
-                fa->dna = own;
-            }
-        }
-        fa->dna_size = n;
-        guard.p = nullptr;
-        *out = fa;
-        return CRF_OK;
     }
-    if (n >= 2 && t[0] == 0x1f && t[1] == 0x8b) {
-        bool bad = false;
-        std::vector<BgzfBlock> blocks;
-        uint64_t total = 0;
-        const bool bgzf = bgzf_index(file, blocks, &total);
-        if (bgzf) {                                     // a BAM file: its first inflated bytes are "BAM\1"
-            std::vector<uint8_t> head;                  // (the first 4 inflated bytes, from as many blocks as they span)
-            BgzfInflater inf(t);
-            bool head_ok = true;
-            for (size_t b = 0; b < blocks.size() && head.size() < 4 && head_ok; ++b) {
-                const size_t at = head.size();
-                head.resize(at + blocks[b].isize);
-                head_ok = inf.run(blocks[b], head.data() + at);
-            }
-            if (head_ok && is_bam_magic(head.data(), head.size())) {
-                struct Guard {
-                    crf_fasta *p;
-                    ~Guard() { if (p) crf_fasta_close(p); }
-                } guard{new crf_fasta};
-                crf_fasta *fa = guard.p;
-                fa->n_threads = n_threads;
-                fa->text_pinned = pinned;
-                const int rc = parse_bam(path, t, blocks, total, n_threads, pinned, fa);
-                if (rc != CRF_OK) return rc;
-                lap("bam");
-                guard.p = nullptr;
-                *out = fa;
-                return CRF_OK;
-            }
-            if (!inflated.reserve(total + 64)) throw std::bad_alloc();
-            inflated.size = total;
-            bad = !inflate_blocks(t, blocks, 0, blocks.size(), n_threads, inflated.p);
-        }
-        if (bgzf && bad) { set_err("crf_fasta_open: %s has a corrupt BGZF block", path); return CRF_ERR_ARG; }
-        // a plain gzip stream: the reader's own decoder (crf_inflate.h); whatever it does not take goes to zlib, which decides
-        const bool own = !bgzf && getenv("CRF_GUNZIP_ZLIB") == nullptr && crf_inflate::gunzip(file.data, file.size, inflated, n_threads);
-        if (!bgzf && !own && !inflate_all(file, plain)) { set_err("crf_fasta_open: %s is not a valid gzip stream", path); return CRF_ERR_ARG; }
-        t = bgzf || own ? inflated.p : plain.data();
-        n = bgzf || own ? inflated.size : plain.size();
-        if (is_bam_magic(t, n)) {
-            set_err("crf_fasta_open: %s is a BAM file compressed as plain gzip, not BGZF: BAM input must be BGZF "
-                    "(as samtools writes it)", path);
-            return CRF_ERR_ARG;
-        }
-        lap(bgzf ? "bgzf" : own ? "gunzip" : "gzip/zlib");
-    }
-    lap("read");
+};
 
-    struct Guard {                                      // frees the handle unless it is handed to the caller
-        crf_fasta *p;
-        ~Guard() { if (p) crf_fasta_close(p); }
-    } guard{new crf_fasta};
-    crf_fasta *fa = guard.p;
-
+// ---- FASTA ----
+// A record is a '>' at the start of a line, its header line (the name: its first whitespace-delimited token), then the
+// body lines up to the next record, joined without their line ends.
+static int parse_fasta(const uint8_t *t, uint64_t n, unsigned n_threads, int pinned, crf_fasta *fa, OpenTrace &trace) {
     const uint64_t PIECE = 8u << 20;
-    uint64_t lead = 0;                                  // a FASTQ file: '@' is its first byte that is not whitespace
-    while (lead < n && is_space(t[lead])) ++lead;
-    if (lead < n && t[lead] == '@') {
-        bool serial = false;
-        const int rc = parse_fastq(path, t, n, lead, n_threads, PIECE, pinned, fa, &serial);
-        if (rc != CRF_OK) return rc;
-        lap(serial ? "fastq-serial" : "fastq");
-        guard.p = nullptr;
-        *out = fa;
-        return CRF_OK;
-    }
-
     // headers: a '>' at the start of a line
     std::vector<std::vector<uint64_t>> hdr_in((n + PIECE - 1) / PIECE);
     run_parallel(n_threads, hdr_in.size(), [&](size_t i) {
@@ -1134,7 +1004,7 @@ static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf
         fa->names.push_back('\0');
     }
 
-    lap("headers");
+    trace.lap("headers");
     // bodies in pieces of <= 8 MiB of text: count line ends, prefix-sum, compact
     std::vector<Piece> pieces;
     std::vector<uint64_t> first_piece(n_rec + 1);
@@ -1149,7 +1019,7 @@ static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf
         for (uint64_t p = pc.begin; p < pc.end; ++p) c += (t[p] == '\n') | (t[p] == '\r');
         pc.n_eol = c;
     });
-    lap("count");
+    trace.lap("count");
     fa->offsets.assign(n_rec + 1, 0);
     uint64_t total = 0;
     for (uint64_t r = 0; r < n_rec; ++r) {
@@ -1164,7 +1034,7 @@ static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf
 
     if (!alloc_bases(fa, total, pinned)) { set_err("crf_fasta_open: out of host memory (%llu bases)", (unsigned long long)total); return CRF_ERR_NOMEM; }
 
-    lap("alloc");
+    trace.lap("alloc");
     uint8_t *dst = fa->bases;
     run_parallel(n_threads, pieces.size(), [&](size_t i) {
         const Piece &pc = pieces[i];
@@ -1191,9 +1061,113 @@ static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf
             if (c != '\n' && c != '\r') *o++ = c;
         }
     });
-    lap("compact");
-    guard.p = nullptr;
-    *out = fa;
+    trace.lap("compact");
+    return CRF_OK;
+}
+
+// Whether a BGZF file is BAM: its first inflated bytes are "BAM\1" (read from as many blocks as they span).
+static bool bgzf_is_bam(const uint8_t *file, const std::vector<BgzfBlock> &blocks) {
+    std::vector<uint8_t> head;
+    BgzfInflater inf(file);
+    bool head_ok = true;
+    for (size_t b = 0; b < blocks.size() && head.size() < 4 && head_ok; ++b) {
+        const size_t at = head.size();
+        head.resize(at + blocks[b].isize);
+        head_ok = inf.run(blocks[b], head.data() + at);
+    }
+    return head_ok && is_bam_magic(head.data(), head.size());
+}
+
+}  // namespace fasta_detail
+
+static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf_fasta **out);
+extern "C" int crf_fasta_close(crf_fasta *fa);
+
+extern "C" int crf_fasta_open(const char *path, uint32_t n_threads, int pinned, crf_fasta **out) {
+    if (!path || !out) { set_err("crf_fasta_open: null argument"); return CRF_ERR_ARG; }
+    *out = nullptr;
+    try {                                               // no exception crosses the C boundary
+        return fasta_open_impl(path, n_threads, pinned, out);
+    } catch (const std::bad_alloc &) {
+        set_err("crf_fasta_open: out of host memory reading %s", path);
+        return CRF_ERR_NOMEM;
+    } catch (const std::exception &ex) {
+        set_err("crf_fasta_open: %s", ex.what());
+        return CRF_ERR_ARG;
+    }
+}
+
+static int fasta_open_impl(const char *path, uint32_t n_threads, int pinned, crf_fasta **out) {
+    using namespace fasta_detail;
+    OpenTrace trace;
+    FileBytes file;
+    std::vector<uint8_t> plain;
+    crf_inflate::OutBuf inflated;
+    if (!open_bytes(path, file)) { set_err("crf_fasta_open: cannot read %s", path); return CRF_ERR_ARG; }
+    const uint8_t *t = file.data;
+    uint64_t n = file.size;
+    if (n_threads == 0) n_threads = std::min(16u, std::max(1u, std::thread::hardware_concurrency()));
+    std::unique_ptr<crf_fasta, int (*)(crf_fasta *)> fa(new crf_fasta, crf_fasta_close);   // unless handed to the caller
+    fa->n_threads = n_threads;
+    fa->pinned = pinned;
+    const bool gz = n >= 2 && t[0] == 0x1f && t[1] == 0x8b;
+    std::vector<BgzfBlock> blocks;
+    uint64_t total = 0;
+    const bool bgzf = gz && bgzf_index(file, blocks, &total);
+    int rc;
+    if (is_twobit(t, n)) {                              // (the raw file: a .2bit file is never compressed)
+        rc = parse_twobit(path, t, n, fa.get());
+        if (rc != CRF_OK) return rc;
+        trace.lap("2bit-index");
+        if ((pinned & 3) && copy_page_locked(fa->codes, t, n, n_threads, false)) {   // the bytes that get uploaded, page-locked
+            trace.lap("2bit-pin");
+        } else if (file.map) {                          // the mapping goes to the handle
+            fa->codes.adopt(file.map, n);
+            file.map = nullptr;
+        } else {
+            if (!fa->codes.alloc(std::max<uint64_t>(n, 1), false)) throw std::bad_alloc();
+            memcpy(fa->codes.p, t, n);
+        }
+    } else if (bgzf && bgzf_is_bam(t, blocks)) {        // inflated a window at a time by parse_bam
+        rc = parse_bam(path, t, blocks, total, n_threads, pinned, fa.get());
+        if (rc != CRF_OK) return rc;
+        trace.lap("bam");
+    } else {
+        if (gz) {
+            if (bgzf) {
+                if (!inflated.reserve(total + 64)) throw std::bad_alloc();
+                inflated.size = total;
+                if (!inflate_blocks(t, blocks, 0, blocks.size(), n_threads, inflated.p)) {
+                    set_err("crf_fasta_open: %s has a corrupt BGZF block", path);
+                    return CRF_ERR_ARG;
+                }
+            }
+            // a plain gzip stream: the reader's own decoder (crf_inflate.h); whatever it does not take goes to zlib, which decides
+            const bool own = !bgzf && getenv("CRF_GUNZIP_ZLIB") == nullptr && crf_inflate::gunzip(file.data, file.size, inflated, n_threads);
+            if (!bgzf && !own && !inflate_all(file, plain)) { set_err("crf_fasta_open: %s is not a valid gzip stream", path); return CRF_ERR_ARG; }
+            t = bgzf || own ? inflated.p : plain.data();
+            n = bgzf || own ? inflated.size : plain.size();
+            if (is_bam_magic(t, n)) {
+                set_err("crf_fasta_open: %s is a BAM file compressed as plain gzip, not BGZF: BAM input must be BGZF "
+                        "(as samtools writes it)", path);
+                return CRF_ERR_ARG;
+            }
+            trace.lap(bgzf ? "bgzf" : own ? "gunzip" : "gzip/zlib");
+        }
+        trace.lap("read");
+        uint64_t lead = 0;                              // a FASTQ file: '@' is its first byte that is not whitespace
+        while (lead < n && is_space(t[lead])) ++lead;
+        if (lead < n && t[lead] == '@') {
+            bool serial = false;
+            rc = parse_fastq(path, t, n, lead, n_threads, 8u << 20, pinned, fa.get(), &serial);
+            if (rc != CRF_OK) return rc;
+            trace.lap(serial ? "fastq-serial" : "fastq");
+        } else {
+            rc = parse_fasta(t, n, n_threads, pinned, fa.get(), trace);
+            if (rc != CRF_OK) return rc;
+        }
+    }
+    *out = fa.release();
     return CRF_OK;
 }
 
@@ -1233,7 +1207,7 @@ extern "C" int crf_fasta_info(const crf_fasta *fa, uint64_t *n_records, uint64_t
     if (!fa) { set_err("null fasta handle"); return CRF_ERR_ARG; }
     if (n_records) *n_records = fa->offsets.size() - 1;
     if (total_bases) *total_bases = fa->total;
-    if (pinned) *pinned = fa->pinned ? 1 : 0;
+    if (pinned) *pinned = fa->bases_buf.pinned() ? 1 : 0;
     return CRF_OK;
 }
 
@@ -1262,8 +1236,8 @@ extern "C" int crf_fasta_index(const crf_fasta *fa, const uint64_t **offsets, co
 extern "C" int crf_fasta_twobit(const crf_fasta *fa, const uint8_t **dna, const uint64_t **rec_byte, const uint64_t **runs,
                                 uint64_t *n_runs) {
     if (!fa || !dna || !rec_byte || !runs || !n_runs) { set_err("crf_fasta_twobit: null argument"); return CRF_ERR_ARG; }
-    if (fa->format != 2) { set_err("crf_fasta_twobit: not a .2bit file"); return CRF_ERR_ARG; }
-    *dna = fa->dna;
+    if (fa->format != FORMAT_2BIT) { set_err("crf_fasta_twobit: not a .2bit file"); return CRF_ERR_ARG; }
+    *dna = fa->codes.p;
     *rec_byte = fa->rec_byte.data();
     *runs = fa->n_runs.data();
     *n_runs = fa->n_runs.size() / 2;
@@ -1273,8 +1247,8 @@ extern "C" int crf_fasta_twobit(const crf_fasta *fa, const uint8_t **dna, const 
 extern "C" int crf_fasta_nibbles(const crf_fasta *fa, const uint8_t **nib, const uint64_t **rec_byte, const uint64_t **exotic,
                                  uint64_t *n_exotic) {
     if (!fa || !nib || !rec_byte || !exotic || !n_exotic) { set_err("crf_fasta_nibbles: null argument"); return CRF_ERR_ARG; }
-    if (fa->format != 3) { set_err("crf_fasta_nibbles: not a BAM file"); return CRF_ERR_ARG; }
-    *nib = fa->nib;
+    if (fa->format != FORMAT_BAM) { set_err("crf_fasta_nibbles: not a BAM file"); return CRF_ERR_ARG; }
+    *nib = fa->codes.p;
     *rec_byte = fa->rec_byte.data();
     *exotic = fa->nib_exotic.data();
     *n_exotic = fa->nib_exotic.size();
@@ -1294,18 +1268,6 @@ extern "C" int crf_fasta_quals(const crf_fasta *fa, const uint8_t **quals) {
 }
 
 extern "C" int crf_fasta_close(crf_fasta *fa) {
-    if (!fa) return CRF_OK;
-    if (fa->pinned) cudaFreeHost(fa->bases);
-    else free(fa->bases);
-    if (fa->quals_map) munmap(fa->quals, fa->quals_map);
-    else free(fa->quals);
-    if (fa->nib_pinned) cudaFreeHost(fa->nib);
-    else if (fa->nib_map) munmap(fa->nib, fa->nib_map);
-    if (fa->dna_pinned) cudaFreeHost((void *)fa->dna);
-    else if (fa->dna_map) munmap(fa->dna_map, fa->dna_size);
-    else free((void *)fa->dna);
-    if (fa->planes_pinned) cudaFreeHost(fa->planes);
-    else free(fa->planes);
     delete fa;
     return CRF_OK;
 }

@@ -175,26 +175,22 @@ extern "C" int crf_fasta_packed(crf_fasta *fa, uint32_t n_threads, const uint32_
     if (!fa || !H || !L || !NM || !exotic || !n_exotic) { set_err("crf_fasta_packed: null argument"); return CRF_ERR_ARG; }
     if (n_threads == 0) n_threads = std::min(16u, std::max(1u, std::thread::hardware_concurrency()));
     try {
-        if (!fa->planes) {
+        if (!fa->planes.p) {
             const int rc = fasta_detail::decode_text(fa);   // (a .2bit or BAM file: its text, decoded on first use)
             if (rc != CRF_OK) return rc;
             const uint64_t n_words = (fa->total + 31) / 32 + 1;
-            const size_t bytes = (size_t)n_words * 12;
-            void *p = nullptr;
-            if (fa->want_pinned_planes && cudaHostAlloc(&p, bytes, cudaHostAllocDefault) == cudaSuccess) fa->planes_pinned = true;
-            else { cudaGetLastError(); p = malloc(bytes); }
-            if (!p) { set_err("crf_fasta_packed: out of host memory"); return CRF_ERR_NOMEM; }
-            fa->planes = (uint32_t *)p;
+            if (!fa->planes.alloc((size_t)n_words * 12, fa->pinned & 3)) { set_err("crf_fasta_packed: out of host memory"); return CRF_ERR_NOMEM; }
+            uint32_t *planes = (uint32_t *)fa->planes.p;
             fa->plane_words = n_words;
-            pack_detail::pack_all(fa->bases, fa->total, n_threads, fa->planes, fa->planes + n_words, fa->planes + 2 * n_words,
-                                  fa->exotic);
-            fa->planes[n_words - 1] = 0; fa->planes[2 * n_words - 1] = 0; fa->planes[3 * n_words - 1] = 0xFFFFFFFFu;
+            pack_detail::pack_all(fa->bases, fa->total, n_threads, planes, planes + n_words, planes + 2 * n_words, fa->exotic);
+            planes[n_words - 1] = 0; planes[2 * n_words - 1] = 0; planes[3 * n_words - 1] = 0xFFFFFFFFu;
         }
     } catch (const std::bad_alloc &) {
         set_err("crf_fasta_packed: out of host memory");
         return CRF_ERR_NOMEM;
     }
-    *H = fa->planes; *L = fa->planes + fa->plane_words; *NM = fa->planes + 2 * fa->plane_words;
+    const uint32_t *planes = (const uint32_t *)fa->planes.p;
+    *H = planes; *L = planes + fa->plane_words; *NM = planes + 2 * fa->plane_words;
     *exotic = fa->exotic.data();
     *n_exotic = fa->exotic.size();
     return CRF_OK;

@@ -1,6 +1,6 @@
 // Native BED / TSV row writer (host only): result rows -> text, replacing the per-row Python of
 // perfect_repeat_finder.py:148-149 (BED: chrom, start, end, motif) and :166-170 (TSV with header).  Rows are formatted on
-// several threads, the motif column read back from the host copy of the text (or from a .2bit file's packed bases).
+// several threads, the motif column read back from the host copy of the text (or from a .2bit or BAM file's codes).
 //
 // Included at the end of crf_api.cu (shares set_err()); tests/fuzz_reader.cpp compiles it without the CUDA runtime.
 #pragma once
@@ -14,6 +14,8 @@
 #include <system_error>
 #include <thread>
 #include <vector>
+
+#include "crf_codes.h"
 
 static inline char *put_u64(char *p, uint64_t v) {
     char tmp[20];
@@ -38,26 +40,15 @@ struct TextMotif {
     }
 };
 
-// ... or a .2bit file's packed bases (record r's base i: bits 7-6 of byte rec_byte[r] + i / 4 for i % 4 == 0, then 5-4, ...;
-// T=0 C=1 A=2 G=3).  A motif never holds an N, so the codes alone give the letters the text has, upper-cased.
-struct TwoBitMotif {
-    const uint8_t *dna;
+// ... or codes (crf_codes.h): a .2bit file's packed bases (BITS = 2) or a BAM file's 4-bit codes (BITS = 4), record r's
+// codes from byte rec_byte[r].  A motif never holds an N, so the codes alone give the letters the text has, upper-cased.
+template <int BITS>
+struct CodeMotif {
+    const uint8_t *codes;
     const uint64_t *rec_byte;
     char *operator()(char *p, uint32_t r, uint32_t start, uint32_t k) const {
-        const uint8_t *d = dna + rec_byte[r];
-        for (uint64_t i = start, e = (uint64_t)start + k; i < e; ++i) *p++ = "TCAG"[(d[i >> 2] >> (6 - 2 * (i & 3))) & 3];
-        return p;
-    }
-};
-
-// ... or a BAM file's 4-bit codes (record r's base i: nibble i & 1, high nibble first, of byte rec_byte[r] + i / 2), the
-// letters the decoded text has.
-struct NibbleMotif {
-    const uint8_t *nib;
-    const uint64_t *rec_byte;
-    char *operator()(char *p, uint32_t r, uint32_t start, uint32_t k) const {
-        const uint8_t *d = nib + rec_byte[r];
-        for (uint64_t i = start, e = (uint64_t)start + k; i < e; ++i) *p++ = "=ACMGRSVTWYHKDBN"[(d[i >> 1] >> (i & 1 ? 0 : 4)) & 15];
+        const uint8_t *d = codes + rec_byte[r];
+        for (uint64_t i = start, e = (uint64_t)start + k; i < e; ++i) *p++ = (char)code_letter<BITS>(d, i);
         return p;
     }
 };
@@ -144,20 +135,29 @@ static int write_rows_impl(const char *path, int append, int tsv, const char *na
     return CRF_OK;
 }
 
-extern "C" int crf_write_rows_at(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
-                                 const uint64_t *offsets, const uint64_t *origin, const uint32_t *record, const uint32_t *start,
-                                 const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
-    if (!path || (n_rows && (!bases || !offsets || !record || !start || !end || !motif_size)) || (!tsv && !names)) {
+// The argument checks and the C boundary of every rows entry point: Motif{src, index} reads the motif column.
+template <class Motif>
+static int write_rows_checked(const char *path, int append, int tsv, const char *names, const uint8_t *src,
+                              const uint64_t *index, const uint64_t *origin, const uint32_t *record, const uint32_t *start,
+                              const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
+    if (!path || (n_rows && (!src || !index || !record || !start || !end || !motif_size)) || (!tsv && !names)) {
         set_err("crf_write_rows: null argument");
         return CRF_ERR_ARG;
     }
     try {                                            // no exception crosses the C boundary
-        return write_rows_impl(path, append, tsv, names, TextMotif{bases, offsets}, origin, record, start, end, motif_size, n_rows,
+        return write_rows_impl(path, append, tsv, names, Motif{src, index}, origin, record, start, end, motif_size, n_rows,
                                bytes);
     } catch (const std::bad_alloc &) {
         set_err("crf_write_rows: out of host memory");
         return CRF_ERR_NOMEM;
     }
+}
+
+extern "C" int crf_write_rows_at(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
+                                 const uint64_t *offsets, const uint64_t *origin, const uint32_t *record, const uint32_t *start,
+                                 const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
+    return write_rows_checked<TextMotif>(path, append, tsv, names, bases, offsets, origin, record, start, end, motif_size, n_rows,
+                                         bytes);
 }
 
 extern "C" int crf_write_rows(const char *path, int append, int tsv, const char *names, const uint8_t *bases,
@@ -171,17 +171,8 @@ extern "C" int crf_write_rows(const char *path, int append, int tsv, const char 
 extern "C" int crf_write_rows_twobit(const char *path, int append, int tsv, const char *names, const uint8_t *dna,
                                      const uint64_t *rec_byte, const uint32_t *record, const uint32_t *start,
                                      const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
-    if (!path || (n_rows && (!dna || !rec_byte || !record || !start || !end || !motif_size)) || (!tsv && !names)) {
-        set_err("crf_write_rows: null argument");
-        return CRF_ERR_ARG;
-    }
-    try {
-        return write_rows_impl(path, append, tsv, names, TwoBitMotif{dna, rec_byte}, nullptr, record, start, end, motif_size,
-                               n_rows, bytes);
-    } catch (const std::bad_alloc &) {
-        set_err("crf_write_rows: out of host memory");
-        return CRF_ERR_NOMEM;
-    }
+    return write_rows_checked<CodeMotif<2>>(path, append, tsv, names, dna, rec_byte, nullptr, record, start, end, motif_size,
+                                            n_rows, bytes);
 }
 
 // The rows of reads from a BAM file (crf_fasta_nibbles: nib, rec_byte), the motif read from the codes: the same bytes
@@ -189,15 +180,6 @@ extern "C" int crf_write_rows_twobit(const char *path, int append, int tsv, cons
 extern "C" int crf_write_rows_nibbles(const char *path, int append, int tsv, const char *names, const uint8_t *nib,
                                       const uint64_t *rec_byte, const uint32_t *record, const uint32_t *start,
                                       const uint32_t *end, const uint32_t *motif_size, uint64_t n_rows, uint64_t *bytes) {
-    if (!path || (n_rows && (!nib || !rec_byte || !record || !start || !end || !motif_size)) || (!tsv && !names)) {
-        set_err("crf_write_rows: null argument");
-        return CRF_ERR_ARG;
-    }
-    try {
-        return write_rows_impl(path, append, tsv, names, NibbleMotif{nib, rec_byte}, nullptr, record, start, end, motif_size,
-                               n_rows, bytes);
-    } catch (const std::bad_alloc &) {
-        set_err("crf_write_rows: out of host memory");
-        return CRF_ERR_NOMEM;
-    }
+    return write_rows_checked<CodeMotif<4>>(path, append, tsv, names, nib, rec_byte, nullptr, record, start, end, motif_size,
+                                            n_rows, bytes);
 }

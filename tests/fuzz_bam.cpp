@@ -1,4 +1,4 @@
-// Sanitizer harness for BAM input: the reader (csrc/crf_fasta.h, fasta_detail::parse_bam and bam_decode) and the rows
+// Sanitizer harness for BAM input: the reader (csrc/crf_fasta.h, fasta_detail::parse_bam and decode_text) and the rows
 // writer that reads the motif from the 4-bit codes (csrc/crf_rows.h, crf_write_rows_nibbles), compiled WITHOUT the CUDA
 // runtime -- the page-locked allocation is stubbed to "no device" -- under AddressSanitizer + UBSan.
 //  * Reader: seeded random BAMs (all flags that matter, every code, absent qualities, names up to 254 characters, CIGAR

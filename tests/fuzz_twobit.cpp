@@ -1,4 +1,4 @@
-// Sanitizer harness for .2bit input: the reader (csrc/crf_fasta.h, fasta_detail::parse_twobit and twobit_decode) and the
+// Sanitizer harness for .2bit input: the reader (csrc/crf_fasta.h, fasta_detail::parse_twobit and decode_text) and the
 // rows writer that reads the motif from the packed bases (csrc/crf_rows.h, crf_write_rows_twobit), compiled WITHOUT the
 // CUDA runtime -- the page-locked allocation is stubbed to "no device" -- under AddressSanitizer + UBSan.
 //  * Reader: seeded random .2bit files (both byte orders, versions 0 and 1, records of 0 to 300 bases in shuffled data
